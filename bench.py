@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the hot path: Pallas MSM Gpoints/s (BASELINE.json metric), with the
 fold-step, batched-verify, size-sweep, strong-scaling and drop-in measurements as extra keys on the same JSON line.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--log2n L]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--log2n L] [--dump-outputs DIR]
 
 One "step" = one commitment MSM over n = 2^L synthetic scalars against a device-resident generator set
 (P_i = (k0 + i d) G, generated on the device; generators are fixed for the life of PublicParams in the
@@ -54,7 +54,19 @@ def parse_args():
     ap.add_argument("--no-extra", action="store_true", help="skip every side measurement")
     ap.add_argument("--no-sweep", action="store_true", help="skip the 2^20..2^26 size sweep / strong-scaling leg")
     ap.add_argument("--cpu-budget-s", type=float, default=150.0, help="wall-time budget of the CPU reference arm")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy "
+                    "(float64), to compare two builds output for output")
     return ap.parse_args()
+
+
+def dump_outputs(out_dir: str, points96: dict) -> None:
+    """Each 96-byte point (X, Y, Z; four little-endian u64 limbs per coordinate, Montgomery form, include/vdfgpu.h) as
+    DIR/<name>.npy: a (3, 8) float64 array of its 32-bit limbs, which float64 holds exactly."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, b in points96.items():
+        limbs = np.frombuffer(bytes(b), dtype="<u4").reshape(3, 8)
+        np.save(os.path.join(out_dir, f"{name}.npy"), limbs.astype(np.float64))
 
 
 def workload_config(log2n: int, world: int):
@@ -176,8 +188,10 @@ def run_reference(args):
         C.msm(0, pts, scal, True, cores)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        C.msm(0, pts, scal, True, cores)
+        out = C.msm(0, pts, scal, True, cores)
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"commitment": out})
     v = n / dt / 1e9
     same = n == n_full
     sample = (f"each step = one Pallas MSM over {'the full' if same else 'a bounded sample of'} n=2^{n.bit_length() - 1} points "
@@ -855,6 +869,9 @@ def run_ours(args):
     launches = lib.vdfgpu_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
     value = world * n / (ms_per_step * 1e-3) / 1e9
+    if args.dump_outputs:   # the commitment the last timed step returned, before later passes reuse its buffer
+        last = (steps - 1) % args.inflight
+        last_out = (total_dev[last] if world > 1 else runner.outs[last]).cpu().numpy().tobytes()
     barrier()
     # the same K commitments one at a time on one stream (runs last: slot 0 then holds the final result)
     serial_ms = ms_per_step if args.inflight == 1 else max_over_ranks(runner.timed(steps, 1, warm=1, after=after))
@@ -1039,6 +1056,8 @@ def run_ours(args):
         _lib.check(lib.vdfgpu_trim())
         torch.cuda.empty_cache()
         line["extra"] = extra_measurements(lib, _lib, torch, args)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"commitment": last_out})
     print_json(json.dumps(line))
     if world > 1:
         dist.barrier()

@@ -2,15 +2,19 @@
 TEST INFRASTRUCTURE + CPU BASELINE ONLY -- see the header of cpu_ref.c.  PARITY UNPINNED vs the Rust crates."""
 from __future__ import annotations
 
+import atexit
 import ctypes
 import os
+import shutil
 import subprocess
+import tempfile
 from ctypes import c_int, c_size_t, c_uint64, c_void_p
 from pathlib import Path
 
 _DIR = Path(__file__).resolve().parent
 _LIB = _DIR / "libvdf_cpu_ref.so"
 _lib = None
+_tmp_lib = None
 
 
 def _host_signature() -> str:
@@ -29,18 +33,33 @@ def _host_signature() -> str:
     return model + " " + hashlib.sha1(flags.encode()).hexdigest()[:12]
 
 
+def _make(out: Path) -> None:
+    try:
+        subprocess.run(["make", "-s", "-B", "-C", str(_DIR), f"OUT={out}"], check=True)
+    except (subprocess.CalledProcessError, OSError):
+        subprocess.run(["make", "-s", "-B", "-C", str(_DIR), f"OUT={out}", "ARCH=x86-64-v3"], check=True)
+
+
 def build() -> Path:
+    """Path of a library compiled for this host: the one beside the source, rebuilt there when it is stale, or -- when
+    the tree is read-only -- a copy compiled into a temporary directory that is removed when the process exits."""
+    global _tmp_lib
     sig_file = _DIR / "libvdf_cpu_ref.host"
     sig = _host_signature()
     stale = (not _LIB.exists() or _LIB.stat().st_mtime < (_DIR / "cpu_ref.c").stat().st_mtime
              or not sig_file.exists() or sig_file.read_text() != sig)
-    if stale:
-        try:
-            subprocess.run(["make", "-s", "-B", "-C", str(_DIR)], check=True)
-        except (subprocess.CalledProcessError, OSError):
-            subprocess.run(["make", "-s", "-B", "-C", str(_DIR), "ARCH=x86-64-v3"], check=True)
+    if not stale:
+        return _LIB
+    if os.access(_DIR, os.W_OK):
+        _make(_LIB)
         sig_file.write_text(sig)
-    return _LIB
+        return _LIB
+    if _tmp_lib is None:
+        tmp = tempfile.mkdtemp(prefix="vdf_cpu_ref-")
+        atexit.register(shutil.rmtree, tmp, True)
+        _make(Path(tmp) / _LIB.name)
+        _tmp_lib = Path(tmp) / _LIB.name
+    return _tmp_lib
 
 
 def load() -> ctypes.CDLL:
