@@ -134,6 +134,15 @@ struct CooMatrix {  // Vec<(usize, usize, Scalar)>
   std::vector<Fe> vals;
 };
 
+// Verdict of RelaxedR1CSShape::is_sat_relaxed / R1CSShape::is_sat (the report of vdfgpu_r1cs_is_sat_relaxed):
+// rows where Az.Bz != u.Cz + E, and each commitment check as 1 = equal, 0 = different, 2 = not checked
+struct SatReport {
+  uint64_t bad_rows = 0;
+  uint64_t first_bad_row = 0;   // num_cons when no row is violated
+  uint64_t comm_W = 2, comm_E = 2;
+  bool ok() const { return bad_rows == 0 && comm_W != 0 && comm_E != 0; }
+};
+
 class R1CSShape {
  public:
   R1CSShape(int field, size_t num_cons, size_t num_vars, size_t num_io, const CooMatrix& A, const CooMatrix& B,
@@ -186,8 +195,33 @@ class R1CSShape {
           "vdfgpu_commit_T");
     return {std::move(T), comm};
   }
+  // is_sat_relaxed(gens, U, W): Az.Bz = u.Cz + E per row, comm_W = commit(W), comm_E = commit(E).  E empty means
+  // E = 0; gens or a commitment nullptr: that commitment is not checked.  Commitments may be un-normalised Jacobian.
+  SatReport is_sat_relaxed(const Generators* gens, const std::vector<Fe>& W, const std::vector<Fe>& E, const Fe& u,
+                           const std::vector<Fe>& X, const Point* comm_W, const Point* comm_E) const {
+    if (W.size() != vars_ || X.size() != io_ || (!E.empty() && E.size() != cons_))
+      throw std::invalid_argument("is_sat_relaxed: InvalidWitnessLength");
+    return check(gens, W, E.empty() ? nullptr : E.data(), u.data(), X, comm_W, comm_E);
+  }
+  // is_sat(gens, U, W) of a fresh instance: Az.Bz = Cz (u = 1, E = 0), comm_W = commit(W)
+  SatReport is_sat(const Generators* gens, const std::vector<Fe>& W, const std::vector<Fe>& X, const Point* comm_W) const {
+    if (W.size() != vars_ || X.size() != io_) throw std::invalid_argument("is_sat: InvalidWitnessLength");
+    return check(gens, W, nullptr, nullptr, X, comm_W, nullptr);
+  }
 
  private:
+  SatReport check(const Generators* gens, const std::vector<Fe>& W, const Fe* E, const uint8_t* u,
+                  const std::vector<Fe>& X, const Point* comm_W, const Point* comm_E) const {
+    if (!gens && (comm_W || comm_E)) throw std::invalid_argument("is_sat: checking a commitment needs the generators");
+    if (gens && (gens->len() < cons_ || gens->len() < vars_))
+      throw std::invalid_argument("is_sat: fewer generators than max(vars, cons)");
+    uint64_t rep[4];
+    ok_or_throw(vdfgpu_r1cs_is_sat_relaxed(h_, gens ? gens->handle() : nullptr, W.data(), E, u, X.data(),
+                                           comm_W ? comm_W->data() : nullptr, comm_E ? comm_E->data() : nullptr, rep),
+                "vdfgpu_r1cs_is_sat_relaxed");
+    return SatReport{rep[0], rep[1], rep[2], rep[3]};
+  }
+
   int field_;
   size_t cons_, vars_, io_;
   vdfgpu_r1cs* h_ = nullptr;
@@ -229,6 +263,13 @@ class RunningWitness {
     E.resize(cons_);
     X.resize(io_);
     ok_or_throw(vdfgpu_running_get(h_, W.data(), E.data(), u.data(), X.data()), "vdfgpu_running_get");
+  }
+  // is_sat_relaxed of the resident running instance (nothing is copied back); a commitment nullptr is not checked
+  SatReport check(const Point* comm_W, const Point* comm_E) const {
+    uint64_t rep[4];
+    ok_or_throw(vdfgpu_running_check(h_, comm_W ? comm_W->data() : nullptr, comm_E ? comm_E->data() : nullptr, rep),
+                "vdfgpu_running_check");
+    return SatReport{rep[0], rep[1], rep[2], rep[3]};
   }
 
  private:

@@ -183,12 +183,34 @@ int vdfgpu_running_create(const vdfgpu_r1cs* s, vdfgpu_gens* gens, vdfgpu_runnin
 int vdfgpu_running_destroy(vdfgpu_running* f);
 int vdfgpu_running_set(vdfgpu_running* f, const void* W_host, const void* E_host, const void* u_host,
                             const void* X_host);
-int vdfgpu_running_get(const vdfgpu_running* f, void* W_host, void* E_host, void* u_host, void* X_host);
+int vdfgpu_running_get(const vdfgpu_running* f, void* W_host, void* E_host, void* u_host, void* X_host);   /* CompressedSNARK::prove's input */
 /* upload fresh witness, commit to it, compute T and comm_T; W2/T stay on the device for running_finish */
 int vdfgpu_running_commit(vdfgpu_running* f, const void* W2_host, const void* X2_host,
                        void* comm_W2_point96_host, void* comm_T_point96_host);
 /* W <- W + r*W2, E <- E + r*T, u <- u + r, X <- X + r*X2 */
 int vdfgpu_running_finish(vdfgpu_running* f, const void* r32_host);
+
+/* ---- RecursiveSNARK::verify (src/nova/proof.rs:382): RelaxedR1CSShape::is_sat_relaxed / R1CSShape::is_sat [R] of
+ * the primary and secondary running instances and of the last fresh secondary instance.  Each check fills a report of
+ * four uint64_t:
+ *   [0] rows with Az.Bz != u.Cz + E      [1] smallest such row, num_cons when there is none
+ *   [2] comm_W == commit(W): 1 yes, 0 no, 2 not checked       [3] comm_E == commit(E): same coding
+ * An unsatisfied instance is a verdict, not an error: the call returns 0.
+ * E_host NULL => E = 0; u_host NULL => u = 1 (both NULL: the strict R1CS check of a fresh instance).
+ * gens NULL => no commitment check (comm pointers must be NULL); comm_E96_host requires E_host; gens must hold at least
+ * max(num_vars, num_cons) points of the curve whose scalar field is the shape's.
+ * Commitments are compared as group elements: the caller's points may be un-normalised Jacobian. ---- */
+int vdfgpu_r1cs_is_sat_relaxed(const vdfgpu_r1cs* s, vdfgpu_gens* gens, const void* W_host, const void* E_host,
+                               const void* u_host, const void* X_host, const void* comm_W96_host,
+                               const void* comm_E96_host, uint64_t* report4_host);
+/* row check only, on the calling thread's stream, no synchronisation; the call initialises counts2_dev
+ * ([0] violating rows, [1] smallest violating row); E_dev may be NULL (E = 0); uX = [u | X] */
+int vdfgpu_r1cs_is_sat_relaxed_dev(const vdfgpu_r1cs* s, const void* W_dev, const void* E_dev, const void* uX_dev,
+                                   uint64_t* counts2_dev);
+/* the same check on a device-resident running instance (W, E, u, X never leave HBM) with its generators; either
+ * commitment may be NULL (not checked).  Before vdfgpu_running_set: VDFGPU_ERR_STATE. */
+int vdfgpu_running_check(const vdfgpu_running* f, const void* comm_W96_host, const void* comm_E96_host,
+                         uint64_t* report4_host);
 
 /* SURVEY 8f rank 1 -- the step-circuit part of the fresh witness never crosses PCIe.  A bank holds, for all n steps
  * of one proof, the 4t+1 values InverseMinRootCircuit::synthesize allocates (src/nova/proof.rs:107-126, :162-189),

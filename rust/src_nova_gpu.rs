@@ -13,6 +13,8 @@
 //!   * `WitnessBank`  the 4t+1 step-circuit variables of every step (`InverseMinRootCircuit::synthesize`,
 //!                    reference src/nova/proof.rs:87-140, :155-230) generated on the device
 //!   * `check_batch`  `MinRootVDF::check` (reference src/minroot.rs:369-371) over many independent chains
+//!   * `GpuShape::is_sat_relaxed`, `GpuRunning::check`  the satisfiability checks of `RecursiveSNARK::verify`
+//!                    (reference src/nova/proof.rs:382): rows and both commitments, `NovaError::UnSat` on failure
 //! The public API of the crate (`public_params`, `eval_and_make_circuits`, `NovaVDFProof::{prove_recursively,
 //! compress, verify}`) is unchanged; the unmodified nova-snark already reaches the GPU for every commitment through
 //! the patched pasta-msm (rust/patches/), and the types below are for a nova-snark whose `NIFS::prove` is patched
@@ -23,6 +25,7 @@
 use std::marker::PhantomData;
 
 use ff::PrimeField;
+use nova_snark::errors::NovaError; // [R]: UnSat, InvalidWitnessLength
 use pasta_curves::{pallas, vesta};
 use vdfgpu_sys as sys;
 
@@ -139,6 +142,9 @@ pub struct GpuShape<G: GpuCurve> {
     _g: PhantomData<G>,
 }
 
+unsafe impl<G: GpuCurve> Send for GpuShape<G> {}
+unsafe impl<G: GpuCurve> Sync for GpuShape<G> {} // read-only after creation; verify checks from several threads
+
 fn split_coo<F: Copy>(m: &[(usize, usize, F)]) -> (Vec<u64>, Vec<u64>, Vec<F>) {
     (m.iter().map(|e| e.0 as u64).collect(), m.iter().map(|e| e.1 as u64).collect(), m.iter().map(|e| e.2).collect())
 }
@@ -179,7 +185,50 @@ impl<G: GpuCurve> GpuShape<G> {
         })?;
         Ok((az, bz, cz))
     }
+    /// `RelaxedR1CSShape::is_sat_relaxed(gens, U, W)` [R] with the vectors on the host: `e = None` is E = 0 and
+    /// `u = None` is u = 1 (both `None`: `R1CSShape::is_sat` of a fresh instance).  `NovaError::UnSat` when a row or a
+    /// given commitment does not check out; a commitment that is `None` is not checked.  Infallible otherwise, like
+    /// nova's (a failing GPU call panics).
+    #[allow(clippy::too_many_arguments)]
+    pub fn is_sat_relaxed(
+        &self,
+        gens: &GpuGens<G>,
+        w: &[G::Scalar],
+        e: Option<&[G::Scalar]>,
+        u: Option<&G::Scalar>,
+        x: &[G::Scalar],
+        comm_w: Option<&G::Point>,
+        comm_e: Option<&G::Point>,
+    ) -> Result<(), NovaError> {
+        if w.len() != self.num_vars || x.len() != self.num_io || e.map_or(false, |e| e.len() != self.num_cons) {
+            return Err(NovaError::InvalidWitnessLength);
+        }
+        let mut rep = [0u64; 4];
+        let rc = unsafe {
+            sys::vdfgpu_r1cs_is_sat_relaxed(
+                self.h, gens.h, w.as_ptr().cast(), e.map_or(std::ptr::null(), |e| e.as_ptr().cast()),
+                u.map_or(std::ptr::null(), |u| (u as *const G::Scalar).cast()), x.as_ptr().cast(),
+                point_ptr::<G>(comm_w), point_ptr::<G>(comm_e), rep.as_mut_ptr(),
+            )
+        };
+        assert_eq!(rc, 0, "vdfgpu_r1cs_is_sat_relaxed: {}", sys::last_error());
+        sat_verdict(&rep)
+    }
 }
+
+fn point_ptr<G: GpuCurve>(p: Option<&G::Point>) -> *const libc::c_void {
+    p.map_or(std::ptr::null(), |p| (p as *const G::Point).cast())
+}
+
+/// report = [violating rows, first violating row, comm_W check, comm_E check] (1 equal, 0 different, 2 not checked)
+fn sat_verdict(rep: &[u64; 4]) -> Result<(), NovaError> {
+    if rep[0] == 0 && rep[2] != 0 && rep[3] != 0 {
+        Ok(())
+    } else {
+        Err(NovaError::UnSat)
+    }
+}
+
 impl<G: GpuCurve> Drop for GpuShape<G> {
     fn drop(&mut self) {
         unsafe { sys::vdfgpu_r1cs_destroy(self.h) };
@@ -260,7 +309,7 @@ impl<'a, G: GpuCurve> GpuRunning<'a, G> {
     pub fn fold(&mut self, r: &G::Scalar) -> Result<(), GpuError> {
         check(unsafe { sys::vdfgpu_running_finish(self.h, (r as *const G::Scalar).cast()) })
     }
-    /// Read the running witness back (needed by `RecursiveSNARK::verify` / `CompressedSNARK::prove` only).
+    /// Read the running witness back (needed by `CompressedSNARK::prove` only; `check` verifies it in place).
     pub fn get(&self) -> Result<(Vec<G::Scalar>, Vec<G::Scalar>, G::Scalar, Vec<G::Scalar>), GpuError> {
         let zero = <G::Scalar as ff::Field>::zero();
         let (mut w, mut e, mut u, mut x) =
@@ -270,6 +319,14 @@ impl<'a, G: GpuCurve> GpuRunning<'a, G> {
                                     (&mut u as *mut G::Scalar).cast(), x.as_mut_ptr().cast())
         })?;
         Ok((w, e, u, x))
+    }
+    /// `is_sat_relaxed` of the resident running instance against the instance's commitments (`U.comm_W`, `U.comm_E`):
+    /// the relaxed half of `RecursiveSNARK::verify` without copying W and E back.  `NovaError::UnSat` on a failed check.
+    pub fn check(&self, comm_w: Option<&G::Point>, comm_e: Option<&G::Point>) -> Result<(), NovaError> {
+        let mut rep = [0u64; 4];
+        let rc = unsafe { sys::vdfgpu_running_check(self.h, point_ptr::<G>(comm_w), point_ptr::<G>(comm_e), rep.as_mut_ptr()) };
+        assert_eq!(rc, 0, "vdfgpu_running_check: {}", sys::last_error());
+        sat_verdict(&rep)
     }
 }
 impl<'a, G: GpuCurve> Drop for GpuRunning<'a, G> {

@@ -127,6 +127,16 @@ extern "C" {
                                  comm_w2_point96_host: *mut c_void, comm_t_point96_host: *mut c_void) -> c_int;
     pub fn vdfgpu_running_finish(f: *mut vdfgpu_running, r32_host: *const c_void) -> c_int;
 
+    // ---- RecursiveSNARK::verify: is_sat_relaxed / is_sat; report = [bad rows, first bad row, comm_W ok, comm_E ok]
+    pub fn vdfgpu_r1cs_is_sat_relaxed(s: *const vdfgpu_r1cs, gens: *mut vdfgpu_gens, w_host: *const c_void,
+                                      e_host: *const c_void, u_host: *const c_void, x_host: *const c_void,
+                                      comm_w96_host: *const c_void, comm_e96_host: *const c_void,
+                                      report4_host: *mut u64) -> c_int;
+    pub fn vdfgpu_r1cs_is_sat_relaxed_dev(s: *const vdfgpu_r1cs, w_dev: *const c_void, e_dev: *const c_void,
+                                          ux_dev: *const c_void, counts2_dev: *mut u64) -> c_int;
+    pub fn vdfgpu_running_check(f: *const vdfgpu_running, comm_w96_host: *const c_void, comm_e96_host: *const c_void,
+                                report4_host: *mut u64) -> c_int;
+
     // ---- SURVEY 8f rank 1: step-circuit witnesses generated and kept on the device
     pub fn vdfgpu_witness_bank_create(field: c_int, z_in_state96_host: *const c_void, t: u64, n: size_t,
                                       out: *mut *mut vdfgpu_witness_bank) -> c_int;

@@ -73,6 +73,10 @@ PROTOTYPES = {
     "vdfgpu_running_get": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "vdfgpu_running_commit": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "vdfgpu_running_finish": (c_int, [c_void_p, c_void_p]),
+    "vdfgpu_r1cs_is_sat_relaxed": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                           POINTER(c_uint64)]),
+    "vdfgpu_r1cs_is_sat_relaxed_dev": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vdfgpu_running_check": (c_int, [c_void_p, c_void_p, c_void_p, POINTER(c_uint64)]),
     "vdfgpu_eq_evals": (c_int, [c_int, c_void_p, c_size_t, c_void_p]),
     "vdfgpu_eq_evals_dev": (c_int, [c_int, c_void_p, c_size_t, c_void_p]),
     "vdfgpu_sumcheck_cubic": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p]),

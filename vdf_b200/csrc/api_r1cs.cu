@@ -88,6 +88,85 @@ void upload_constants_r1cs() { VDF_CUDA_CHECK(upload_field_constants()); }
 
 static fe host_one(int field) { return field == VDFGPU_FP ? Fp::one() : Fq::one(); }
 
+// ---- satisfiability checks (vdfgpu_r1cs_is_sat_relaxed*, vdfgpu_running_check) ----------------------------------
+// counts2: the two u64 of the C ABI, as four u32 words on the device (see SatInitFn)
+static void launch_sat(CudaLaunch& L, const vdfgpu_r1cs* s, ZView z, const fe* E, uint64_t* counts2) {
+  uint32_t* words = reinterpret_cast<uint32_t*>(counts2);
+  uint32_t* bad = words;
+  uint32_t* first = words + 2;
+  L.run<32>(1, SatInitFn{words, s->cons});
+  if (s->field == VDFGPU_FP) L.run<128, 8>(s->cons, RelaxedSatFn<Fp>{s->view(), z, E, bad, first});
+  else L.run<128, 8>(s->cons, RelaxedSatFn<Fq>{s->view(), z, E, bad, first});
+}
+
+// What one check brings back to the host: the two counters and commit(W), commit(E) as un-normalised points, in ONE
+// device block [counts2 | pad to 96 B | point | point] copied with one D2H.
+struct SatResult {
+  uint64_t counts[2] = {0, 0};
+  uint8_t comm[2][96] = {};
+};
+constexpr size_t SAT_BLOCK = 3 * sizeof(jac_t);
+static_assert(sizeof(jac_t) == 96, "points are 96 bytes");
+
+// pinned landing zone of the read-back, one per calling thread (the previous call on this thread has been waited for)
+static uint8_t* pinned_sat() {
+  static thread_local uint8_t* p = nullptr;
+  if (!p) VDF_CUDA_CHECK(cudaHostAlloc((void**)&p, SAT_BLOCK, cudaHostAllocDefault));
+  return p;
+}
+
+static void check_sat_gens(const vdfgpu_r1cs* s, const vdfgpu_gens* g, const char* what) {
+  check_gens_field(s, g);
+  if (g->n < s->cons || g->n < s->vars) throw ArgError(std::string(what) + ": fewer generators than max(vars, cons)");
+}
+
+// Row check, then commit(W) and commit(E) in ONE batched MSM pass (as running_commit_enqueue batches commit(W2) and
+// commit(T)), then one D2H into pinned memory; the wait happens after the context lock is released.  The points are
+// computed un-normalised whatever the set's flags and normalised on the host once they have landed (`res`).
+static void sat_enqueue(const vdfgpu_r1cs* s, vdfgpu_gens* gens, const fe* W, const fe* E, const fe* uX, bool want_W,
+                        bool want_E, SatResult& res) {
+  Context& c = ctx();
+  cudaStream_t st = cur_stream();
+  CudaLaunch L(st);
+  DevBuf<jac_t> out(3, st);
+  launch_sat(L, s, ZView{W, uX, uX + 1}, E, reinterpret_cast<uint64_t*>(out.p));
+  c.launches += L.launches;
+  const fe* vecs[2];
+  size_t lens[2];
+  uint32_t k = 0;
+  if (want_W) { vecs[k] = W; lens[k++] = s->vars; }
+  if (want_E) { vecs[k] = E; lens[k++] = s->cons; }
+  if (k) msm_batch_on_device(gens, vecs, lens, k, out.p + 1, true);
+  uint8_t* pin = pinned_sat();
+  d2h(pin, out.p, 96 + k * sizeof(jac_t), st);
+  sync_after_unlock(st);
+  copy_after_sync(res.counts, pin, sizeof(res.counts));
+  for (uint32_t j = 0, slot = 0; j < 2; j++) {
+    if (!(j == 0 ? want_W : want_E)) continue;
+    copy_after_sync(res.comm[j], pin + 96 * (1 + slot++), 96);
+    normalise_after_sync(res.comm[j], 1, gens->curve);
+  }
+}
+
+// 1 = the caller's point is the same group element as the computed one, 0 = it is not
+static uint64_t same_point(int curve, const uint8_t* computed96, const void* given96) {
+  uint8_t g[96];
+  std::memcpy(g, given96, 96);
+  vdfgpu_point_normalise_host(curve, g, 1);   // Jacobian of any Z -> (x, y, 1) or (0, 0, 0), as `computed96` is
+  return std::memcmp(g, computed96, 96) == 0 ? 1 : 0;
+}
+
+// runs after guarded() has waited: fills the report (2 = commitment not checked)
+static int sat_report(int rc, const SatResult& res, const vdfgpu_gens* gens, const void* comm_W, const void* comm_E,
+                      uint64_t* report4) {
+  if (rc != VDFGPU_OK) return rc;
+  report4[0] = res.counts[0];
+  report4[1] = res.counts[1];
+  report4[2] = comm_W ? same_point(gens->curve, res.comm[0], comm_W) : 2;
+  report4[3] = comm_E ? same_point(gens->curve, res.comm[1], comm_E) : 2;
+  return VDFGPU_OK;
+}
+
 }  // namespace vdf
 
 using namespace vdf;
@@ -265,6 +344,43 @@ int vdfgpu_multiply_vec_dev(const vdfgpu_r1cs* s, const void* W_dev, const void*
   });
 }
 
+int vdfgpu_r1cs_is_sat_relaxed(const vdfgpu_r1cs* s, vdfgpu_gens* gens, const void* W_host, const void* E_host,
+                               const void* u_host, const void* X_host, const void* comm_W96_host,
+                               const void* comm_E96_host, uint64_t* report4_host) {
+  SatResult res;
+  const int rc = guarded([&] {
+    if (!s || !W_host || !report4_host) throw ArgError("r1cs_is_sat_relaxed: null pointer");
+    if (s->io && !X_host) throw ArgError("r1cs_is_sat_relaxed: null X");
+    if (!gens && (comm_W96_host || comm_E96_host)) throw ArgError("r1cs_is_sat_relaxed: commitments given without generators");
+    if (comm_E96_host && !E_host) throw ArgError("r1cs_is_sat_relaxed: comm_E given without E");
+    if (gens) check_sat_gens(s, gens, "r1cs_is_sat_relaxed");
+    require_ready();
+    cudaStream_t st = cur_stream();
+    const size_t nv = s->vars, io = s->io, nc = s->cons;
+    DevBuf<fe> W(nv ? nv : 1, st), E(E_host ? nc : 1, st), uX(1 + io, st);
+    h2d_scalars(W.p, W_host, nv * 32, st);
+    if (E_host) h2d_scalars(E.p, E_host, nc * 32, st);
+    const fe one = host_one(s->field);
+    h2d(uX.p, u_host ? u_host : &one, 32, st);   // pageable 32-byte copies are staged before cudaMemcpyAsync returns
+    h2d(uX.p + 1, X_host, io * 32, st);
+    sat_enqueue(s, gens, W.p, E_host ? E.p : nullptr, uX.p, comm_W96_host != nullptr, comm_E96_host != nullptr, res);
+  });
+  return sat_report(rc, res, gens, comm_W96_host, comm_E96_host, report4_host);
+}
+
+int vdfgpu_r1cs_is_sat_relaxed_dev(const vdfgpu_r1cs* s, const void* W_dev, const void* E_dev, const void* uX_dev,
+                                   uint64_t* counts2_dev) {
+  return guarded([&] {
+    if (!s || !uX_dev || !counts2_dev || (s->vars && !W_dev)) throw ArgError("r1cs_is_sat_relaxed_dev: null pointer");
+    require_ready();
+    Context& c = ctx();
+    CudaLaunch L(cur_stream());
+    const fe* ux = reinterpret_cast<const fe*>(uX_dev);
+    launch_sat(L, s, ZView{reinterpret_cast<const fe*>(W_dev), ux, ux + 1}, reinterpret_cast<const fe*>(E_dev), counts2_dev);
+    c.launches += L.launches;
+  });
+}
+
 static void launch_bind_rows(CudaLaunch& L, const vdfgpu_r1cs* s, const fe* eq, const fe* coef, fe* eq3, fe* out) {
   const size_t ncols = (size_t)s->vars + 1 + s->io;
   const CscView v = s->col_view();
@@ -417,6 +533,20 @@ int vdfgpu_running_get(const vdfgpu_running* f, void* W_host, void* E_host, void
     if (X_host) d2h(X_host, f->uX + 1, (size_t)f->shape->io * 32, cur_stream());
     sync_after_unlock(cur_stream());
   });
+}
+
+// is_sat_relaxed of the resident running instance: W, E, u, X never leave HBM.  Between running_commit and
+// running_finish this is still the running (not yet folded) instance: only W2, uX2 and T have changed.
+int vdfgpu_running_check(const vdfgpu_running* f, const void* comm_W96_host, const void* comm_E96_host,
+                         uint64_t* report4_host) {
+  SatResult res;
+  const int rc = guarded([&] {
+    if (!f || !report4_host) throw ArgError("running_check: null pointer");
+    if (!f->have_running) throw StateError("running_check: no running instance set");
+    require_ready();
+    sat_enqueue(f->shape, f->gens, f->W, f->E, f->uX, comm_W96_host != nullptr, comm_E96_host != nullptr, res);
+  });
+  return sat_report(rc, res, f ? f->gens : nullptr, comm_W96_host, comm_E96_host, report4_host);
 }
 
 // uX2 = [1 | X2] in one copy from the instance's pinned staging area (the previous step's copy has long completed:

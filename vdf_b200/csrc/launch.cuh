@@ -30,6 +30,16 @@ VDF_HD uint32_t atomic_add_u32(uint32_t* p, uint32_t v) {
 #endif
 }
 
+VDF_HD uint32_t atomic_min_u32(uint32_t* p, uint32_t v) {
+#if defined(__CUDA_ARCH__)
+  return atomicMin(p, v);
+#else
+  uint32_t old = *p;
+  if (v < old) *p = v;
+  return old;
+#endif
+}
+
 // ---- workspace arena ------------------------------------------------------------------------------
 // Host-side bookkeeping of ONE preallocated device block per stream: the pipelines allocate and free their
 // temporaries here (first fit, lowest address, 256-byte granules) instead of calling cudaMallocAsync /

@@ -115,6 +115,70 @@ struct CrossTermFn {
   }
 };
 
+// ---- satisfiability: RelaxedR1CSShape::is_sat_relaxed / R1CSShape::is_sat [R], the row part of
+// RecursiveSNARK::verify (src/nova/proof.rs:382) ------------------------------------------------------------------
+// The two little-endian u64 counters of the C ABI (violating rows, smallest violating row), written as four u32
+// words: RelaxedSatFn updates the low words (both values stay below 2^30) and only ever accesses them as u32.
+struct SatInitFn {
+  uint32_t* words;   // [4]
+  uint32_t cons;
+  VDF_HD void operator()(size_t) const {
+    words[0] = 0; words[1] = 0;      // violating rows
+    words[2] = cons; words[3] = 0;   // smallest violating row: cons = none
+  }
+};
+
+// one thread per constraint row: d = Az*Bz - u*Cz - E[row] (E == nullptr: E = 0); the row violates the relation iff
+// d != 0 (inputs are canonical, so zero has one encoding).  *bad counts the violating rows, *first ends as the smallest
+// of them (it starts at cons).  Violations are rare in real use: one warp ballot, then lane 0 issues the atomics.
+template <class F>
+struct RelaxedSatFn {
+  CsrView m;
+  ZView z;
+  const fe* E;
+  uint32_t* bad;
+  uint32_t* first;
+  VDF_HD void operator()(size_t idx) const {
+    const uint32_t row = (uint32_t)idx;
+    const fe one = F::one(), minus_one = F::neg(F::one());
+    uint32_t ptr[3][2];
+#pragma unroll
+    for (uint32_t mat = 0; mat < 3; mat++) {   // six independent loads, as in CrossTermFn
+      ptr[mat][0] = m.row_ptr[mat * m.cons + row];
+      ptr[mat][1] = m.row_ptr[mat * m.cons + row + 1];
+    }
+    fe d;   // Az, then Az*Bz, then the difference: one accumulator and one running value live at a time
+#pragma unroll
+    for (uint32_t mat = 0; mat < 3; mat++) {
+      fe acc = F::zero();
+      for (uint32_t k = ptr[mat][0]; k < ptr[mat][1]; k++)
+        acc = mul_acc<F>(acc, fe_load(m.val + k), z_at<F>(z, m.vars, m.col[k]), one, minus_one);
+      if (mat == 0) d = acc;
+      else if (mat == 1) d = F::mul(d, acc);
+      else d = F::sub(d, F::mul(fe_load(z.u), acc));
+    }
+    if (E) d = F::sub(d, fe_load(E + row));
+    const bool violated = !F::eq(d, F::zero());
+#if defined(__CUDA_ARCH__)
+    // The lanes of this warp that hold a row: functor_kernel has already returned for i >= n, so the last warp is
+    // partial when cons % 32 != 0.  The mask is computed from cons rather than taken from __activemask(): after the
+    // data-dependent loops above the lanes need not have reconverged, and a ballot over a subset would lose counts.
+    const uint32_t lane = threadIdx.x & 31u, base = row - lane;
+    const uint32_t live = m.cons - base >= 32u ? 0xffffffffu : (1u << (m.cons - base)) - 1u;
+    const uint32_t votes = __ballot_sync(live, violated);
+    if (lane == 0 && votes) {
+      atomic_add_u32(bad, (uint32_t)__popc(votes));
+      atomic_min_u32(first, base + (uint32_t)(__ffs(votes) - 1));
+    }
+#else
+    if (violated) {
+      atomic_add_u32(bad, 1);
+      atomic_min_u32(first, row);
+    }
+#endif
+  }
+};
+
 // ---- transposed product for Spartan's inner sum-check (SURVEY 8f rank 2) ---------------------------------------
 // M(y) = sum_x eq(x) * (rA A[x,y] + rB B[x,y] + rC C[x,y]) for every column y: nova-snark's
 // compute_eval_table_sparse combined with the three challenges [R], reached from CompressedSNARK::prove

@@ -30,6 +30,37 @@ def _coo_arrays(M: Coo, m: int):
     return rows, cols, vals, len(M)
 
 
+@dataclass
+class SatReport:
+    """Verdict of one satisfiability check (RelaxedR1CSShape::is_sat_relaxed / R1CSShape::is_sat): the rows where
+    Az.Bz != u.Cz + E, and whether each commitment equals the commitment of its vector (None: not checked)."""
+    bad_rows: int
+    first_bad_row: Optional[int]
+    comm_W_ok: Optional[bool]
+    comm_E_ok: Optional[bool]
+
+    @property
+    def ok(self) -> bool:
+        return self.bad_rows == 0 and self.comm_W_ok is not False and self.comm_E_ok is not False
+
+    @classmethod
+    def from_words(cls, rep, num_cons: int) -> "SatReport":
+        verdict = {0: False, 1: True, 2: None}
+        return cls(int(rep[0]), None if rep[1] == num_cons else int(rep[1]), verdict[rep[2]], verdict[rep[3]])
+
+
+def _point_arg(p, base: int) -> Optional[bytes]:
+    """A commitment as the 96-byte Jacobian point the C ABI compares: an affine tuple, or 96 raw bytes (any Z, the
+    identity as Z = 0).  None: not checked."""
+    if p is None:
+        return None
+    if isinstance(p, (bytes, bytearray)):
+        if len(p) != POINT_BYTES:
+            raise ValueError("a commitment is a 96-byte Jacobian point")
+        return bytes(p)
+    return fe_to_bytes(p[0], base) + fe_to_bytes(p[1], base) + fe_to_bytes(1, base)
+
+
 class R1CSShape:
     """nova R1CSShape: A, B, C in COO over z = [W | u | X]; uploaded once as CSR."""
 
@@ -77,6 +108,39 @@ class R1CSShape:
             _lib.as_ptr(T), _lib.as_ptr(comm) if gens else None))
         cT = point_from_bytes(bytes(comm), CURVE_BASE[gens.curve]) if gens else None
         return fes_from_bytes(bytes(T), m), cT
+
+    def is_sat_relaxed(self, gens: Optional[Generators], W: Sequence[int], E: Optional[Sequence[int]],
+                       U: "RelaxedR1CSInstance") -> SatReport:
+        """RelaxedR1CSShape::is_sat_relaxed: Az.Bz = u.Cz + E on every row, comm_W = commit(W), comm_E = commit(E).
+        E None means E = 0; a commitment of U that is None is not checked (gens None: neither is)."""
+        if len(W) != self.num_vars or len(U.X) != self.num_io or (E is not None and len(E) != self.num_cons):
+            raise ValueError("W, E or X has the wrong length")  # nova: NovaError::InvalidWitnessLength
+        m = self.m
+        return self._check(gens, fes_to_bytes(W, m), None if E is None else fes_to_bytes(E, m), fe_to_bytes(U.u, m),
+                           fes_to_bytes(U.X, m), U.comm_W, U.comm_E)
+
+    def is_sat(self, gens: Optional[Generators], W: Sequence[int], X: Sequence[int], comm_W=None) -> SatReport:
+        """R1CSShape::is_sat of a fresh instance: Az.Bz = Cz (u = 1, E = 0) and comm_W = commit(W)."""
+        if len(W) != self.num_vars or len(X) != self.num_io:
+            raise ValueError("W or X has the wrong length")  # nova: NovaError::InvalidWitnessLength
+        m = self.m
+        return self._check(gens, fes_to_bytes(W, m), None, None, fes_to_bytes(X, m), comm_W, None)
+
+    def _check(self, gens, Wb, Eb, ub, Xb, comm_W, comm_E) -> SatReport:
+        if gens is None and (comm_W is not None or comm_E is not None):
+            raise ValueError("checking a commitment needs the generators")
+        cW, cE = (_point_arg(c, CURVE_BASE[gens.curve]) if gens else None for c in (comm_W, comm_E))
+        rep = (ctypes.c_uint64 * 4)()
+        _lib.check(_lib.load().vdfgpu_r1cs_is_sat_relaxed(
+            self._h, gens._h if gens else None, _lib.as_ptr(Wb), _lib.as_ptr(Eb), _lib.as_ptr(ub), _lib.as_ptr(Xb),
+            _lib.as_ptr(cW), _lib.as_ptr(cE), rep))
+        return SatReport.from_words(rep, self.num_cons)
+
+    def is_sat_relaxed_dev(self, W_dev, E_dev, uX_dev, counts2_dev) -> None:
+        """Row check on device buffers (torch tensors or raw pointers), enqueued on the calling thread's stream:
+        counts2_dev receives (violating rows, smallest violating row or num_cons) as two u64."""
+        _lib.check(_lib.load().vdfgpu_r1cs_is_sat_relaxed_dev(self._h, _lib.as_ptr(W_dev), _lib.as_ptr(E_dev),
+                                                              _lib.as_ptr(uX_dev), _lib.as_ptr(counts2_dev)))
 
     def close(self):
         if self._h:
@@ -185,6 +249,15 @@ class RunningProver:
         return (fes_from_bytes(bytes(W), m), fes_from_bytes(bytes(E), m), fes_from_bytes(bytes(u), m)[0],
                 fes_from_bytes(bytes(X[:s.num_io * 32]), m))
 
+    def check(self) -> SatReport:
+        """is_sat_relaxed of the resident running instance against self.U's commitments (None: not checked); W, E,
+        u and X stay on the device."""
+        base = CURVE_BASE[self.gens.curve]
+        cW, cE = (_point_arg(c, base) for c in ((self.U.comm_W, self.U.comm_E) if self.U else (None, None)))
+        rep = (ctypes.c_uint64 * 4)()
+        _lib.check(_lib.load().vdfgpu_running_check(self._h, _lib.as_ptr(cW), _lib.as_ptr(cE), rep))
+        return SatReport.from_words(rep, self.shape.num_cons)
+
     def prove_step_bytes(self, W2: bytes, X2: bytes, r: Optional[int] = None):
         """One fold of a fresh satisfying (W2, X2): returns (comm_W2, comm_T, r) with points as 96-byte
         buffers.  Timed region of the fold-steps/s benchmark."""
@@ -268,4 +341,9 @@ class RecursiveProver:
             b = self.primary.prove_step_bank_bytes(bank, step, step_offset, pri_W2, pri_X2, r_pri)
         self.steps += 1
         return a, b
+
+    def check(self) -> Tuple[SatReport, SatReport]:
+        """is_sat_relaxed of the primary and the secondary running instance (RecursiveSNARK::verify's two relaxed
+        checks, src/nova/proof.rs:382), on the device-resident vectors."""
+        return self.primary.check(), self.secondary.check()
 
