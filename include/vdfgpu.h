@@ -97,7 +97,9 @@ void mult_pippenger_vesta(void* out_point96, const void* points_affine72, size_t
 int vdfgpu_dropin_cache_clear(void);
 int vdfgpu_dropin_cache_stats(uint64_t* hits, uint64_t* misses, uint64_t* entries);
 
-/* Generators are fixed for the life of PublicParams (src/nova/proof.rs:232-237): upload/repack once. */
+/* Generators are fixed for the life of PublicParams (src/nova/proof.rs:232-237): upload/repack once.
+ * window_bits (2..24, 0 = by size) applies to VDFGPU_GENS_TABLE sets, whose table levels are built for it.  A plain set
+ * ignores it and picks the window size per call from the number of scalars; vdfgpu_gens_window_bits reports either. */
 int vdfgpu_gens_create(int curve, const void* points_affine72_host, size_t n, uint32_t flags,
                        uint32_t window_bits /* 0 = auto */, vdfgpu_gens** out);
 /* synthetic set P_i = (k0 + i*d) * G, G = (-1, 2), generated on the device (bench/tests, SURVEY 8d C2);

@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 from oracle import pasta as O
+from tests.msm_cases import families, signed_digits
 from tests.util import aligned, edge_field_values, nova_like_scalars, ptr, rand_scalars
 
 SZ = ctypes.c_size_t
@@ -74,6 +75,51 @@ def test_msm_pipeline(emul, cid, table):
             continue  # W bucket sets of 2^14+ buckets: too slow for the CPU loop; the table layout covers the path
         assert _msm(emul, cid, table, c, S, G, logm, pts, sc) == want, (c, S, G, logm)
     assert _msm(emul, cid, table, 8, 16, 4, 3, pts, sc, is_mont=0) == want
+
+
+def test_msm_case_families_hit_their_branches():
+    """Each scalar family of tests/msm_cases.py reaches the recoding branch it is named for, at every window size."""
+    for c in range(2, 25):
+        K, B = 254 // c, 1 << (c - 1)
+        for order in (O.PALLAS.order, O.VESTA.order):
+            fam = families(c, order)
+            dg, cin = signed_digits(fam["top_bucket"], c)
+            assert dg[:K] == [B] * K and not any(cin)
+            dg, cin = signed_digits(fam["neg_chain"], c)
+            assert all(x <= 0 for x in dg[:K]) and all(cin[1:K + 1])
+            dg, cin = signed_digits(fam["zero_with_carry"], c)
+            assert dg[0] == -1 and dg[1:K] == [0] * (K - 1) and all(cin[1:K + 1]) and dg[K] == 1
+            assert any(x == 0 and ci for x, ci in zip(*signed_digits(fam["zero_with_carry_254"], c)))
+            for d in {1, B - 1, B}:
+                dg, cin = signed_digits(fam[f"one_digit_{d}"], c)
+                assert dg[:K] == [d] * K and not any(dg[K:]) and not any(cin)
+            for d in {1, B - 1}:
+                dg, cin = signed_digits(fam[f"alt_sign_{d}"], c)
+                assert dg[:K - 1] == [-d] * (K - 1) and dg[K - 1] == d and not any(dg[K:])
+            for name in ("order-1", "order-2", "half", "2^253", "2^254-B", "zero", "one"):
+                signed_digits(fam[name], c)
+
+
+def test_msm_digit_families(emul):
+    """The scalar families through the emulated pipeline at every window size: c = 2..24 in the table layout (one
+    bucket set), c = 2..10 in the plain layout (W sets), Montgomery and raw scalars, logm 3 and 8 (stage 6 takes the
+    tree, the latency or the hybrid path), without and with batched-affine halving rounds."""
+    k0, d = 3, 7
+    pts = {cid: O.CURVES[cid].progression(k0, d, 24) for cid in (O.CURVE_PALLAS, O.CURVE_VESTA)}
+    settings = ((1, 3, (0, 0)), (0, 8, (2, 5)))   # (is_mont, logm, affine rounds and K)
+    try:
+        for table, cs in ((1, range(2, 25)), (0, range(2, 11))):
+            for c in cs:
+                for cid in (O.CURVE_PALLAS, O.CURVE_VESTA):
+                    cv = O.CURVES[cid]
+                    sc = list(families(c, cv.order).values())
+                    sc += rand_scalars(O.XorShiftRng(), cv.order, 24 - len(sc))
+                    is_mont, logm, aff = settings[(c + cid) % 2]
+                    emul.emul_set_affine(*aff)
+                    got = _msm(emul, cid, table, c, 3, 4, logm, pts[cid], sc, is_mont)
+                    assert got == O.jac_to_bytes(cv, cv.msm_known_dlog(sc, k0, d)), (table, c, cid, is_mont, logm)
+    finally:
+        emul.emul_set_affine(0, 0)
 
 
 def test_msm_skewed_and_edges(emul):

@@ -38,7 +38,7 @@ def test_msm_small_vs_oracle(gpu_lib, cid, table):
     pts[9], sc[9] = pts[8], sc[8]       # duplicate point, same scalar (doubling inside a bucket)
     pts[11], sc[11] = cv.neg(pts[10]), sc[10]  # P and -P cancel
     want = O.jac_to_bytes(cv, cv.msm(sc, pts))
-    for wb in (0, 5, 9, 13):
+    for wb in ((0, 5, 9, 13) if table else (0,)):   # a plain set picks c from n and ignores window_bits
         g = G.Generators.from_points(cid, pts, table=table, window_bits=wb)
         assert g.commit_bytes(O.fes_to_bytes(sc, cv.order)) == want, (cid, table, wb)
         # prefix commits (nova commits to vectors shorter than the generator set)
