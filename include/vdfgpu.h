@@ -29,7 +29,11 @@
  * is what the literal pasta-msm entry points need).  Every entry point may be called from any thread: the library
  * takes an internal lock only while it ENQUEUES work and waits for the GPU after releasing it, so calls from
  * several threads overlap on the device; the stream is a per-THREAD setting; the caller's current CUDA device is
- * restored before a call returns.  A handle must not be destroyed while another thread uses it; a generator set or
+ * restored before a call returns.  Ordering: the work a call does on a handle's own device state (a running instance's
+ * W, E, u, X, W2, T) is ordered behind the previous call on that handle whatever the stream or thread of either, so
+ * vdfgpu_running_finish may return before its fold has run and the next call may come from another stream or thread.
+ * Device buffers the caller passes to "_dev" entry points are ordered by the caller's stream only: whatever writes
+ * them on another stream must be made visible to it (an event) before the call.  A handle must not be destroyed while another thread uses it; a generator set or
  * shape held by a running instance cannot be destroyed (VDFGPU_ERR_STATE) until that instance is.
  *
  * Inputs: every 32-byte field element must be the canonical Montgomery image of a value < m, as pasta_curves'
@@ -189,7 +193,8 @@ int vdfgpu_running_get(const vdfgpu_running* f, void* W_host, void* E_host, void
 /* upload fresh witness, commit to it, compute T and comm_T; W2/T stay on the device for running_finish */
 int vdfgpu_running_commit(vdfgpu_running* f, const void* W2_host, const void* X2_host,
                        void* comm_W2_point96_host, void* comm_T_point96_host);
-/* W <- W + r*W2, E <- E + r*T, u <- u + r, X <- X + r*X2 */
+/* W <- W + r*W2, E <- E + r*T, u <- u + r, X <- X + r*X2; returns once enqueued (the next call on f, on any stream or
+ * thread, is ordered behind it) */
 int vdfgpu_running_finish(vdfgpu_running* f, const void* r32_host);
 
 /* ---- RecursiveSNARK::verify (src/nova/proof.rs:382): RelaxedR1CSShape::is_sat_relaxed / R1CSShape::is_sat [R] of

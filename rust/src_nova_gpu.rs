@@ -305,7 +305,8 @@ impl<'a, G: GpuCurve> GpuRunning<'a, G> {
         Ok((cw, ct))
     }
     /// `RelaxedR1CSWitness::fold` + the scalar half of `RelaxedR1CSInstance::fold`:
-    /// W += r W2, E += r T, u += r, X += r X2.  Returns at once; the next call is ordered behind it on the GPU.
+    /// W += r W2, E += r T, u += r, X += r X2.  Returns at once; the next call on this instance is ordered behind it
+    /// on the GPU, whichever stream (`vdfgpu_set_stream`) or thread it comes from: a verifier thread may `check` it.
     pub fn fold(&mut self, r: &G::Scalar) -> Result<(), GpuError> {
         check(unsafe { sys::vdfgpu_running_finish(self.h, (r as *const G::Scalar).cast()) })
     }

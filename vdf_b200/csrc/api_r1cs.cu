@@ -37,6 +37,9 @@ struct vdfgpu_running {
   vdf::fe* r = nullptr;   // challenge
   vdf::jac_t* comm = nullptr;  // [2] comm_W2, comm_T
   uint8_t* bounce = nullptr;   // pinned: both commitments come back with one asynchronous copy; [1 + io] staging of uX2 behind it
+  // recorded behind the work of every call on this instance, waited on before the next one enqueues: a call on another
+  // stream or thread (vdfgpu_running_finish returns before its fold has run) is ordered behind the previous one
+  cudaEvent_t done = nullptr;
   bool have_running = false, have_fresh = false;
 };
 
@@ -87,6 +90,11 @@ static void check_gens_field(const vdfgpu_r1cs* s, const vdfgpu_gens* g) {
 void upload_constants_r1cs() { VDF_CUDA_CHECK(upload_field_constants()); }
 
 static fe host_one(int field) { return field == VDFGPU_FP ? Fp::one() : Fq::one(); }
+
+// every vdfgpu_running_* call that enqueues work: running_after() before its first operation on `st`,
+// running_done() after its last
+static void running_after(const vdfgpu_running* f, cudaStream_t st) { VDF_CUDA_CHECK(cudaStreamWaitEvent(st, f->done, 0)); }
+static void running_done(const vdfgpu_running* f, cudaStream_t st) { VDF_CUDA_CHECK(cudaEventRecord(f->done, st)); }
 
 // ---- satisfiability checks (vdfgpu_r1cs_is_sat_relaxed*, vdfgpu_running_check) ----------------------------------
 // counts2: the two u64 of the C ABI, as four u32 words on the device (see SatInitFn)
@@ -475,6 +483,7 @@ int vdfgpu_running_create(const vdfgpu_r1cs* s, vdfgpu_gens* gens, vdfgpu_runnin
       VDF_CUDA_CHECK(cudaMalloc((void**)&f->r, 32));
       VDF_CUDA_CHECK(cudaMalloc((void**)&f->comm, 2 * sizeof(jac_t)));
       VDF_CUDA_CHECK(cudaHostAlloc((void**)&f->bounce, 2 * sizeof(jac_t) + io1 * sizeof(fe), cudaHostAllocDefault));
+      VDF_CUDA_CHECK(cudaEventCreateWithFlags(&f->done, cudaEventDisableTiming));
     } catch (...) {
       if (f->bounce) cudaFreeHost(f->bounce);
       cudaFree(f->W); cudaFree(f->W2); cudaFree(f->E); cudaFree(f->T); cudaFree(f->uX); cudaFree(f->uX2);
@@ -498,6 +507,7 @@ int vdfgpu_running_destroy(vdfgpu_running* f) {
     f->shape->refs--;
     f->gens->refs--;
     cudaFreeHost(f->bounce);
+    cudaEventDestroy(f->done);
     cudaFree(f->W); cudaFree(f->W2); cudaFree(f->E); cudaFree(f->T); cudaFree(f->uX); cudaFree(f->uX2);
     cudaFree(f->r); cudaFree(f->comm);
     delete f;
@@ -510,12 +520,14 @@ int vdfgpu_running_set(vdfgpu_running* f, const void* W_host, const void* E_host
     if (!f || !W_host || !E_host || !u_host) throw ArgError("running_set: null pointer");
     if (f->shape->io && !X_host) throw ArgError("running_set: null X");
     require_ready();
-    Context& c = ctx();
-    h2d(f->W, W_host, (size_t)f->shape->vars * 32, cur_stream());
-    h2d(f->E, E_host, (size_t)f->shape->cons * 32, cur_stream());
-    h2d(f->uX, u_host, 32, cur_stream());
-    h2d(f->uX + 1, X_host, (size_t)f->shape->io * 32, cur_stream());
-    sync_after_unlock(cur_stream());
+    cudaStream_t st = cur_stream();
+    running_after(f, st);
+    h2d(f->W, W_host, (size_t)f->shape->vars * 32, st);
+    h2d(f->E, E_host, (size_t)f->shape->cons * 32, st);
+    h2d(f->uX, u_host, 32, st);
+    h2d(f->uX + 1, X_host, (size_t)f->shape->io * 32, st);
+    running_done(f, st);
+    sync_after_unlock(st);
     f->have_running = true;
     f->have_fresh = false;
   });
@@ -526,12 +538,14 @@ int vdfgpu_running_get(const vdfgpu_running* f, void* W_host, void* E_host, void
     if (!f) throw ArgError("running_get: null handle");
     if (!f->have_running) throw StateError("running_get: no running instance set");
     require_ready();
-    Context& c = ctx();
-    if (W_host) d2h(W_host, f->W, (size_t)f->shape->vars * 32, cur_stream());
-    if (E_host) d2h(E_host, f->E, (size_t)f->shape->cons * 32, cur_stream());
-    if (u_host) d2h(u_host, f->uX, 32, cur_stream());
-    if (X_host) d2h(X_host, f->uX + 1, (size_t)f->shape->io * 32, cur_stream());
-    sync_after_unlock(cur_stream());
+    cudaStream_t st = cur_stream();
+    running_after(f, st);
+    if (W_host) d2h(W_host, f->W, (size_t)f->shape->vars * 32, st);
+    if (E_host) d2h(E_host, f->E, (size_t)f->shape->cons * 32, st);
+    if (u_host) d2h(u_host, f->uX, 32, st);
+    if (X_host) d2h(X_host, f->uX + 1, (size_t)f->shape->io * 32, st);
+    running_done(f, st);
+    sync_after_unlock(st);
   });
 }
 
@@ -544,7 +558,9 @@ int vdfgpu_running_check(const vdfgpu_running* f, const void* comm_W96_host, con
     if (!f || !report4_host) throw ArgError("running_check: null pointer");
     if (!f->have_running) throw StateError("running_check: no running instance set");
     require_ready();
+    running_after(f, cur_stream());
     sat_enqueue(f->shape, f->gens, f->W, f->E, f->uX, comm_W96_host != nullptr, comm_E96_host != nullptr, res);
+    running_done(f, cur_stream());
   });
   return sat_report(rc, res, f ? f->gens : nullptr, comm_W96_host, comm_E96_host, report4_host);
 }
@@ -572,6 +588,7 @@ static void running_commit_enqueue(vdfgpu_running* f, void* comm_W2_point96_host
   const bool hn = host_normalise_wanted(f->gens);
   msm_batch_on_device(f->gens, vecs, lens, 2, f->comm, hn);
   d2h(f->bounce, f->comm, 2 * sizeof(jac_t), st);      // pinned: asynchronous, waited for outside the lock
+  running_done(f, st);
   sync_after_unlock(st);
   copy_after_sync(comm_W2_point96_host, f->bounce, sizeof(jac_t));
   copy_after_sync(comm_T_point96_host, f->bounce + sizeof(jac_t), sizeof(jac_t));
@@ -591,6 +608,7 @@ int vdfgpu_running_commit(vdfgpu_running* f, const void* W2_host, const void* X2
     require_ready();
     cudaStream_t st = cur_stream();
     const vdfgpu_r1cs* s = f->shape;
+    running_after(f, st);
     h2d(f->W2, W2_host, (size_t)s->vars * 32, st);
     upload_ux2(f, X2_host, st);
     running_commit_enqueue(f, comm_W2_point96_host, comm_T_point96_host);
@@ -686,6 +704,7 @@ int vdfgpu_running_commit_step(vdfgpu_running* f, const vdfgpu_witness_bank* ban
     require_ready();
     cudaStream_t st = cur_stream();
     const uint8_t* w2 = reinterpret_cast<const uint8_t*>(W2_host);
+    running_after(f, st);
     // W2 = [ host part | 4t+1 step variables from the bank | host part ]: the step range never crosses PCIe
     h2d(f->W2, w2, step_offset * 32, st);
     h2d(f->W2 + step_offset + per, w2 + (step_offset + per) * 32, (nv - step_offset - per) * 32, st);
@@ -702,17 +721,20 @@ int vdfgpu_running_finish(vdfgpu_running* f, const void* r32_host) {
     if (!f->have_fresh) throw StateError("running_finish: fold_commit has not been called for this step");
     require_ready();
     Context& c = ctx();
-    CudaLaunch L(cur_stream());
+    cudaStream_t st = cur_stream();
+    CudaLaunch L(st);
     const vdfgpu_r1cs* s = f->shape;
-    h2d(f->r, r32_host, 32, cur_stream());
+    running_after(f, st);
+    h2d(f->r, r32_host, 32, st);
     launch_fold(L, s->field, f->W, f->W2, s->vars, f->E, f->T, s->cons, f->r);
     // u <- u + r*1, X <- X + r*X2: the same kernel over the (1 + io)-element tail
     launch_fold(L, s->field, f->uX, f->uX2, 1 + (size_t)s->io, nullptr, nullptr, 0, f->r);
     c.launches += L.launches;
-    // No wait: the next call on this instance is ordered behind the fold on the stream.  Only a pinned r32_host would
-    // still be in flight after return (pageable copies are staged before cudaMemcpyAsync returns).
+    running_done(f, st);
+    // No wait: the next call on this instance, on any stream or thread, waits for f->done.  Only a pinned r32_host
+    // would still be in flight after return (pageable copies are staged before cudaMemcpyAsync returns).
     cudaPointerAttributes at;
-    if (cudaPointerGetAttributes(&at, r32_host) == cudaSuccess && at.type == cudaMemoryTypeHost) sync_after_unlock(cur_stream());
+    if (cudaPointerGetAttributes(&at, r32_host) == cudaSuccess && at.type == cudaMemoryTypeHost) sync_after_unlock(st);
     else cudaGetLastError();
     f->have_fresh = false;
   });
