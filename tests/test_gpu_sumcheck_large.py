@@ -240,27 +240,32 @@ def test_inner_product_and_vec_lincomb_lengths(gpu_lib, n):
 @pytest.mark.parametrize("cid", [O.CURVE_PALLAS, O.CURVE_VESTA])
 def test_points_lincomb_infinity_inside_a_chunk(gpu_lib, cid):
     """Outputs at infinity between finite outputs of one 4-output chunk (the batched inversion skips them), lengths
-    n = 1, 2, 3 (mod 4), weights 0, 1 and order - 1."""
+    n = 1, 2, 3 (mod 4), weights 0, 1 and order - 1.  Q = kP with k random, k = 1 (the precomputed P + Q doubles) and
+    k = -1 (P + Q is the identity); one P given as the identity with the x / y bytes of a real point, which the
+    infinity flag overrides."""
     cv = O.CURVES[cid]
     m = cv.order
     py = random.Random(70 + cid)
     for n in (9, 14, 23):
         P = [cv.mul(py.randrange(1, m), cv.gen) for _ in range(n)]
-        k = py.randrange(2, m)
-        Q = [cv.mul(py.randrange(1, m), cv.gen) for _ in range(n)]
-        for i in range(1, n, 4):          # Q = k P at positions 1, 5, 9, ...: w1 P + w2 Q = (w1 + k w2) P
-            Q[i] = cv.mul(k, P[i])
-        Q[n - 1] = cv.mul(k, P[n - 1])    # and the last output of the ragged last chunk
-        for w2 in (py.randrange(1, m), 1, m - 1):
-            w1 = (-k * w2) % m
-            got = SP.points_lincomb(cid, O.affines_to_bytes(cv, P), O.affines_to_bytes(cv, Q), w1, w2)
-            want = [cv.add(cv.mul(w1, p), cv.mul(w2, q)) for p, q in zip(P, Q)]
-            assert want[1] is None and want[0] is not None and want[2] is not None
-            assert [O.affine_from_bytes(cv, got[72 * i:72 * i + 72]) for i in range(n)] == want, (n, w2)
-        for w1, w2 in ((0, 1), (1, 0), (m - 1, 1), (0, 0)):
-            got = SP.points_lincomb(cid, O.affines_to_bytes(cv, P), O.affines_to_bytes(cv, Q), w1, w2)
-            want = [cv.add(cv.mul(w1, p), cv.mul(w2, q)) for p, q in zip(P, Q)]
-            assert [O.affine_from_bytes(cv, got[72 * i:72 * i + 72]) for i in range(n)] == want, (n, w1, w2)
+        junk = O.affine_to_bytes(cv, P[n - 3])[:64] + b"\x01" + bytes(7)
+        P[n - 3] = None
+        Pb = O.affines_to_bytes(cv, P[:n - 3]) + junk + O.affines_to_bytes(cv, P[n - 2:])
+        for k in (py.randrange(2, m), 1, m - 1):
+            Q = [cv.mul(py.randrange(1, m), cv.gen) for _ in range(n)]
+            for i in range(1, n, 4):          # Q = k P at positions 1, 5, 9, ...: w1 P + w2 Q = (w1 + k w2) P
+                Q[i] = cv.mul(k, P[i])
+            Q[n - 1] = cv.mul(k, P[n - 1])    # and the last output of the ragged last chunk
+            for w2 in (py.randrange(1, m), 1, m - 1):
+                w1 = (-k * w2) % m
+                got = SP.points_lincomb(cid, Pb, O.affines_to_bytes(cv, Q), w1, w2)
+                want = [cv.add(cv.mul(w1, p), cv.mul(w2, q)) for p, q in zip(P, Q)]
+                assert want[1] is None and want[0] is not None and want[2] is not None
+                assert [O.affine_from_bytes(cv, got[72 * i:72 * i + 72]) for i in range(n)] == want, (n, k, w2)
+            for w1, w2 in ((0, 1), (1, 0), (m - 1, 1), (0, 0)):
+                got = SP.points_lincomb(cid, Pb, O.affines_to_bytes(cv, Q), w1, w2)
+                want = [cv.add(cv.mul(w1, p), cv.mul(w2, q)) for p, q in zip(P, Q)]
+                assert [O.affine_from_bytes(cv, got[72 * i:72 * i + 72]) for i in range(n)] == want, (n, k, w1, w2)
 
 
 def _interp(points, r, m):
