@@ -48,6 +48,13 @@ static const Mod FQ_MOD = {{0x8c46eb2100000001ull, 0x224698fc0994a8ddull, 0x0000
                            {0x5b2b3e9cfffffffdull, 0x992c350be3420567ull, 0xffffffffffffffffull, 0x3fffffffffffffffull},
                            0x8c46eb20ffffffffull};
 
+static const Mod& mod_of(Fp) { return FP_MOD; }
+static const Mod& mod_of(Fq) { return FQ_MOD; }
+// the coordinate field of `curve`
+static const Mod& coord_mod(int curve) {
+  return with_curve(curve, "point_normalise_host", [](auto, auto f, auto) -> const Mod& { return mod_of(f); });
+}
+
 static void mul(uint64_t* r, const uint64_t* a, const uint64_t* b, const Mod& f) {   // Montgomery CIOS, 4 x 64
   uint64_t t[6] = {0, 0, 0, 0, 0, 0};
   for (int i = 0; i < 4; i++) {
@@ -79,7 +86,7 @@ static void inv(uint64_t* r, const uint64_t* a, const Mod& f) {   // a^(m-2)
 
 // (X, Y, Z) Jacobian, Montgomery limbs -> (X / Z^2, Y / Z^3, 1), or all zero for the identity
 static void normalise(uint8_t* p96, int curve) {
-  const Mod& f = curve == VDFGPU_PALLAS ? FP_MOD : FQ_MOD;
+  const Mod& f = coord_mod(curve);
   uint64_t X[4], Y[4], Z[4];
   std::memcpy(X, p96, 32); std::memcpy(Y, p96 + 32, 32); std::memcpy(Z, p96 + 64, 32);
   if ((Z[0] | Z[1] | Z[2] | Z[3]) == 0) {
@@ -97,7 +104,7 @@ static void normalise(uint8_t* p96, int curve) {
 
 // the same for m <= 16 points with one inversion: 1 / (Z_0 ... Z_{m-1}), then the individual inverses by back-substitution
 static void normalise_batch(uint8_t* const* pts, size_t m, int curve) {
-  const Mod& f = curve == VDFGPU_PALLAS ? FP_MOD : FQ_MOD;
+  const Mod& f = coord_mod(curve);
   uint64_t Z[16][4], pre[16][4], run[4];
   std::memcpy(run, f.one, 32);
   for (size_t k = 0; k < m; k++) {
@@ -449,7 +456,9 @@ static size_t msm_workspace_bytes(const MsmPlan& p) {
 }
 
 static size_t plan_bytes(int curve, const MsmPlan& p) {
-  return curve == VDFGPU_PALLAS ? msm_workspace_bytes<Pallas, Fq>(p) : msm_workspace_bytes<Vesta, Fp>(p);
+  return with_curve(curve, "msm", [&](auto C, auto, auto SF) {
+    return msm_workspace_bytes<decltype(C), decltype(SF)>(p);
+  });
 }
 
 // Workspace for one MSM on stream `s`.  The affine rounds need ~52 B per sorted entry on top of the sort's 12 B:
@@ -491,9 +500,8 @@ static void msm_dispatch(vdfgpu_gens* g, const MsmPlan& p, Workspace* w, cudaStr
   Context& c = ctx();
   const size_t E = (size_t)p.n * p.W * p.batch;
   if (!w || !graphs_enabled() || c.prof.enabled || E > GRAPH_MAX_ENTRIES) {
-    CudaLaunch L(st, &c.prof, w ? &w->arena : nullptr);
+    CudaLaunch L = api_launch(st, &c.prof, w ? &w->arena : nullptr);
     enqueue(L);
-    c.launches += L.launches;
     return;
   }
   std::vector<uint64_t> key = {(uint64_t)g->curve, p.n, p.c, p.W, p.B, p.NB, p.table, p.level_stride, p.S, p.G, p.logm, p.is_mont, p.batch,
@@ -513,7 +521,8 @@ static void msm_dispatch(vdfgpu_gens* g, const MsmPlan& p, Workspace* w, cudaStr
       c.graph_replays++;
       return;
     }
-  // capture (the arena is already large enough: nothing below allocates device memory)
+  // capture (the arena is already large enough: nothing below allocates device memory); its launches count when
+  // the graph runs
   cudaGraph_t graph = nullptr;
   CudaLaunch L(st, nullptr, &w->arena);
   VDF_CUDA_CHECK(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
@@ -561,10 +570,10 @@ void msm_on_device(vdfgpu_gens* g, size_t first, const fe* d_scalars, size_t n, 
   Workspace* w = n ? plan_workspace(g->curve, p, st) : nullptr;
   const affine_t* pts = g->pts + first;
   ScalarSet ss{{d_scalars, nullptr, nullptr, nullptr}};
-  const int curve = g->curve;
   msm_dispatch(g, p, w, st, ss, pts, d_out, [&](CudaLaunch& L) {
-    if (curve == VDFGPU_PALLAS) msm_run<CudaLaunch, Pallas, Fq>(L, p, pts, ss, d_out);
-    else msm_run<CudaLaunch, Vesta, Fp>(L, p, pts, ss, d_out);
+    with_curve(g->curve, "msm", [&](auto C, auto, auto SF) {
+      msm_run<CudaLaunch, decltype(C), decltype(SF)>(L, p, pts, ss, d_out);
+    });
   });
 }
 
@@ -575,7 +584,7 @@ void msm_host_chunked(vdfgpu_gens* g, const void* h_scalars, size_t n, jac_t* d_
   Context& c = ctx();
   cudaStream_t st = cur_stream();
   c.prof.n_marks = 0;
-  CudaLaunch L(st, nullptr);
+  CudaLaunch L = api_launch(st);
   MsmPlan full = make_plan(g, n, true);
   check_refs(full, g, n);
   const size_t NBK = (size_t)full.NB * full.B;
@@ -591,28 +600,24 @@ void msm_host_chunked(vdfgpu_gens* g, const void* h_scalars, size_t n, jac_t* d_
                                             cudaMemcpyHostToDevice, c.copy_stream));
     VDF_CUDA_CHECK(cudaEventRecord(c.chunk_ev[k], c.copy_stream));
   }
-  for (int k = 0; k < chunks; k++) {
-    size_t lo = (size_t)k * per, len = lo < n ? (lo + per <= n ? per : n - lo) : 0;
-    VDF_CUDA_CHECK(cudaStreamWaitEvent(st, c.chunk_ev[k], 0));
-    if (!len) continue;
-    MsmPlan p = full;
-    p.n = (uint32_t)len;
-    p.len[0] = (uint32_t)len;
-    ScalarSet ss{{d_scalars + lo, nullptr, nullptr, nullptr}};
-    const affine_t* pts = g->pts + lo;
-    xyzz_t* dst = k ? chunk_buckets.p : buckets.p;
-    if (k) L.zero(dst, NBK * sizeof(xyzz_t));
-    if (g->curve == VDFGPU_PALLAS) {
-      msm_accumulate<CudaLaunch, Pallas, Fq>(L, p, pts, ss, dst);
-      if (k) msm_merge_buckets<CudaLaunch, Pallas>(L, full, buckets.p, chunk_buckets.p);
-    } else {
-      msm_accumulate<CudaLaunch, Vesta, Fp>(L, p, pts, ss, dst);
-      if (k) msm_merge_buckets<CudaLaunch, Vesta>(L, full, buckets.p, chunk_buckets.p);
+  with_curve(g->curve, "msm", [&](auto C, auto, auto SF) {
+    using Cv = decltype(C);
+    for (int k = 0; k < chunks; k++) {
+      size_t lo = (size_t)k * per, len = lo < n ? (lo + per <= n ? per : n - lo) : 0;
+      VDF_CUDA_CHECK(cudaStreamWaitEvent(st, c.chunk_ev[k], 0));
+      if (!len) continue;
+      MsmPlan p = full;
+      p.n = (uint32_t)len;
+      p.len[0] = (uint32_t)len;
+      ScalarSet ss{{d_scalars + lo, nullptr, nullptr, nullptr}};
+      const affine_t* pts = g->pts + lo;
+      xyzz_t* dst = k ? chunk_buckets.p : buckets.p;
+      if (k) L.zero(dst, NBK * sizeof(xyzz_t));
+      msm_accumulate<CudaLaunch, Cv, decltype(SF)>(L, p, pts, ss, dst);
+      if (k) msm_merge_buckets<CudaLaunch, Cv>(L, full, buckets.p, chunk_buckets.p);
     }
-  }
-  if (g->curve == VDFGPU_PALLAS) msm_finish<CudaLaunch, Pallas>(L, full, buckets.p, d_out);
-  else msm_finish<CudaLaunch, Vesta>(L, full, buckets.p, d_out);
-  c.launches += L.launches;
+    msm_finish<CudaLaunch, Cv>(L, full, buckets.p, d_out);
+  });
 }
 
 // k scalar vectors over the same generators in ONE pass of the pipeline (one bucket set per vector):
@@ -637,11 +642,11 @@ void msm_batch_on_device(vdfgpu_gens* g, const fe* const* d_scalars, const size_
     p.len[j] = (uint32_t)lens[j];
   }
   Workspace* w = n ? plan_workspace(g->curve, p, st) : nullptr;
-  const int curve = g->curve;
   const affine_t* pts = g->pts;
   msm_dispatch(g, p, w, st, ss, pts, d_out, [&](CudaLaunch& L) {
-    if (curve == VDFGPU_PALLAS) msm_run<CudaLaunch, Pallas, Fq>(L, p, pts, ss, d_out);
-    else msm_run<CudaLaunch, Vesta, Fp>(L, p, pts, ss, d_out);
+    with_curve(g->curve, "msm", [&](auto C, auto, auto SF) {
+      msm_run<CudaLaunch, decltype(C), decltype(SF)>(L, p, pts, ss, d_out);
+    });
   });
 }
 
@@ -651,31 +656,56 @@ static void build_table(vdfgpu_gens* g, CudaLaunch& L) {
     const affine_t* prev = g->pts + (size_t)(l - 1) * g->n;
     affine_t* next = g->pts + (size_t)l * g->n;
     size_t threads = (g->n + 7) / 8;
-    if (g->curve == VDFGPU_PALLAS) L.run<128>(threads, TableLevelFn<Pallas, Fp>{prev, next, g->n, g->c});
-    else L.run<128>(threads, TableLevelFn<Vesta, Fq>{prev, next, g->n, g->c});
+    with_curve(g->curve, "gens", [&](auto C, auto BF, auto) {
+      L.run<128>(threads, TableLevelFn<decltype(C), decltype(BF)>{prev, next, g->n, g->c});
+    });
   }
 }
 
-static vdfgpu_gens* gens_alloc(int curve, size_t n, uint32_t flags, uint32_t window_bits) {
-  if (curve != VDFGPU_PALLAS && curve != VDFGPU_VESTA) throw ArgError("gens: unknown curve");
+// the arguments of a new generator set, checked before any device work
+static void gens_check(int curve, size_t n, uint32_t window_bits) {
+  with_curve(curve, "gens", [](auto, auto, auto) {});
   if (n == 0) throw ArgError("gens: empty generator set");
   if (window_bits != 0 && (window_bits < 2 || window_bits > 24)) throw ArgError("gens: window_bits out of range");
-  vdfgpu_gens* g = new vdfgpu_gens();
+}
+
+// the one release path of a generator set: failed creation, drop-in eviction, vdfgpu_gens_destroy
+struct GensRelease {
+  void operator()(vdfgpu_gens* g) const {
+    graphs_drop_if(nullptr, g->pts);
+    cudaFree(g->pts);
+    delete g;
+  }
+};
+using GensPtr = std::unique_ptr<vdfgpu_gens, GensRelease>;
+
+static GensPtr gens_alloc(int curve, size_t n, uint32_t flags, uint32_t window_bits) {
+  const bool table = flags & VDFGPU_GENS_TABLE;
+  if (!window_bits) window_bits = (uint32_t)env_long("VDFGPU_WINDOW_BITS", 0, 0, 24);   // tuning knob; 0 = by size
+  if (window_bits == 1) window_bits = 2;
+  const uint32_t c = window_bits ? window_bits : msm_pick_c(n, table), W = table ? msm_windows(c) : 1;
+  void* p = nullptr;
+  cudaError_t e = cudaMalloc(&p, (size_t)W * n * sizeof(affine_t));
+  if (e != cudaSuccess) throw std::runtime_error(std::string("gens: cudaMalloc failed: ") + cudaGetErrorString(e));
+  GensPtr g(new vdfgpu_gens());
   g->curve = curve;
   g->n = n;
   g->flags = flags;
-  bool table = flags & VDFGPU_GENS_TABLE;
-  if (!window_bits) window_bits = (uint32_t)env_long("VDFGPU_WINDOW_BITS", 0, 0, 24);   // tuning knob; 0 = by size
-  if (window_bits == 1) window_bits = 2;
-  g->c = window_bits ? window_bits : msm_pick_c(n, table);
-  g->W = table ? msm_windows(g->c) : 1;
-  void* p = nullptr;
-  cudaError_t e = cudaMalloc(&p, (size_t)g->W * n * sizeof(affine_t));
-  if (e != cudaSuccess) {
-    delete g;
-    throw std::runtime_error(std::string("gens: cudaMalloc failed: ") + cudaGetErrorString(e));
-  }
+  g->c = c;
+  g->W = W;
   g->pts = reinterpret_cast<affine_t*>(p);
+  return g;
+}
+
+// a resident set of the caller's 72-byte affine points (vdfgpu_gens_create, the drop-in cache)
+static GensPtr gens_upload(int curve, const void* points72_host, size_t n, uint32_t flags, uint32_t window_bits,
+                           cudaStream_t st) {
+  GensPtr g = gens_alloc(curve, n, flags, window_bits);
+  CudaLaunch L = api_launch(st);
+  DevBuf<uint8_t> raw(n * 72, st);
+  h2d(raw.p, points72_host, n * 72, st);
+  L.run<256>(n, RepackFn{raw.p, g->pts});
+  if (flags & VDFGPU_GENS_TABLE) build_table(g.get(), L);
   return g;
 }
 
@@ -890,23 +920,11 @@ int vdfgpu_gens_create(int curve, const void* points_affine72_host, size_t n, ui
                        uint32_t window_bits, vdfgpu_gens** out) {
   return guarded([&] {
     if (!out || !points_affine72_host) throw ArgError("gens_create: null pointer");
+    gens_check(curve, n, window_bits);
     require_ready();
-    Context& c = ctx();
-    vdfgpu_gens* g = gens_alloc(curve, n, flags, window_bits);
-    try {
-      CudaLaunch L(cur_stream());
-      DevBuf<uint8_t> raw(n * 72, cur_stream());
-      h2d(raw.p, points_affine72_host, n * 72, cur_stream());
-      L.run<256>(n, RepackFn{raw.p, g->pts});
-      if (flags & VDFGPU_GENS_TABLE) build_table(g, L);
-      c.launches += L.launches;
-      sync_after_unlock(cur_stream());
-    } catch (...) {
-      cudaFree(g->pts);
-      delete g;
-      throw;
-    }
-    *out = g;
+    GensPtr g = gens_upload(curve, points_affine72_host, n, flags, window_bits, cur_stream());
+    sync_after_unlock(cur_stream());
+    *out = g.release();
   });
 }
 
@@ -914,33 +932,23 @@ int vdfgpu_gens_progression(int curve, const void* k0_le32, const void* d_le32, 
                             uint32_t window_bits, vdfgpu_gens** out) {
   return guarded([&] {
     if (!out || !k0_le32 || !d_le32) throw ArgError("gens_progression: null pointer");
+    gens_check(curve, n, window_bits);
+    const size_t threads = (n + PROG_CH - 1) / PROG_CH;
+    if (threads >= (1ull << 32)) throw ArgError("gens_progression: n too large");
     require_ready();
-    Context& c = ctx();
-    vdfgpu_gens* g = gens_alloc(curve, n, flags, window_bits);
-    try {
-      CudaLaunch L(cur_stream());
-      fe k0, d;
-      std::memcpy(k0.v, k0_le32, 32);
-      std::memcpy(d.v, d_le32, 32);
-      DevBuf<ProgSetup> setup(1, cur_stream());
-      size_t threads = (n + PROG_CH - 1) / PROG_CH;
-      if (threads >= (1ull << 32)) throw ArgError("gens_progression: n too large");
-      if (curve == VDFGPU_PALLAS) {
-        L.run<32>(1, ProgressionSetupFn<Pallas, Fp>{k0, d, setup.p});
-        L.run<128>(threads, ProgressionFn<Pallas, Fp>{setup.p, g->pts, n});
-      } else {
-        L.run<32>(1, ProgressionSetupFn<Vesta, Fq>{k0, d, setup.p});
-        L.run<128>(threads, ProgressionFn<Vesta, Fq>{setup.p, g->pts, n});
-      }
-      if (flags & VDFGPU_GENS_TABLE) build_table(g, L);
-      c.launches += L.launches;
-      sync_after_unlock(cur_stream());
-    } catch (...) {
-      cudaFree(g->pts);
-      delete g;
-      throw;
-    }
-    *out = g;
+    GensPtr g = gens_alloc(curve, n, flags, window_bits);
+    CudaLaunch L = api_launch(cur_stream());
+    fe k0, d;
+    std::memcpy(k0.v, k0_le32, 32);
+    std::memcpy(d.v, d_le32, 32);
+    DevBuf<ProgSetup> setup(1, cur_stream());
+    with_curve(curve, "gens", [&](auto C, auto BF, auto) {
+      L.run<32>(1, ProgressionSetupFn<decltype(C), decltype(BF)>{k0, d, setup.p});
+      L.run<128>(threads, ProgressionFn<decltype(C), decltype(BF)>{setup.p, g->pts, n});
+    });
+    if (flags & VDFGPU_GENS_TABLE) build_table(g.get(), L);
+    sync_after_unlock(cur_stream());
+    *out = g.release();
   });
 }
 
@@ -949,12 +957,10 @@ int vdfgpu_gens_export(const vdfgpu_gens* g, size_t first, size_t count, void* p
     if (!g || !points_affine72_host) throw ArgError("gens_export: null pointer");
     if (first + count > (size_t)g->W * g->n) throw ArgError("gens_export: range out of bounds");
     require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
+    CudaLaunch L = api_launch(cur_stream());
     DevBuf<uint8_t> raw(count * 72, cur_stream());
     L.run<256>(count, UnpackFn{g->pts + first, raw.p});
     d2h(points_affine72_host, raw.p, count * 72, cur_stream());
-    c.launches += L.launches;
     sync_after_unlock(cur_stream());
   });
 }
@@ -978,10 +984,8 @@ int vdfgpu_gens_destroy(vdfgpu_gens* g) {
     if (ctx().ready) {
       VDF_CUDA_CHECK(cudaSetDevice(ctx().device));
       cudaDeviceSynchronize();   // MSMs on any stream (asynchronous slots, other threads) may still read the points
-      graphs_drop_if(nullptr, g->pts);
     }
-    cudaFree(g->pts);
-    delete g;
+    GensRelease()(g);
   });
 }
 
@@ -1106,28 +1110,25 @@ int vdfgpu_msm_range_dev(vdfgpu_gens* g, size_t first, const void* scalars32_dev
 int vdfgpu_point_sum(int curve, const void* points96_host, size_t k, void* out_point96_host) {
   return guarded([&] {
     if (!out_point96_host || (k && !points96_host)) throw ArgError("point_sum: null pointer");
-    if (curve != VDFGPU_PALLAS && curve != VDFGPU_VESTA) throw ArgError("point_sum: unknown curve");
-    require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
-    DevBuf<jac_t> in(k ? k : 1, cur_stream());
-    DevBuf<jac_t> res(1, cur_stream());
-    h2d(in.p, points96_host, k * sizeof(jac_t), cur_stream());
-    if (curve == VDFGPU_PALLAS) L.run<32>(32, JacSumFn<Pallas>{in.p, (uint32_t)k, res.p});
-    else L.run<32>(32, JacSumFn<Vesta>{in.p, (uint32_t)k, res.p});
-    d2h(out_point96_host, res.p, sizeof(jac_t), cur_stream());
-    c.launches += L.launches;
-    sync_after_unlock(cur_stream());
+    with_curve(curve, "point_sum", [&](auto C, auto, auto) {
+      require_ready();
+      CudaLaunch L = api_launch(cur_stream());
+      DevBuf<jac_t> in(k ? k : 1, cur_stream());
+      DevBuf<jac_t> res(1, cur_stream());
+      h2d(in.p, points96_host, k * sizeof(jac_t), cur_stream());
+      L.run<32>(32, JacSumFn<decltype(C)>{in.p, (uint32_t)k, res.p});
+      d2h(out_point96_host, res.p, sizeof(jac_t), cur_stream());
+      sync_after_unlock(cur_stream());
+    });
   });
 }
 
 int vdfgpu_point_normalise_host(int curve, void* points96_host, size_t count) {
-  if (curve != VDFGPU_PALLAS && curve != VDFGPU_VESTA) {
-    set_error("point_normalise_host: unknown curve");
-    return VDFGPU_ERR_ARG;
-  }
-  if (count && !points96_host) {
-    set_error("point_normalise_host: null pointer");
+  try {   // host arithmetic only: no device, no lock
+    hostfield::coord_mod(curve);   // ArgError for an unknown curve
+    if (count && !points96_host) throw ArgError("point_normalise_host: null pointer");
+  } catch (const ArgError& e) {
+    set_error(e.what());
     return VDFGPU_ERR_ARG;
   }
   for (size_t k = 0; k < count;) {   // 16 points per inversion
@@ -1143,15 +1144,12 @@ int vdfgpu_point_normalise_host(int curve, void* points96_host, size_t count) {
 int vdfgpu_point_sum_dev(int curve, const void* points96_dev, size_t k, void* out_point96_dev) {
   return guarded([&] {
     if (!out_point96_dev || (k && !points96_dev)) throw ArgError("point_sum_dev: null pointer");
-    if (curve != VDFGPU_PALLAS && curve != VDFGPU_VESTA) throw ArgError("point_sum_dev: unknown curve");
-    require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
-    const jac_t* in = reinterpret_cast<const jac_t*>(points96_dev);
-    jac_t* out = reinterpret_cast<jac_t*>(out_point96_dev);
-    if (curve == VDFGPU_PALLAS) L.run<32>(32, JacSumFn<Pallas>{in, (uint32_t)k, out});
-    else L.run<32>(32, JacSumFn<Vesta>{in, (uint32_t)k, out});
-    c.launches += L.launches;
+    with_curve(curve, "point_sum_dev", [&](auto C, auto, auto) {
+      require_ready();
+      CudaLaunch L = api_launch(cur_stream());
+      L.run<32>(32, JacSumFn<decltype(C)>{reinterpret_cast<const jac_t*>(points96_dev), (uint32_t)k,
+                                          reinterpret_cast<jac_t*>(out_point96_dev)});
+    });
   });
 }
 
@@ -1201,12 +1199,8 @@ static int dropin_verify_mode() {   // 0 off, 1 sample, 2 full
 }
 
 static void dropin_drop(DropinEntry& e) {
-  if (e.gens) {
-    graphs_drop_if(nullptr, e.gens->pts);
-    cudaFree(e.gens->pts);
-    delete e.gens;
-    e.gens = nullptr;
-  }
+  if (e.gens) GensRelease()(e.gens);
+  e.gens = nullptr;
 }
 
 static void dropin_clear_locked() {
@@ -1267,20 +1261,7 @@ static vdfgpu_gens* dropin_lookup(int curve, const void* points, size_t npoints)
   if ((uint64_t)msm_windows(c_bits) * npoints >= (1ull << 31) ||
       (size_t)msm_windows(c_bits) * npoints * sizeof(affine_t) > free_b / 3)
     flags = 0;
-  vdfgpu_gens* g = gens_alloc(curve, npoints, flags, 0);
-  cudaStream_t st = cur_stream();
-  try {
-    CudaLaunch L(st);
-    DevBuf<uint8_t> raw(npoints * 72, st);
-    h2d(raw.p, points, npoints * 72, st);
-    L.run<256>(npoints, RepackFn{raw.p, g->pts});
-    if (flags & VDFGPU_GENS_TABLE) build_table(g, L);
-    c.launches += L.launches;
-  } catch (...) {
-    cudaFree(g->pts);
-    delete g;
-    throw;
-  }
+  GensPtr g = gens_upload(curve, points, npoints, flags, 0, cur_stream());
   DropinEntry e;
   e.curve = curve;
   e.host_ptr = points;
@@ -1290,16 +1271,15 @@ static vdfgpu_gens* dropin_lookup(int curve, const void* points, size_t npoints)
   for (size_t k = 0; k < e.sample_idx.size(); k++)
     std::memcpy(&e.sample_bytes[k * 65], pts72 + e.sample_idx[k] * 72, 65);
   if (mode == 2) e.full_hash = dropin_full_hash(pts72, npoints);
-  e.gens = g;
+  e.gens = g.release();
   e.last_use = ++c.tick;
   c.dropin.push_back(std::move(e));
-  return g;
+  return c.dropin.back().gens;
 }
 
 static void mult_pippenger_body(int curve, void* out, const void* points, size_t npoints, const void* scalars,
                                 bool is_mont) {
   require_ready();
-  Context& c = ctx();
   cudaStream_t st = cur_stream();
   if (workspaces_enabled()) {
     if (vdfgpu_gens* cached = dropin_lookup(curve, points, npoints)) {
@@ -1324,12 +1304,11 @@ static void mult_pippenger_body(int curve, void* out, const void* points, size_t
     g.n = npoints;
     g.flags = 0;
     g.W = 1;
-    CudaLaunch L(st);
+    CudaLaunch L = api_launch(st);
     DevBuf<uint8_t> raw(npoints * 72, st);
     DevBuf<affine_t> pts(npoints, st);
     h2d(raw.p, points, npoints * 72, st);
     L.run<256>(npoints, RepackFn{raw.p, pts.p});
-    c.launches += L.launches;
     g.pts = pts.p;
     msm_on_device(&g, 0, sc.p, npoints, res.p, is_mont);
   }
@@ -1393,77 +1372,68 @@ int vdfgpu_minroot_check_batch_dev(int field, const void* results_dev, const voi
                                    const uint64_t* t_each_dev, uint64_t t_uniform, size_t n,
                                    uint8_t* ok_out_dev) {
   return guarded([&] {
-    if (field != VDFGPU_FP && field != VDFGPU_FQ) throw ArgError("minroot_check: unknown field");
-    if (n && (!results_dev || !originals_dev || !ok_out_dev)) throw ArgError("minroot_check: null pointer");
-    require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
-    if (field == VDFGPU_FP) minroot_check_dispatch<Fp>(L, results_dev, originals_dev, t_each_dev, t_uniform, n, ok_out_dev);
-    else minroot_check_dispatch<Fq>(L, results_dev, originals_dev, t_each_dev, t_uniform, n, ok_out_dev);
-    c.launches += L.launches;
+    with_field(field, "minroot_check", [&](auto f) {
+      if (n && (!results_dev || !originals_dev || !ok_out_dev)) throw ArgError("minroot_check: null pointer");
+      require_ready();
+      CudaLaunch L = api_launch(cur_stream());
+      minroot_check_dispatch<decltype(f)>(L, results_dev, originals_dev, t_each_dev, t_uniform, n, ok_out_dev);
+    });
   });
 }
 
 int vdfgpu_minroot_check_batch(int field, const void* results_host, const void* originals_host,
                                const uint64_t* t_each, uint64_t t_uniform, size_t n, uint8_t* ok_out_host) {
   return guarded([&] {
-    if (field != VDFGPU_FP && field != VDFGPU_FQ) throw ArgError("minroot_check: unknown field");
-    if (n && (!results_host || !originals_host || !ok_out_host)) throw ArgError("minroot_check: null pointer");
-    if (n == 0) return;
-    require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
-    DevBuf<state_t> res(n, cur_stream()), orig(n, cur_stream());
-    DevBuf<uint64_t> tt(t_each ? n : 1, cur_stream());
-    DevBuf<uint8_t> ok(n, cur_stream());
-    h2d(res.p, results_host, n * sizeof(state_t), cur_stream());
-    h2d(orig.p, originals_host, n * sizeof(state_t), cur_stream());
-    if (t_each) h2d(tt.p, t_each, n * 8, cur_stream());
-    const uint64_t* tp = t_each ? tt.p : nullptr;
-    if (field == VDFGPU_FP) minroot_check_dispatch<Fp>(L, res.p, orig.p, tp, t_uniform, n, ok.p);
-    else minroot_check_dispatch<Fq>(L, res.p, orig.p, tp, t_uniform, n, ok.p);
-    d2h(ok_out_host, ok.p, n, cur_stream());
-    c.launches += L.launches;
-    sync_after_unlock(cur_stream());
+    with_field(field, "minroot_check", [&](auto f) {
+      if (n && (!results_host || !originals_host || !ok_out_host)) throw ArgError("minroot_check: null pointer");
+      if (n == 0) return;
+      require_ready();
+      CudaLaunch L = api_launch(cur_stream());
+      DevBuf<state_t> res(n, cur_stream()), orig(n, cur_stream());
+      DevBuf<uint64_t> tt(t_each ? n : 1, cur_stream());
+      DevBuf<uint8_t> ok(n, cur_stream());
+      h2d(res.p, results_host, n * sizeof(state_t), cur_stream());
+      h2d(orig.p, originals_host, n * sizeof(state_t), cur_stream());
+      if (t_each) h2d(tt.p, t_each, n * 8, cur_stream());
+      minroot_check_dispatch<decltype(f)>(L, res.p, orig.p, t_each ? tt.p : nullptr, t_uniform, n, ok.p);
+      d2h(ok_out_host, ok.p, n, cur_stream());
+      sync_after_unlock(cur_stream());
+    });
   });
 }
 
 int vdfgpu_minroot_inverse_eval_batch(int field, const void* results_host, uint64_t t, size_t n,
                                       void* out_host) {
   return guarded([&] {
-    if (field != VDFGPU_FP && field != VDFGPU_FQ) throw ArgError("minroot_inverse_eval: unknown field");
-    if (n && (!results_host || !out_host)) throw ArgError("minroot_inverse_eval: null pointer");
-    if (n == 0) return;
-    require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
-    DevBuf<state_t> res(n, cur_stream()), out(n, cur_stream());
-    h2d(res.p, results_host, n * sizeof(state_t), cur_stream());
-    if (field == VDFGPU_FP) L.run<128>(n, MinRootInverseEvalFn<Fp>{res.p, t, out.p});
-    else L.run<128>(n, MinRootInverseEvalFn<Fq>{res.p, t, out.p});
-    d2h(out_host, out.p, n * sizeof(state_t), cur_stream());
-    c.launches += L.launches;
-    sync_after_unlock(cur_stream());
+    with_field(field, "minroot_inverse_eval", [&](auto f) {
+      if (n && (!results_host || !out_host)) throw ArgError("minroot_inverse_eval: null pointer");
+      if (n == 0) return;
+      require_ready();
+      CudaLaunch L = api_launch(cur_stream());
+      DevBuf<state_t> res(n, cur_stream()), out(n, cur_stream());
+      h2d(res.p, results_host, n * sizeof(state_t), cur_stream());
+      L.run<128>(n, MinRootInverseEvalFn<decltype(f)>{res.p, t, out.p});
+      d2h(out_host, out.p, n * sizeof(state_t), cur_stream());
+      sync_after_unlock(cur_stream());
+    });
   });
 }
 
 int vdfgpu_minroot_witness_batch(int field, const void* results_host, uint64_t t, size_t n, void* out_host) {
   return guarded([&] {
-    if (field != VDFGPU_FP && field != VDFGPU_FQ) throw ArgError("minroot_witness: unknown field");
-    if (n && (!results_host || !out_host)) throw ArgError("minroot_witness: null pointer");
-    if (n == 0) return;
-    require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
-    const size_t per = 4 * (size_t)t + 1;
-    DevBuf<state_t> res(n, cur_stream());
-    DevBuf<fe> out(n * per, cur_stream());
-    h2d(res.p, results_host, n * sizeof(state_t), cur_stream());
-    if (field == VDFGPU_FP) L.run<128>(n, MinRootWitnessFn<Fp>{res.p, t, out.p});
-    else L.run<128>(n, MinRootWitnessFn<Fq>{res.p, t, out.p});
-    d2h(out_host, out.p, n * per * 32, cur_stream());
-    c.launches += L.launches;
-    sync_after_unlock(cur_stream());
+    with_field(field, "minroot_witness", [&](auto f) {
+      if (n && (!results_host || !out_host)) throw ArgError("minroot_witness: null pointer");
+      if (n == 0) return;
+      require_ready();
+      CudaLaunch L = api_launch(cur_stream());
+      const size_t per = 4 * (size_t)t + 1;
+      DevBuf<state_t> res(n, cur_stream());
+      DevBuf<fe> out(n * per, cur_stream());
+      h2d(res.p, results_host, n * sizeof(state_t), cur_stream());
+      L.run<128>(n, MinRootWitnessFn<decltype(f)>{res.p, t, out.p});
+      d2h(out_host, out.p, n * per * 32, cur_stream());
+      sync_after_unlock(cur_stream());
+    });
   });
 }
 
@@ -1471,32 +1441,29 @@ int vdfgpu_minroot_witness_batch(int field, const void* results_host, uint64_t t
 int vdfgpu_field_mul_batch(int field, const void* a_host, const void* b_host, size_t n, uint32_t iters,
                            void* out_host) {
   return guarded([&] {
-    if (field != VDFGPU_FP && field != VDFGPU_FQ) throw ArgError("field_mul_batch: unknown field");
-    if (n && (!a_host || !b_host || !out_host)) throw ArgError("field_mul_batch: null pointer");
-    if (n == 0) return;
-    require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
-    DevBuf<fe> a(n, cur_stream()), b(n, cur_stream()), o(n, cur_stream());
-    h2d(a.p, a_host, n * 32, cur_stream());
-    h2d(b.p, b_host, n * 32, cur_stream());
-    if (field == VDFGPU_FP) L.run<256>(n, FieldMulFn<Fp>{a.p, b.p, o.p, iters});
-    else L.run<256>(n, FieldMulFn<Fq>{a.p, b.p, o.p, iters});
-    d2h(out_host, o.p, n * 32, cur_stream());
-    c.launches += L.launches;
-    sync_after_unlock(cur_stream());
+    with_field(field, "field_mul_batch", [&](auto f) {
+      if (n && (!a_host || !b_host || !out_host)) throw ArgError("field_mul_batch: null pointer");
+      if (n == 0) return;
+      require_ready();
+      CudaLaunch L = api_launch(cur_stream());
+      DevBuf<fe> a(n, cur_stream()), b(n, cur_stream()), o(n, cur_stream());
+      h2d(a.p, a_host, n * 32, cur_stream());
+      h2d(b.p, b_host, n * 32, cur_stream());
+      L.run<256>(n, FieldMulFn<decltype(f)>{a.p, b.p, o.p, iters});
+      d2h(out_host, o.p, n * 32, cur_stream());
+      sync_after_unlock(cur_stream());
+    });
   });
 }
 
 int vdfgpu_imad_peak(double* mul32_per_s_wide, double* imad_per_s_lo, double* iadd3_per_s) {
   return guarded([&] {
     require_ready();
-    Context& c = ctx();
     DevBuf<uint32_t> sink(4, cur_stream());
     double w = probe_rate<0>(cur_stream(), sink.p);
     double l = probe_rate<1>(cur_stream(), sink.p);
     double a = probe_rate<2>(cur_stream(), sink.p);
-    c.launches += 9;
+    ctx().launches += 9;
     if (mul32_per_s_wide) *mul32_per_s_wide = w;
     if (imad_per_s_lo) *imad_per_s_lo = l;
     if (iadd3_per_s) *iadd3_per_s = a;

@@ -1,6 +1,8 @@
 // C ABI, part 2: R1CS shape upload (COO -> CSR), multiply_vec, commit_T, fold, and the device-resident
 // running instance used for a chain of fold steps.  Contract and reference pointers: include/vdfgpu.h.
 #include <cstring>
+#include <memory>
+#include <type_traits>
 #include <vector>
 
 #include "ctx.cuh"
@@ -23,6 +25,10 @@ struct vdfgpu_r1cs {
   mutable int refs = 0;   // running instances holding this shape (vdfgpu_r1cs_destroy refuses while > 0)
   vdf::CsrView view() const { return vdf::CsrView{row_ptr, col, val, cons, vars, io}; }
   vdf::CscView col_view() const { return vdf::CscView{col_ptr, csc_row, csc_val, heavy, vdf::HostCsc::HEAVY}; }
+  ~vdfgpu_r1cs() {   // the one release path: failed create, vdfgpu_r1cs_destroy
+    cudaFree(row_ptr); cudaFree(col); cudaFree(val);
+    cudaFree(col_ptr); cudaFree(csc_row); cudaFree(csc_val); cudaFree(heavy);
+  }
 };
 
 struct vdfgpu_running {
@@ -41,6 +47,12 @@ struct vdfgpu_running {
   // stream or thread (vdfgpu_running_finish returns before its fold has run) is ordered behind the previous one
   cudaEvent_t done = nullptr;
   bool have_running = false, have_fresh = false;
+  ~vdfgpu_running() {   // the one release path: failed create, vdfgpu_running_destroy
+    if (bounce) cudaFreeHost(bounce);
+    if (done) cudaEventDestroy(done);
+    cudaFree(W); cudaFree(W2); cudaFree(E); cudaFree(T); cudaFree(uX); cudaFree(uX2);
+    cudaFree(r); cudaFree(comm);
+  }
 };
 
 // Step-circuit witnesses of all n steps of one proof, generated on the device (SURVEY 8f rank 1) on a side stream
@@ -51,45 +63,46 @@ struct vdfgpu_witness_bank {
   vdf::fe* w = nullptr;         // [n][4t + 1]
   cudaStream_t stream = nullptr;
   cudaEvent_t ready = nullptr;
+  ~vdfgpu_witness_bank() {   // the one release path: failed create, vdfgpu_witness_bank_destroy
+    if (w) cudaFree(w);
+    if (ready) cudaEventDestroy(ready);
+    if (stream) cudaStreamDestroy(stream);
+  }
 };
 
 namespace vdf {
 
-template <class Fn0, class Fn1>
-static void by_field(int field, Fn0 fp, Fn1 fq) {
-  if (field == VDFGPU_FP) fp();
-  else fq();
-}
-
 static void launch_multiply_vec(CudaLaunch& L, const vdfgpu_r1cs* s, ZView z, fe* Az, fe* Bz, fe* Cz) {
-  size_t rows = 3 * (size_t)s->cons;
-  if (s->field == VDFGPU_FP) L.run<128>(rows, MultiplyVecFn<Fp>{s->view(), z, Az, Bz, Cz});
-  else L.run<128>(rows, MultiplyVecFn<Fq>{s->view(), z, Az, Bz, Cz});
+  with_field(s->field, "r1cs", [&](auto f) {
+    L.run<128>(3 * (size_t)s->cons, MultiplyVecFn<decltype(f)>{s->view(), z, Az, Bz, Cz});
+  });
 }
 
 static void launch_cross_term(CudaLaunch& L, const vdfgpu_r1cs* s, ZView z1, ZView z2, fe* T) {
 #ifndef VDF_CT_MINB
 #define VDF_CT_MINB 8
 #endif
-  if (s->field == VDFGPU_FP) L.run<128, VDF_CT_MINB>(s->cons, CrossTermFn<Fp>{s->view(), z1, z2, T});
-  else L.run<128, VDF_CT_MINB>(s->cons, CrossTermFn<Fq>{s->view(), z1, z2, T});
+  with_field(s->field, "r1cs", [&](auto f) {
+    L.run<128, VDF_CT_MINB>(s->cons, CrossTermFn<decltype(f)>{s->view(), z1, z2, T});
+  });
 }
 
-static void launch_fold(CudaLaunch& L, int field, fe* W1, const fe* W2, size_t nW, fe* E1, const fe* T, size_t nE,
-                        const fe* r) {
-  if (field == VDFGPU_FP) L.run<256>(nW + nE, FoldFn<Fp>{W1, W2, nW, E1, T, nE, r});
-  else L.run<256>(nW + nE, FoldFn<Fq>{W1, W2, nW, E1, T, nE, r});
+template <class F>
+static void launch_fold(CudaLaunch& L, fe* W1, const fe* W2, size_t nW, fe* E1, const fe* T, size_t nE, const fe* r) {
+  L.run<256>(nW + nE, FoldFn<F>{W1, W2, nW, E1, T, nE, r});
 }
 
 // the scalar field of the commitment curve must be the R1CS field
 static void check_gens_field(const vdfgpu_r1cs* s, const vdfgpu_gens* g) {
-  int scalar_field = g->curve == VDFGPU_PALLAS ? VDFGPU_FQ : VDFGPU_FP;
-  if (scalar_field != s->field) throw ArgError("generator curve's scalar field differs from the R1CS field");
+  const bool same = with_curve(g->curve, "gens", [&](auto, auto, auto SF) {
+    return with_field(s->field, "r1cs", [](auto f) { return std::is_same<decltype(f), decltype(SF)>::value; });
+  });
+  if (!same) throw ArgError("generator curve's scalar field differs from the R1CS field");
 }
 
 void upload_constants_r1cs() { VDF_CUDA_CHECK(upload_field_constants()); }
 
-static fe host_one(int field) { return field == VDFGPU_FP ? Fp::one() : Fq::one(); }
+static fe host_one(int field) { return with_field(field, "r1cs", [](auto f) { return decltype(f)::one(); }); }
 
 // every vdfgpu_running_* call that enqueues work: running_after() before its first operation on `st`,
 // running_done() after its last
@@ -103,8 +116,9 @@ static void launch_sat(CudaLaunch& L, const vdfgpu_r1cs* s, ZView z, const fe* E
   uint32_t* bad = words;
   uint32_t* first = words + 2;
   L.run<32>(1, SatInitFn{words, s->cons});
-  if (s->field == VDFGPU_FP) L.run<128, 8>(s->cons, RelaxedSatFn<Fp>{s->view(), z, E, bad, first});
-  else L.run<128, 8>(s->cons, RelaxedSatFn<Fq>{s->view(), z, E, bad, first});
+  with_field(s->field, "r1cs", [&](auto f) {
+    L.run<128, 8>(s->cons, RelaxedSatFn<decltype(f)>{s->view(), z, E, bad, first});
+  });
 }
 
 // What one check brings back to the host: the two counters and commit(W), commit(E) as un-normalised points, in ONE
@@ -133,12 +147,10 @@ static void check_sat_gens(const vdfgpu_r1cs* s, const vdfgpu_gens* g, const cha
 // computed un-normalised whatever the set's flags and normalised on the host once they have landed (`res`).
 static void sat_enqueue(const vdfgpu_r1cs* s, vdfgpu_gens* gens, const fe* W, const fe* E, const fe* uX, bool want_W,
                         bool want_E, SatResult& res) {
-  Context& c = ctx();
   cudaStream_t st = cur_stream();
-  CudaLaunch L(st);
+  CudaLaunch L = api_launch(st);
   DevBuf<jac_t> out(3, st);
   launch_sat(L, s, ZView{W, uX, uX + 1}, E, reinterpret_cast<uint64_t*>(out.p));
-  c.launches += L.launches;
   const fe* vecs[2];
   size_t lens[2];
   uint32_t k = 0;
@@ -189,7 +201,7 @@ int vdfgpu_r1cs_create(int field, size_t num_cons, size_t num_vars, size_t num_i
                        vdfgpu_r1cs** out) {
   return guarded([&] {
     if (!out) throw ArgError("r1cs_create: null out");
-    if (field != VDFGPU_FP && field != VDFGPU_FQ) throw ArgError("r1cs_create: unknown field");
+    with_field(field, "r1cs_create", [](auto) {});
     if (num_cons == 0 || num_cons >= (1ull << 30) || num_vars >= (1ull << 31)) throw ArgError("r1cs_create: bad dimensions");
     const uint64_t* rows[3] = {a_rows, b_rows, c_rows};
     const uint64_t* cols[3] = {a_cols, b_cols, c_cols};
@@ -209,38 +221,30 @@ int vdfgpu_r1cs_create(int field, size_t num_cons, size_t num_vars, size_t num_i
     std::vector<uint32_t>& row_ptr = csr.row_ptr;
     std::vector<uint32_t>& col = csr.col;
     std::vector<uint8_t>& val = csr.val;
-    vdfgpu_r1cs* s = new vdfgpu_r1cs();
+    std::unique_ptr<vdfgpu_r1cs> s(new vdfgpu_r1cs());
     s->field = field;
     s->cons = (uint32_t)num_cons;
     s->vars = (uint32_t)num_vars;
     s->io = (uint32_t)num_io;
     s->nnz = nnz;
-    Context& c = ctx();
-    try {
-      VDF_CUDA_CHECK(cudaMalloc((void**)&s->row_ptr, (R + 1) * 4));
-      VDF_CUDA_CHECK(cudaMalloc((void**)&s->col, (nnz ? nnz : 1) * 4));
-      VDF_CUDA_CHECK(cudaMalloc((void**)&s->val, (nnz ? nnz : 1) * 32));
-      h2d(s->row_ptr, row_ptr.data(), (R + 1) * 4, cur_stream());
-      h2d(s->col, col.data(), nnz * 4, cur_stream());
-      h2d(s->val, val.data(), nnz * 32, cur_stream());
-      const HostCsc csc = csr_to_csc(csr, ncols);
-      s->n_heavy = (uint32_t)csc.heavy.size();
-      VDF_CUDA_CHECK(cudaMalloc((void**)&s->col_ptr, (ncols + 1) * 4));
-      VDF_CUDA_CHECK(cudaMalloc((void**)&s->csc_row, (nnz ? nnz : 1) * 4));
-      VDF_CUDA_CHECK(cudaMalloc((void**)&s->csc_val, (nnz ? nnz : 1) * 32));
-      VDF_CUDA_CHECK(cudaMalloc((void**)&s->heavy, (s->n_heavy ? s->n_heavy : 1) * 4));
-      h2d(s->col_ptr, csc.col_ptr.data(), (ncols + 1) * 4, cur_stream());
-      h2d(s->csc_row, csc.srow.data(), nnz * 4, cur_stream());
-      h2d(s->csc_val, csc.val.data(), nnz * 32, cur_stream());
-      h2d(s->heavy, csc.heavy.data(), (size_t)s->n_heavy * 4, cur_stream());
-      sync_after_unlock(cur_stream());
-    } catch (...) {
-      cudaFree(s->row_ptr); cudaFree(s->col); cudaFree(s->val);
-      cudaFree(s->col_ptr); cudaFree(s->csc_row); cudaFree(s->csc_val); cudaFree(s->heavy);
-      delete s;
-      throw;
-    }
-    *out = s;
+    VDF_CUDA_CHECK(cudaMalloc((void**)&s->row_ptr, (R + 1) * 4));
+    VDF_CUDA_CHECK(cudaMalloc((void**)&s->col, (nnz ? nnz : 1) * 4));
+    VDF_CUDA_CHECK(cudaMalloc((void**)&s->val, (nnz ? nnz : 1) * 32));
+    h2d(s->row_ptr, row_ptr.data(), (R + 1) * 4, cur_stream());
+    h2d(s->col, col.data(), nnz * 4, cur_stream());
+    h2d(s->val, val.data(), nnz * 32, cur_stream());
+    const HostCsc csc = csr_to_csc(csr, ncols);
+    s->n_heavy = (uint32_t)csc.heavy.size();
+    VDF_CUDA_CHECK(cudaMalloc((void**)&s->col_ptr, (ncols + 1) * 4));
+    VDF_CUDA_CHECK(cudaMalloc((void**)&s->csc_row, (nnz ? nnz : 1) * 4));
+    VDF_CUDA_CHECK(cudaMalloc((void**)&s->csc_val, (nnz ? nnz : 1) * 32));
+    VDF_CUDA_CHECK(cudaMalloc((void**)&s->heavy, (s->n_heavy ? s->n_heavy : 1) * 4));
+    h2d(s->col_ptr, csc.col_ptr.data(), (ncols + 1) * 4, cur_stream());
+    h2d(s->csc_row, csc.srow.data(), nnz * 4, cur_stream());
+    h2d(s->csc_val, csc.val.data(), nnz * 32, cur_stream());
+    h2d(s->heavy, csc.heavy.data(), (size_t)s->n_heavy * 4, cur_stream());
+    sync_after_unlock(cur_stream());
+    *out = s.release();
   });
 }
 
@@ -252,8 +256,6 @@ int vdfgpu_r1cs_destroy(vdfgpu_r1cs* s) {
       VDF_CUDA_CHECK(cudaSetDevice(ctx().device));
       cudaDeviceSynchronize();
     }
-    cudaFree(s->row_ptr); cudaFree(s->col); cudaFree(s->val);
-    cudaFree(s->col_ptr); cudaFree(s->csc_row); cudaFree(s->csc_val); cudaFree(s->heavy);
     delete s;
   });
 }
@@ -262,8 +264,7 @@ int vdfgpu_multiply_vec(const vdfgpu_r1cs* s, const void* z_host, void* Az_host,
   return guarded([&] {
     if (!s || !z_host || !Az_host || !Bz_host || !Cz_host) throw ArgError("multiply_vec: null pointer");
     require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
+    CudaLaunch L = api_launch(cur_stream());
     size_t nz = (size_t)s->vars + 1 + s->io;
     DevBuf<fe> z(nz, cur_stream()), out(3 * (size_t)s->cons, cur_stream());
     h2d(z.p, z_host, nz * 32, cur_stream());
@@ -272,7 +273,6 @@ int vdfgpu_multiply_vec(const vdfgpu_r1cs* s, const void* z_host, void* Az_host,
     d2h(Az_host, out.p, (size_t)s->cons * 32, cur_stream());
     d2h(Bz_host, out.p + s->cons, (size_t)s->cons * 32, cur_stream());
     d2h(Cz_host, out.p + 2 * (size_t)s->cons, (size_t)s->cons * 32, cur_stream());
-    c.launches += L.launches;
     sync_after_unlock(cur_stream());
   });
 }
@@ -289,8 +289,7 @@ int vdfgpu_commit_T(const vdfgpu_r1cs* s, vdfgpu_gens* gens, const void* W1_host
       if (gens->n < s->cons) throw ArgError("commit_T: fewer generators than constraints");
     }
     require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
+    CudaLaunch L = api_launch(cur_stream());
     const size_t nv = s->vars, io = s->io, nc = s->cons;
     DevBuf<fe> W1(nv ? nv : 1, cur_stream()), W2(nv ? nv : 1, cur_stream()), uX1(1 + io, cur_stream()), uX2(1 + io, cur_stream());
     DevBuf<fe> T(nc, cur_stream());
@@ -303,7 +302,6 @@ int vdfgpu_commit_T(const vdfgpu_r1cs* s, vdfgpu_gens* gens, const void* W1_host
     h2d(uX2.p, &one, 32, cur_stream());  // u2 = 1 (fresh instance); pageable 32-byte copy is staged by the driver
     h2d(uX2.p + 1, X2_host, io * 32, cur_stream());
     launch_cross_term(L, s, ZView{W1.p, uX1.p, uX1.p + 1}, ZView{W2.p, uX2.p, uX2.p + 1}, T.p);
-    c.launches += L.launches;
     const bool hn = gens && host_normalise_wanted(gens);
     if (gens) {
       msm_on_device(gens, 0, T.p, nc, comm.p, true, nullptr, hn);
@@ -318,23 +316,22 @@ int vdfgpu_commit_T(const vdfgpu_r1cs* s, vdfgpu_gens* gens, const void* W1_host
 int vdfgpu_fold(int field, void* W1_host, const void* W2_host, size_t nW, void* E1_host, const void* T_host,
                 size_t nE, const void* r32_host) {
   return guarded([&] {
-    if (field != VDFGPU_FP && field != VDFGPU_FQ) throw ArgError("fold: unknown field");
-    if (!r32_host || (nW && (!W1_host || !W2_host)) || (nE && (!E1_host || !T_host))) throw ArgError("fold: null pointer");
-    if (nW + nE == 0) return;
-    require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
-    DevBuf<fe> W1(nW ? nW : 1, cur_stream()), W2(nW ? nW : 1, cur_stream()), E1(nE ? nE : 1, cur_stream()), T(nE ? nE : 1, cur_stream()), r(1, cur_stream());
-    h2d(W1.p, W1_host, nW * 32, cur_stream());
-    h2d(W2.p, W2_host, nW * 32, cur_stream());
-    h2d(E1.p, E1_host, nE * 32, cur_stream());
-    h2d(T.p, T_host, nE * 32, cur_stream());
-    h2d(r.p, r32_host, 32, cur_stream());
-    launch_fold(L, field, W1.p, W2.p, nW, E1.p, T.p, nE, r.p);
-    d2h(W1_host, W1.p, nW * 32, cur_stream());
-    d2h(E1_host, E1.p, nE * 32, cur_stream());
-    c.launches += L.launches;
-    sync_after_unlock(cur_stream());
+    with_field(field, "fold", [&](auto f) {
+      if (!r32_host || (nW && (!W1_host || !W2_host)) || (nE && (!E1_host || !T_host))) throw ArgError("fold: null pointer");
+      if (nW + nE == 0) return;
+      require_ready();
+      CudaLaunch L = api_launch(cur_stream());
+      DevBuf<fe> W1(nW ? nW : 1, cur_stream()), W2(nW ? nW : 1, cur_stream()), E1(nE ? nE : 1, cur_stream()), T(nE ? nE : 1, cur_stream()), r(1, cur_stream());
+      h2d(W1.p, W1_host, nW * 32, cur_stream());
+      h2d(W2.p, W2_host, nW * 32, cur_stream());
+      h2d(E1.p, E1_host, nE * 32, cur_stream());
+      h2d(T.p, T_host, nE * 32, cur_stream());
+      h2d(r.p, r32_host, 32, cur_stream());
+      launch_fold<decltype(f)>(L, W1.p, W2.p, nW, E1.p, T.p, nE, r.p);
+      d2h(W1_host, W1.p, nW * 32, cur_stream());
+      d2h(E1_host, E1.p, nE * 32, cur_stream());
+      sync_after_unlock(cur_stream());
+    });
   });
 }
 
@@ -342,13 +339,11 @@ int vdfgpu_multiply_vec_dev(const vdfgpu_r1cs* s, const void* W_dev, const void*
   return guarded([&] {
     if (!s || !uX_dev || !AzBzCz_dev || (s->vars && !W_dev)) throw ArgError("multiply_vec_dev: null pointer");
     require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
+    CudaLaunch L = api_launch(cur_stream());
     const fe* ux = reinterpret_cast<const fe*>(uX_dev);
     fe* out = reinterpret_cast<fe*>(AzBzCz_dev);
     launch_multiply_vec(L, s, ZView{reinterpret_cast<const fe*>(W_dev), ux, ux + 1}, out, out + s->cons,
                         out + 2 * (size_t)s->cons);
-    c.launches += L.launches;
   });
 }
 
@@ -381,41 +376,34 @@ int vdfgpu_r1cs_is_sat_relaxed_dev(const vdfgpu_r1cs* s, const void* W_dev, cons
   return guarded([&] {
     if (!s || !uX_dev || !counts2_dev || (s->vars && !W_dev)) throw ArgError("r1cs_is_sat_relaxed_dev: null pointer");
     require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
+    CudaLaunch L = api_launch(cur_stream());
     const fe* ux = reinterpret_cast<const fe*>(uX_dev);
     launch_sat(L, s, ZView{reinterpret_cast<const fe*>(W_dev), ux, ux + 1}, reinterpret_cast<const fe*>(E_dev), counts2_dev);
-    c.launches += L.launches;
   });
 }
 
 static void launch_bind_rows(CudaLaunch& L, const vdfgpu_r1cs* s, const fe* eq, const fe* coef, fe* eq3, fe* out) {
   const size_t ncols = (size_t)s->vars + 1 + s->io;
   const CscView v = s->col_view();
-  if (s->field == VDFGPU_FP) {
-    L.run<128>(3 * (size_t)s->cons, ScaleRowsFn<Fp>{eq, coef, s->cons, eq3});
-    L.run<128>(ncols, BindRowsFn<Fp>{v, eq3, out});
-    if (s->n_heavy) L.run<BindHeavyFn<Fp>::THREADS>((size_t)s->n_heavy * BindHeavyFn<Fp>::THREADS, BindHeavyFn<Fp>{v, eq3, out});
-  } else {
-    L.run<128>(3 * (size_t)s->cons, ScaleRowsFn<Fq>{eq, coef, s->cons, eq3});
-    L.run<128>(ncols, BindRowsFn<Fq>{v, eq3, out});
-    if (s->n_heavy) L.run<BindHeavyFn<Fq>::THREADS>((size_t)s->n_heavy * BindHeavyFn<Fq>::THREADS, BindHeavyFn<Fq>{v, eq3, out});
-  }
+  with_field(s->field, "r1cs", [&](auto f) {
+    using F = decltype(f);
+    L.run<128>(3 * (size_t)s->cons, ScaleRowsFn<F>{eq, coef, s->cons, eq3});
+    L.run<128>(ncols, BindRowsFn<F>{v, eq3, out});
+    if (s->n_heavy) L.run<BindHeavyFn<F>::THREADS>((size_t)s->n_heavy * BindHeavyFn<F>::THREADS, BindHeavyFn<F>{v, eq3, out});
+  });
 }
 
 int vdfgpu_r1cs_bind_rows(const vdfgpu_r1cs* s, const void* eq_rows_host, const void* r_abc_host, void* out_host) {
   return guarded([&] {
     if (!s || !eq_rows_host || !r_abc_host || !out_host) throw ArgError("r1cs_bind_rows: null pointer");
     require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
+    CudaLaunch L = api_launch(cur_stream());
     const size_t ncols = (size_t)s->vars + 1 + s->io;
     DevBuf<fe> eq(s->cons, cur_stream()), coef(3, cur_stream()), eq3(3 * (size_t)s->cons, cur_stream()), out(ncols, cur_stream());
     h2d(eq.p, eq_rows_host, (size_t)s->cons * 32, cur_stream());
     h2d(coef.p, r_abc_host, 96, cur_stream());
     launch_bind_rows(L, s, eq.p, coef.p, eq3.p, out.p);
     d2h(out_host, out.p, ncols * 32, cur_stream());
-    c.launches += L.launches;
     sync_after_unlock(cur_stream());
   });
 }
@@ -425,11 +413,9 @@ int vdfgpu_r1cs_bind_rows_dev(const vdfgpu_r1cs* s, const void* eq_rows_dev, con
   return guarded([&] {
     if (!s || !eq_rows_dev || !r_abc_dev || !scratch_dev || !out_dev) throw ArgError("r1cs_bind_rows_dev: null pointer");
     require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
+    CudaLaunch L = api_launch(cur_stream());
     launch_bind_rows(L, s, reinterpret_cast<const fe*>(eq_rows_dev), reinterpret_cast<const fe*>(r_abc_dev),
                      reinterpret_cast<fe*>(scratch_dev), reinterpret_cast<fe*>(out_dev));
-    c.launches += L.launches;
   });
 }
 
@@ -438,27 +424,25 @@ int vdfgpu_cross_term_dev(const vdfgpu_r1cs* s, const void* W1_dev, const void* 
   return guarded([&] {
     if (!s || !uX1_dev || !uX2_dev || !T_dev || (s->vars && (!W1_dev || !W2_dev))) throw ArgError("cross_term_dev: null pointer");
     require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
+    CudaLaunch L = api_launch(cur_stream());
     const fe* u1 = reinterpret_cast<const fe*>(uX1_dev);
     const fe* u2 = reinterpret_cast<const fe*>(uX2_dev);
     launch_cross_term(L, s, ZView{reinterpret_cast<const fe*>(W1_dev), u1, u1 + 1},
                       ZView{reinterpret_cast<const fe*>(W2_dev), u2, u2 + 1}, reinterpret_cast<fe*>(T_dev));
-    c.launches += L.launches;
   });
 }
 
 int vdfgpu_fold_dev(int field, void* W1_dev, const void* W2_dev, size_t nW, void* E1_dev, const void* T_dev,
                     size_t nE, const void* r32_dev) {
   return guarded([&] {
-    if (field != VDFGPU_FP && field != VDFGPU_FQ) throw ArgError("fold_dev: unknown field");
-    if (!r32_dev || (nW && (!W1_dev || !W2_dev)) || (nE && (!E1_dev || !T_dev))) throw ArgError("fold_dev: null pointer");
-    require_ready();
-    Context& c = ctx();
-    CudaLaunch L(cur_stream());
-    launch_fold(L, field, reinterpret_cast<fe*>(W1_dev), reinterpret_cast<const fe*>(W2_dev), nW,
-                reinterpret_cast<fe*>(E1_dev), reinterpret_cast<const fe*>(T_dev), nE, reinterpret_cast<const fe*>(r32_dev));
-    c.launches += L.launches;
+    with_field(field, "fold_dev", [&](auto f) {
+      if (!r32_dev || (nW && (!W1_dev || !W2_dev)) || (nE && (!E1_dev || !T_dev))) throw ArgError("fold_dev: null pointer");
+      require_ready();
+      CudaLaunch L = api_launch(cur_stream());
+      launch_fold<decltype(f)>(L, reinterpret_cast<fe*>(W1_dev), reinterpret_cast<const fe*>(W2_dev), nW,
+                               reinterpret_cast<fe*>(E1_dev), reinterpret_cast<const fe*>(T_dev), nE,
+                               reinterpret_cast<const fe*>(r32_dev));
+    });
   });
 }
 
@@ -469,31 +453,23 @@ int vdfgpu_running_create(const vdfgpu_r1cs* s, vdfgpu_gens* gens, vdfgpu_runnin
     check_gens_field(s, gens);
     if (gens->n < s->cons || gens->n < s->vars) throw ArgError("running_create: fewer generators than max(cons, vars)");
     require_ready();
-    vdfgpu_running* f = new vdfgpu_running();
+    std::unique_ptr<vdfgpu_running> f(new vdfgpu_running());
     f->shape = s;
     f->gens = gens;
     const size_t nv = s->vars ? s->vars : 1, nc = s->cons, io1 = 1 + s->io;
-    try {
-      VDF_CUDA_CHECK(cudaMalloc((void**)&f->W, nv * 32));
-      VDF_CUDA_CHECK(cudaMalloc((void**)&f->W2, nv * 32));
-      VDF_CUDA_CHECK(cudaMalloc((void**)&f->E, nc * 32));
-      VDF_CUDA_CHECK(cudaMalloc((void**)&f->T, nc * 32));
-      VDF_CUDA_CHECK(cudaMalloc((void**)&f->uX, io1 * 32));
-      VDF_CUDA_CHECK(cudaMalloc((void**)&f->uX2, io1 * 32));
-      VDF_CUDA_CHECK(cudaMalloc((void**)&f->r, 32));
-      VDF_CUDA_CHECK(cudaMalloc((void**)&f->comm, 2 * sizeof(jac_t)));
-      VDF_CUDA_CHECK(cudaHostAlloc((void**)&f->bounce, 2 * sizeof(jac_t) + io1 * sizeof(fe), cudaHostAllocDefault));
-      VDF_CUDA_CHECK(cudaEventCreateWithFlags(&f->done, cudaEventDisableTiming));
-    } catch (...) {
-      if (f->bounce) cudaFreeHost(f->bounce);
-      cudaFree(f->W); cudaFree(f->W2); cudaFree(f->E); cudaFree(f->T); cudaFree(f->uX); cudaFree(f->uX2);
-      cudaFree(f->r); cudaFree(f->comm);
-      delete f;
-      throw;
-    }
+    VDF_CUDA_CHECK(cudaMalloc((void**)&f->W, nv * 32));
+    VDF_CUDA_CHECK(cudaMalloc((void**)&f->W2, nv * 32));
+    VDF_CUDA_CHECK(cudaMalloc((void**)&f->E, nc * 32));
+    VDF_CUDA_CHECK(cudaMalloc((void**)&f->T, nc * 32));
+    VDF_CUDA_CHECK(cudaMalloc((void**)&f->uX, io1 * 32));
+    VDF_CUDA_CHECK(cudaMalloc((void**)&f->uX2, io1 * 32));
+    VDF_CUDA_CHECK(cudaMalloc((void**)&f->r, 32));
+    VDF_CUDA_CHECK(cudaMalloc((void**)&f->comm, 2 * sizeof(jac_t)));
+    VDF_CUDA_CHECK(cudaHostAlloc((void**)&f->bounce, 2 * sizeof(jac_t) + io1 * sizeof(fe), cudaHostAllocDefault));
+    VDF_CUDA_CHECK(cudaEventCreateWithFlags(&f->done, cudaEventDisableTiming));
     s->refs++;
     gens->refs++;
-    *out = f;
+    *out = f.release();
   });
 }
 
@@ -506,10 +482,6 @@ int vdfgpu_running_destroy(vdfgpu_running* f) {
     }
     f->shape->refs--;
     f->gens->refs--;
-    cudaFreeHost(f->bounce);
-    cudaEventDestroy(f->done);
-    cudaFree(f->W); cudaFree(f->W2); cudaFree(f->E); cudaFree(f->T); cudaFree(f->uX); cudaFree(f->uX2);
-    cudaFree(f->r); cudaFree(f->comm);
     delete f;
   });
 }
@@ -577,12 +549,10 @@ static void upload_ux2(vdfgpu_running* f, const void* X2_host, cudaStream_t st) 
 
 // the part of running_commit after W2 / X2 are in place: T, then commit(W2) and commit(T) in one batched pass
 static void running_commit_enqueue(vdfgpu_running* f, void* comm_W2_point96_host, void* comm_T_point96_host) {
-  Context& c = ctx();
   cudaStream_t st = cur_stream();
-  CudaLaunch L(st);
+  CudaLaunch L = api_launch(st);
   const vdfgpu_r1cs* s = f->shape;
   launch_cross_term(L, s, ZView{f->W, f->uX, f->uX + 1}, ZView{f->W2, f->uX2, f->uX2 + 1}, f->T);
-  c.launches += L.launches;
   const fe* vecs[2] = {f->W2, f->T};
   const size_t lens[2] = {s->vars, s->cons};
   const bool hn = host_normalise_wanted(f->gens);
@@ -620,44 +590,34 @@ int vdfgpu_witness_bank_create(int field, const void* z_in_state96_host, uint64_
                                vdfgpu_witness_bank** out) {
   return guarded([&] {
     if (!out || !z_in_state96_host) throw ArgError("witness_bank_create: null pointer");
-    if (field != VDFGPU_FP && field != VDFGPU_FQ) throw ArgError("witness_bank_create: unknown field");
-    if (n == 0 || t == 0 || t >= (1ull << 32)) throw ArgError("witness_bank_create: bad dimensions");
-    require_ready();
-    Context& c = ctx();
-    vdfgpu_witness_bank* b = new vdfgpu_witness_bank();
-    b->field = field;
-    b->t = t;
-    b->n = n;
-    const size_t per = 4 * (size_t)t + 1;
-    state_t* d_states = nullptr;
-    try {
+    with_field(field, "witness_bank_create", [&](auto f) {
+      if (n == 0 || t == 0 || t >= (1ull << 32)) throw ArgError("witness_bank_create: bad dimensions");
+      require_ready();
+      std::unique_ptr<vdfgpu_witness_bank> b(new vdfgpu_witness_bank());
+      b->field = field;
+      b->t = t;
+      b->n = n;
+      const size_t per = 4 * (size_t)t + 1;
+      state_t* d_states = nullptr;
       VDF_CUDA_CHECK(cudaStreamCreateWithFlags(&b->stream, cudaStreamNonBlocking));
       VDF_CUDA_CHECK(cudaEventCreateWithFlags(&b->ready, cudaEventDisableTiming));
       VDF_CUDA_CHECK(cudaMalloc((void**)&b->w, n * per * sizeof(fe)));
       VDF_CUDA_CHECK(cudaMallocAsync((void**)&d_states, n * sizeof(state_t), b->stream));
-      CudaLaunch L(b->stream);
+      CudaLaunch L = api_launch(b->stream);
       h2d(d_states, z_in_state96_host, n * sizeof(state_t), b->stream);
       // one thread per step (the rounds of a step are a sequential chain); 32-thread blocks spread few steps
       // over many SMs.  Runs on the bank's own stream: fold steps of the other curve proceed meanwhile.
-      if (field == VDFGPU_FP) L.run<32>(n, MinRootWitnessFn<Fp>{d_states, t, b->w});
-      else L.run<32>(n, MinRootWitnessFn<Fq>{d_states, t, b->w});
+      L.run<32>(n, MinRootWitnessFn<decltype(f)>{d_states, t, b->w});
       VDF_CUDA_CHECK(cudaFreeAsync(d_states, b->stream));
       VDF_CUDA_CHECK(cudaEventRecord(b->ready, b->stream));
-      c.launches += L.launches;
       // the caller's state array may be reused after return: wait for the upload only if it was asynchronous
       // (pinned memory); pageable copies are staged before cudaMemcpyAsync returns
       cudaPointerAttributes at;
       if (cudaPointerGetAttributes(&at, z_in_state96_host) == cudaSuccess && at.type == cudaMemoryTypeHost)
         sync_after_unlock(b->stream);
       else cudaGetLastError();
-    } catch (...) {
-      if (b->w) cudaFree(b->w);
-      if (b->ready) cudaEventDestroy(b->ready);
-      if (b->stream) cudaStreamDestroy(b->stream);
-      delete b;
-      throw;
-    }
-    *out = b;
+      *out = b.release();
+    });
   });
 }
 
@@ -668,9 +628,6 @@ int vdfgpu_witness_bank_destroy(vdfgpu_witness_bank* b) {
       VDF_CUDA_CHECK(cudaSetDevice(ctx().device));
       cudaDeviceSynchronize();
     }
-    cudaFree(b->w);
-    cudaEventDestroy(b->ready);
-    cudaStreamDestroy(b->stream);
     delete b;
   });
 }
@@ -720,16 +677,16 @@ int vdfgpu_running_finish(vdfgpu_running* f, const void* r32_host) {
     if (!f || !r32_host) throw ArgError("running_finish: null pointer");
     if (!f->have_fresh) throw StateError("running_finish: fold_commit has not been called for this step");
     require_ready();
-    Context& c = ctx();
     cudaStream_t st = cur_stream();
-    CudaLaunch L(st);
+    CudaLaunch L = api_launch(st);
     const vdfgpu_r1cs* s = f->shape;
     running_after(f, st);
     h2d(f->r, r32_host, 32, st);
-    launch_fold(L, s->field, f->W, f->W2, s->vars, f->E, f->T, s->cons, f->r);
-    // u <- u + r*1, X <- X + r*X2: the same kernel over the (1 + io)-element tail
-    launch_fold(L, s->field, f->uX, f->uX2, 1 + (size_t)s->io, nullptr, nullptr, 0, f->r);
-    c.launches += L.launches;
+    with_field(s->field, "running_finish", [&](auto F) {
+      launch_fold<decltype(F)>(L, f->W, f->W2, s->vars, f->E, f->T, s->cons, f->r);
+      // u <- u + r*1, X <- X + r*X2: the same kernel over the (1 + io)-element tail
+      launch_fold<decltype(F)>(L, f->uX, f->uX2, 1 + (size_t)s->io, nullptr, nullptr, 0, f->r);
+    });
     running_done(f, st);
     // No wait: the next call on this instance, on any stream or thread, waits for f->done.  Only a pinned r32_host
     // would still be in flight after return (pageable copies are staged before cudaMemcpyAsync returns).

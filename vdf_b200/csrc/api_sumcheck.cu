@@ -65,18 +65,34 @@ static void dot_enqueue(cudaStream_t st, const fe* a, const fe* b, size_t n, con
   ctx().launches += 2;
 }
 
-// the round loop shared by the cubic (4 tables, 3 evaluations) and quadratic (2 tables, 2 evaluations) sum-checks
-static int sumcheck_run(int field, PolySet P, int n_polys, size_t ell, vdfgpu_round_fn fn, void* user, void* final_host) {
-  if (field != VDFGPU_FP && field != VDFGPU_FQ) { set_error("sumcheck: unknown field"); return VDFGPU_ERR_ARG; }
-  if (ell > 40 || !final_host || (ell && !fn)) { set_error("sumcheck: bad arguments"); return VDFGPU_ERR_ARG; }
-  for (int q = 0; q < n_polys; q++)
-    if (!P.p[q]) { set_error("sumcheck: null table"); return VDFGPU_ERR_ARG; }
+// Both sum-checks, cubic (4 tables, 3 evaluations) and quadratic (2 tables, 2 evaluations), in both forms: tables on
+// the device, bound in place, or on the host (ell <= 30), uploaded first and freed at the end.  Every guarded() section
+// ends before the caller's round callback runs, so the tables and the scratch outlive several of them.
+static int sumcheck(int field, const void* const* tables, int n_polys, bool on_host, size_t ell, vdfgpu_round_fn fn,
+                    void* user, void* final_host) {
   const int n_evals = n_polys == 4 ? 3 : 2;
+  PolySet P{{nullptr, nullptr, nullptr, nullptr}};
   ScScratch s;
   int rc = guarded([&] {
+    with_field(field, "sumcheck", [](auto) {});
+    if (ell > 40 || !final_host || (ell && !fn)) throw ArgError("sumcheck: bad arguments");
+    for (int q = 0; q < n_polys; q++)
+      if (!tables[q]) throw ArgError("sumcheck: null table");
+    if (on_host && ell > 30) throw ArgError("sumcheck: ell too large for the host-table form");
     require_ready();
-    VDF_CUDA_CHECK(cudaMallocAsync((void**)&s.partial, (size_t)148 * 8 * 3 * sizeof(fe), cur_stream()));
-    VDF_CUDA_CHECK(cudaMallocAsync((void**)&s.evals, 4 * sizeof(fe), cur_stream()));
+    cudaStream_t st = cur_stream();
+    const size_t bytes = ((size_t)1 << ell) * sizeof(fe);
+    for (int q = 0; q < n_polys; q++) {
+      if (!on_host) {
+        P.p[q] = reinterpret_cast<fe*>(const_cast<void*>(tables[q]));
+        continue;
+      }
+      VDF_CUDA_CHECK(cudaMalloc((void**)&P.p[q], bytes));
+      h2d(P.p[q], tables[q], bytes, st);
+    }
+    VDF_CUDA_CHECK(cudaMallocAsync((void**)&s.partial, (size_t)148 * 8 * 3 * sizeof(fe), st));
+    VDF_CUDA_CHECK(cudaMallocAsync((void**)&s.evals, 4 * sizeof(fe), st));
+    if (on_host) sync_after_unlock(st);
   });
   size_t len = (size_t)1 << ell;
   for (size_t round = 0; rc == VDFGPU_OK && round < ell; round++) {
@@ -85,13 +101,10 @@ static int sumcheck_run(int field, PolySet P, int n_polys, size_t ell, vdfgpu_ro
     rc = guarded([&] {
       require_ready();
       cudaStream_t st = cur_stream();
-      if (n_polys == 4) {
-        if (field == VDFGPU_FP) cubic_round_enqueue<Fp>(st, P, half, s);
-        else cubic_round_enqueue<Fq>(st, P, half, s);
-      } else {
-        if (field == VDFGPU_FP) quad_round_enqueue<Fp>(st, P, half, s);
-        else quad_round_enqueue<Fq>(st, P, half, s);
-      }
+      with_field(field, "sumcheck", [&](auto f) {
+        if (n_polys == 4) cubic_round_enqueue<decltype(f)>(st, P, half, s);
+        else quad_round_enqueue<decltype(f)>(st, P, half, s);
+      });
       fe* pin = pinned_evals();
       VDF_CUDA_CHECK(cudaMemcpyAsync(pin, s.evals, n_evals * sizeof(fe), cudaMemcpyDeviceToHost, st));
       VDF_CUDA_CHECK(cudaStreamSynchronize(st));
@@ -105,11 +118,10 @@ static int sumcheck_run(int field, PolySet P, int n_polys, size_t ell, vdfgpu_ro
     }
     rc = guarded([&] {
       require_ready();
-      cudaStream_t st = cur_stream();
-      CudaLaunch L(st);
-      if (field == VDFGPU_FP) L.run<256>((size_t)n_polys * half, BindTopValFn<Fp>{P, half, r});
-      else L.run<256>((size_t)n_polys * half, BindTopValFn<Fq>{P, half, r});
-      ctx().launches += L.launches;
+      CudaLaunch L = api_launch(cur_stream());
+      with_field(field, "sumcheck", [&](auto f) {
+        L.run<256>((size_t)n_polys * half, BindTopValFn<decltype(f)>{P, half, r});
+      });
     });
     len = half;
   }
@@ -125,13 +137,39 @@ static int sumcheck_run(int field, PolySet P, int n_polys, size_t ell, vdfgpu_ro
     });
   std::string keep = rc == VDFGPU_OK ? std::string() : std::string(vdfgpu_last_error());
   guarded([&] {
-    if (ctx().ready) {
-      if (s.partial) cudaFreeAsync(s.partial, cur_stream());
-      if (s.evals) cudaFreeAsync(s.evals, cur_stream());
-    }
+    if (!ctx().ready) return;
+    if (s.partial) cudaFreeAsync(s.partial, cur_stream());
+    if (s.evals) cudaFreeAsync(s.evals, cur_stream());
+    if (!on_host) return;
+    cudaStreamSynchronize(cur_stream());
+    for (int q = 0; q < n_polys; q++)
+      if (P.p[q]) cudaFree(P.p[q]);
   });
   if (rc != VDFGPU_OK) set_error(keep);
   return rc;
+}
+
+// eq(r, x) for every x in {0,1}^ell into out_dev, from the ell challenges at r_host: both forms of vdfgpu_eq_evals
+template <class F>
+static void eq_evals_from_host(const void* r_host, size_t ell, fe* out_dev, cudaStream_t st) {
+  CudaLaunch L = api_launch(st);
+  DevBuf<fe> r(ell ? ell : 1, st);
+  h2d(r.p, r_host, ell * 32, st);
+  eq_evals_enqueue<F>(L, r.p, ell, out_dev);
+}
+
+// sum over x of eq(r, x) * poly[x] for a table on the device, into out_host once the wait is over: both forms of
+// vdfgpu_poly_evaluate
+template <class F>
+static void poly_evaluate_enqueue(const fe* poly_dev, const void* r_host, size_t ell, void* out_host, cudaStream_t st) {
+  CudaLaunch L = api_launch(st);
+  const size_t n = (size_t)1 << ell;
+  DevBuf<fe> r(ell ? ell : 1, st), eq(n, st), partial((size_t)148 * 8, st), res(1, st);
+  h2d(r.p, r_host, ell * 32, st);
+  eq_evals_enqueue<F>(L, r.p, ell, eq.p);
+  dot_enqueue<F>(st, eq.p, poly_dev, n, ScScratch{partial.p, res.p});
+  d2h(out_host, res.p, sizeof(fe), st);
+  sync_after_unlock(st);
 }
 
 }  // namespace vdf
@@ -143,217 +181,139 @@ extern "C" {
 
 int vdfgpu_eq_evals_dev(int field, const void* r_host, size_t ell, void* out_dev) {
   return guarded([&] {
-    if (field != VDFGPU_FP && field != VDFGPU_FQ) throw ArgError("eq_evals: unknown field");
-    if (!out_dev || (ell && !r_host) || ell > 40) throw ArgError("eq_evals: bad arguments");
-    require_ready();
-    cudaStream_t st = cur_stream();
-    CudaLaunch L(st);
-    DevBuf<fe> r(ell ? ell : 1, st);
-    h2d(r.p, r_host, ell * 32, st);
-    if (field == VDFGPU_FP) eq_evals_enqueue<Fp>(L, r.p, ell, reinterpret_cast<fe*>(out_dev));
-    else eq_evals_enqueue<Fq>(L, r.p, ell, reinterpret_cast<fe*>(out_dev));
-    ctx().launches += L.launches;
-    // r_host may be pinned (asynchronous copy still in flight): wait; a pageable copy is already staged
-    sync_after_unlock(st);
+    with_field(field, "eq_evals", [&](auto f) {
+      if (!out_dev || (ell && !r_host) || ell > 40) throw ArgError("eq_evals: bad arguments");
+      require_ready();
+      eq_evals_from_host<decltype(f)>(r_host, ell, reinterpret_cast<fe*>(out_dev), cur_stream());
+      // r_host may be pinned (asynchronous copy still in flight): wait; a pageable copy is already staged
+      sync_after_unlock(cur_stream());
+    });
   });
 }
 
 int vdfgpu_eq_evals(int field, const void* r_host, size_t ell, void* out_host) {
-  if (!out_host || ell > 30) {
-    set_error("eq_evals: bad arguments");
-    return VDFGPU_ERR_ARG;
-  }
-  fe* d = nullptr;
-  int rc = guarded([&] {
-    require_ready();
-    VDF_CUDA_CHECK(cudaMalloc((void**)&d, ((size_t)1 << ell) * sizeof(fe)));
-  });
-  if (rc == VDFGPU_OK) rc = vdfgpu_eq_evals_dev(field, r_host, ell, d);
-  if (rc == VDFGPU_OK)
-    rc = guarded([&] {
+  return guarded([&] {
+    with_field(field, "eq_evals", [&](auto f) {
+      if (!out_host || (ell && !r_host) || ell > 30) throw ArgError("eq_evals: bad arguments");
       require_ready();
-      d2h(out_host, d, ((size_t)1 << ell) * sizeof(fe), cur_stream());
-      sync_after_unlock(cur_stream());
+      cudaStream_t st = cur_stream();
+      DevBuf<fe> out((size_t)1 << ell, st);
+      eq_evals_from_host<decltype(f)>(r_host, ell, out.p, st);
+      d2h(out_host, out.p, ((size_t)1 << ell) * sizeof(fe), st);
+      sync_after_unlock(st);
     });
-  std::string keep = rc == VDFGPU_OK ? std::string() : std::string(vdfgpu_last_error());
-  guarded([&] { if (d) cudaFree(d); });
-  if (rc != VDFGPU_OK) set_error(keep);
-  return rc;
+  });
 }
 
 int vdfgpu_sumcheck_cubic_dev(int field, void* A_dev, void* B_dev, void* C_dev, void* D_dev, size_t ell,
                               vdfgpu_round_fn round_fn, void* user, void* final_evals4_host) {
-  PolySet P{{reinterpret_cast<fe*>(A_dev), reinterpret_cast<fe*>(B_dev), reinterpret_cast<fe*>(C_dev), reinterpret_cast<fe*>(D_dev)}};
-  return sumcheck_run(field, P, 4, ell, round_fn, user, final_evals4_host);
+  const void* t[4] = {A_dev, B_dev, C_dev, D_dev};
+  return sumcheck(field, t, 4, false, ell, round_fn, user, final_evals4_host);
 }
 
 int vdfgpu_sumcheck_quad_dev(int field, void* A_dev, void* B_dev, size_t ell, vdfgpu_round_fn round_fn, void* user,
                              void* final_evals2_host) {
-  PolySet P{{reinterpret_cast<fe*>(A_dev), reinterpret_cast<fe*>(B_dev), nullptr, nullptr}};
-  return sumcheck_run(field, P, 2, ell, round_fn, user, final_evals2_host);
-}
-
-// host-table forms: upload, run, free
-static int sumcheck_host(int field, const void* const* tables_host, int n_polys, size_t ell, vdfgpu_round_fn fn,
-                         void* user, void* final_host) {
-  if (ell > 30) {
-    set_error("sumcheck: ell too large for the host-table form");
-    return VDFGPU_ERR_ARG;
-  }
-  for (int q = 0; q < n_polys; q++)
-    if (!tables_host[q]) {
-      set_error("sumcheck: null table");
-      return VDFGPU_ERR_ARG;
-    }
-  const size_t bytes = ((size_t)1 << ell) * sizeof(fe);
-  PolySet P{{nullptr, nullptr, nullptr, nullptr}};
-  int rc = guarded([&] {
-    require_ready();
-    for (int q = 0; q < n_polys; q++) {
-      VDF_CUDA_CHECK(cudaMalloc((void**)&P.p[q], bytes));
-      h2d(P.p[q], tables_host[q], bytes, cur_stream());
-    }
-    sync_after_unlock(cur_stream());
-  });
-  if (rc == VDFGPU_OK) rc = sumcheck_run(field, P, n_polys, ell, fn, user, final_host);
-  std::string keep = rc == VDFGPU_OK ? std::string() : std::string(vdfgpu_last_error());
-  guarded([&] {
-    if (ctx().ready) cudaStreamSynchronize(cur_stream());
-    for (int q = 0; q < n_polys; q++)
-      if (P.p[q]) cudaFree(P.p[q]);
-  });
-  if (rc != VDFGPU_OK) set_error(keep);
-  return rc;
+  const void* t[2] = {A_dev, B_dev};
+  return sumcheck(field, t, 2, false, ell, round_fn, user, final_evals2_host);
 }
 
 int vdfgpu_sumcheck_cubic(int field, const void* A_host, const void* B_host, const void* C_host, const void* D_host,
                           size_t ell, vdfgpu_round_fn round_fn, void* user, void* final_evals4_host) {
   const void* t[4] = {A_host, B_host, C_host, D_host};
-  return sumcheck_host(field, t, 4, ell, round_fn, user, final_evals4_host);
+  return sumcheck(field, t, 4, true, ell, round_fn, user, final_evals4_host);
 }
 
 int vdfgpu_sumcheck_quad(int field, const void* A_host, const void* B_host, size_t ell, vdfgpu_round_fn round_fn,
                          void* user, void* final_evals2_host) {
   const void* t[2] = {A_host, B_host};
-  return sumcheck_host(field, t, 2, ell, round_fn, user, final_evals2_host);
+  return sumcheck(field, t, 2, true, ell, round_fn, user, final_evals2_host);
 }
 
 int vdfgpu_poly_evaluate_dev(int field, const void* poly_dev, const void* r_host, size_t ell, void* out_host) {
   return guarded([&] {
-    if (field != VDFGPU_FP && field != VDFGPU_FQ) throw ArgError("poly_evaluate: unknown field");
-    if (!poly_dev || !out_host || (ell && !r_host) || ell > 40) throw ArgError("poly_evaluate: bad arguments");
-    require_ready();
-    cudaStream_t st = cur_stream();
-    CudaLaunch L(st);
-    const size_t n = (size_t)1 << ell;
-    DevBuf<fe> r(ell ? ell : 1, st), eq(n, st), partial((size_t)148 * 8, st), res(1, st);
-    h2d(r.p, r_host, ell * 32, st);
-    ScScratch s;
-    s.partial = partial.p;
-    s.evals = res.p;
-    if (field == VDFGPU_FP) {
-      eq_evals_enqueue<Fp>(L, r.p, ell, eq.p);
-      dot_enqueue<Fp>(st, eq.p, reinterpret_cast<const fe*>(poly_dev), n, s);
-    } else {
-      eq_evals_enqueue<Fq>(L, r.p, ell, eq.p);
-      dot_enqueue<Fq>(st, eq.p, reinterpret_cast<const fe*>(poly_dev), n, s);
-    }
-    ctx().launches += L.launches;
-    d2h(out_host, res.p, sizeof(fe), st);
-    sync_after_unlock(st);
+    with_field(field, "poly_evaluate", [&](auto f) {
+      if (!poly_dev || !out_host || (ell && !r_host) || ell > 40) throw ArgError("poly_evaluate: bad arguments");
+      require_ready();
+      poly_evaluate_enqueue<decltype(f)>(reinterpret_cast<const fe*>(poly_dev), r_host, ell, out_host, cur_stream());
+    });
   });
 }
 
 int vdfgpu_poly_evaluate(int field, const void* poly_host, const void* r_host, size_t ell, void* out_host) {
-  if (!poly_host || ell > 30) {
-    set_error("poly_evaluate: bad arguments");
-    return VDFGPU_ERR_ARG;
-  }
-  fe* d = nullptr;
-  const size_t bytes = ((size_t)1 << ell) * sizeof(fe);
-  int rc = guarded([&] {
-    require_ready();
-    VDF_CUDA_CHECK(cudaMalloc((void**)&d, bytes));
-    h2d(d, poly_host, bytes, cur_stream());
-    sync_after_unlock(cur_stream());
+  return guarded([&] {
+    with_field(field, "poly_evaluate", [&](auto f) {
+      if (!poly_host || !out_host || (ell && !r_host) || ell > 30) throw ArgError("poly_evaluate: bad arguments");
+      require_ready();
+      cudaStream_t st = cur_stream();
+      const size_t bytes = ((size_t)1 << ell) * sizeof(fe);
+      DevBuf<fe> poly((size_t)1 << ell, st);
+      h2d(poly.p, poly_host, bytes, st);
+      poly_evaluate_enqueue<decltype(f)>(poly.p, r_host, ell, out_host, st);
+    });
   });
-  if (rc == VDFGPU_OK) rc = vdfgpu_poly_evaluate_dev(field, d, r_host, ell, out_host);
-  std::string keep = rc == VDFGPU_OK ? std::string() : std::string(vdfgpu_last_error());
-  guarded([&] {
-    if (ctx().ready) cudaStreamSynchronize(cur_stream());
-    if (d) cudaFree(d);
-  });
-  if (rc != VDFGPU_OK) set_error(keep);
-  return rc;
 }
 
 // ---- inner-product-argument building blocks ------------------------------------------------------------------
 int vdfgpu_vec_lincomb(int field, const void* a_host, const void* b_host, size_t n, const void* x32_host,
                        const void* y32_host, void* out_host) {
   return guarded([&] {
-    if (field != VDFGPU_FP && field != VDFGPU_FQ) throw ArgError("vec_lincomb: unknown field");
-    if (!x32_host || !y32_host || (n && (!a_host || !b_host || !out_host))) throw ArgError("vec_lincomb: null pointer");
-    if (!n) return;
-    require_ready();
-    cudaStream_t st = cur_stream();
-    CudaLaunch L(st);
-    DevBuf<fe> a(n, st), b(n, st), o(n, st), xy(2, st);
-    h2d(a.p, a_host, n * 32, st);
-    h2d(b.p, b_host, n * 32, st);
-    h2d(xy.p, x32_host, 32, st);
-    h2d(xy.p + 1, y32_host, 32, st);
-    if (field == VDFGPU_FP) L.run<256>(n, VecLinCombFn<Fp>{a.p, b.p, xy.p, o.p});
-    else L.run<256>(n, VecLinCombFn<Fq>{a.p, b.p, xy.p, o.p});
-    ctx().launches += L.launches;
-    d2h(out_host, o.p, n * 32, st);
-    sync_after_unlock(st);
+    with_field(field, "vec_lincomb", [&](auto f) {
+      if (!x32_host || !y32_host || (n && (!a_host || !b_host || !out_host))) throw ArgError("vec_lincomb: null pointer");
+      if (!n) return;
+      require_ready();
+      cudaStream_t st = cur_stream();
+      CudaLaunch L = api_launch(st);
+      DevBuf<fe> a(n, st), b(n, st), o(n, st), xy(2, st);
+      h2d(a.p, a_host, n * 32, st);
+      h2d(b.p, b_host, n * 32, st);
+      h2d(xy.p, x32_host, 32, st);
+      h2d(xy.p + 1, y32_host, 32, st);
+      L.run<256>(n, VecLinCombFn<decltype(f)>{a.p, b.p, xy.p, o.p});
+      d2h(out_host, o.p, n * 32, st);
+      sync_after_unlock(st);
+    });
   });
 }
 
 int vdfgpu_inner_product(int field, const void* a_host, const void* b_host, size_t n, void* out32_host) {
   return guarded([&] {
-    if (field != VDFGPU_FP && field != VDFGPU_FQ) throw ArgError("inner_product: unknown field");
-    if (!out32_host || (n && (!a_host || !b_host))) throw ArgError("inner_product: null pointer");
-    require_ready();
-    cudaStream_t st = cur_stream();
-    DevBuf<fe> a(n ? n : 1, st), b(n ? n : 1, st), partial((size_t)148 * 8, st), res(1, st);
-    h2d(a.p, a_host, n * 32, st);
-    h2d(b.p, b_host, n * 32, st);
-    ScScratch s;
-    s.partial = partial.p;
-    s.evals = res.p;
-    if (field == VDFGPU_FP) dot_enqueue<Fp>(st, a.p, b.p, n, s);
-    else dot_enqueue<Fq>(st, a.p, b.p, n, s);
-    d2h(out32_host, res.p, sizeof(fe), st);
-    sync_after_unlock(st);
+    with_field(field, "inner_product", [&](auto f) {
+      if (!out32_host || (n && (!a_host || !b_host))) throw ArgError("inner_product: null pointer");
+      require_ready();
+      cudaStream_t st = cur_stream();
+      DevBuf<fe> a(n ? n : 1, st), b(n ? n : 1, st), partial((size_t)148 * 8, st), res(1, st);
+      h2d(a.p, a_host, n * 32, st);
+      h2d(b.p, b_host, n * 32, st);
+      dot_enqueue<decltype(f)>(st, a.p, b.p, n, ScScratch{partial.p, res.p});
+      d2h(out32_host, res.p, sizeof(fe), st);
+      sync_after_unlock(st);
+    });
   });
 }
 
 int vdfgpu_points_lincomb(int curve, const void* P_affine72_host, const void* Q_affine72_host, size_t n,
                           const void* w1_32_host, const void* w2_32_host, void* out_affine72_host) {
   return guarded([&] {
-    if (curve != VDFGPU_PALLAS && curve != VDFGPU_VESTA) throw ArgError("points_lincomb: unknown curve");
-    if (!w1_32_host || !w2_32_host || (n && (!P_affine72_host || !Q_affine72_host || !out_affine72_host)))
-      throw ArgError("points_lincomb: null pointer");
-    if (!n) return;
-    require_ready();
-    cudaStream_t st = cur_stream();
-    CudaLaunch L(st);
-    DevBuf<uint8_t> raw(2 * n * 72, st);
-    DevBuf<affine_t> pq(2 * n, st), out(n, st);
-    DevBuf<fe> w(2, st);
-    h2d(raw.p, P_affine72_host, n * 72, st);
-    h2d(raw.p + n * 72, Q_affine72_host, n * 72, st);
-    h2d(w.p, w1_32_host, 32, st);
-    h2d(w.p + 1, w2_32_host, 32, st);
-    L.run<256>(2 * n, RepackFn{raw.p, pq.p});
-    const size_t threads = (n + 3) / 4;
-    if (curve == VDFGPU_PALLAS) L.run<64>(threads, PointLinCombFn<Pallas, Fp, Fq>{pq.p, pq.p + n, w.p, out.p, n});
-    else L.run<64>(threads, PointLinCombFn<Vesta, Fq, Fp>{pq.p, pq.p + n, w.p, out.p, n});
-    L.run<256>(n, UnpackFn{out.p, raw.p});
-    ctx().launches += L.launches;
-    d2h(out_affine72_host, raw.p, n * 72, st);
-    sync_after_unlock(st);
+    with_curve(curve, "points_lincomb", [&](auto C, auto BF, auto SF) {
+      if (!w1_32_host || !w2_32_host || (n && (!P_affine72_host || !Q_affine72_host || !out_affine72_host)))
+        throw ArgError("points_lincomb: null pointer");
+      if (!n) return;
+      require_ready();
+      cudaStream_t st = cur_stream();
+      CudaLaunch L = api_launch(st);
+      DevBuf<uint8_t> raw(2 * n * 72, st);
+      DevBuf<affine_t> pq(2 * n, st), out(n, st);
+      DevBuf<fe> w(2, st);
+      h2d(raw.p, P_affine72_host, n * 72, st);
+      h2d(raw.p + n * 72, Q_affine72_host, n * 72, st);
+      h2d(w.p, w1_32_host, 32, st);
+      h2d(w.p + 1, w2_32_host, 32, st);
+      L.run<256>(2 * n, RepackFn{raw.p, pq.p});
+      L.run<64>((n + 3) / 4, PointLinCombFn<decltype(C), decltype(BF), decltype(SF)>{pq.p, pq.p + n, w.p, out.p, n});
+      L.run<256>(n, UnpackFn{out.p, raw.p});
+      d2h(out_affine72_host, raw.p, n * 72, st);
+      sync_after_unlock(st);
+    });
   });
 }
 

@@ -169,6 +169,26 @@ inline void d2d(void* dst, const void* src, size_t bytes, cudaStream_t s) {
   if (bytes) VDF_CUDA_CHECK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, s));
 }
 
+// The launch policy of the entry points: every kernel it launches counts in vdfgpu_launch_count().
+inline CudaLaunch api_launch(cudaStream_t s, StageProfile* p = nullptr, Arena* a = nullptr) {
+  return CudaLaunch(s, p, a, &ctx().launches);
+}
+
+// The ABI's field and curve ids as types: `body` (a generic lambda) is called with Fp{} or Fq{}, or with the curve,
+// its coordinate field and its scalar field.  Any other id is an argument error "<who>: unknown field / curve".
+template <class Body>
+decltype(auto) with_field(int field, const char* who, Body&& body) {
+  if (field == VDFGPU_FP) return body(Fp{});
+  if (field == VDFGPU_FQ) return body(Fq{});
+  throw ArgError(std::string(who) + ": unknown field");
+}
+template <class Body>
+decltype(auto) with_curve(int curve, const char* who, Body&& body) {
+  if (curve == VDFGPU_PALLAS) return body(Pallas{}, Fp{}, Fq{});
+  if (curve == VDFGPU_VESTA) return body(Vesta{}, Fq{}, Fp{});
+  throw ArgError(std::string(who) + ": unknown curve");
+}
+
 // wraps a C-ABI body: locks while the body enqueues, waits for the GPU outside the lock, maps exceptions to
 // status codes + thread-local message, leaves the caller's current device as it found it
 template <class Body>

@@ -7,6 +7,7 @@
 //                  be checked against the oracle in a container without a GPU.  Never linked into
 //                  libvdfgpu.so.
 #pragma once
+#include <atomic>
 #include <cstddef>
 #include <cstdint>
 #include <cstdlib>
@@ -300,11 +301,13 @@ struct StageProfile {
 
 struct CudaLaunch {
   cudaStream_t stream;
-  size_t launches = 0;  // kernels launched through this policy (bench.py reports it)
+  size_t launches = 0;  // kernels launched through this policy
   StageProfile* prof = nullptr;
   Arena* arena = nullptr;   // preallocated workspace of this stream; nullptr: stream-ordered pool allocations
+  std::atomic<uint64_t>* total = nullptr;   // also counted here as they launch (vdfgpu_launch_count; bench.py reports it)
 
-  explicit CudaLaunch(cudaStream_t s, StageProfile* p = nullptr, Arena* a = nullptr) : stream(s), prof(p), arena(a) {}
+  explicit CudaLaunch(cudaStream_t s, StageProfile* p = nullptr, Arena* a = nullptr, std::atomic<uint64_t>* t = nullptr)
+      : stream(s), prof(p), arena(a), total(t) {}
 
   // stage boundary: everything enqueued until the next mark belongs to `stage`
   void mark(int stage) {
@@ -339,7 +342,7 @@ struct CudaLaunch {
     size_t blocks = (n + BLOCK - 1) / BLOCK;
     functor_kernel<BLOCK, MINB, Fn><<<(unsigned)blocks, BLOCK, 0, stream>>>(f, n);
     VDF_CUDA_CHECK(cudaGetLastError());
-    launches++;
+    count(1);
   }
 
   // out[0..n] = exclusive prefix sums of in[0..n), out[n] = total
@@ -356,8 +359,14 @@ struct CudaLaunch {
       scan_add_kernel<BLOCK, ITEMS><<<(unsigned)tiles, BLOCK, 0, stream>>>(out, tile_sums, n);
     }
     VDF_CUDA_CHECK(cudaGetLastError());
-    launches += scan_launches(n);
+    count(scan_launches(n));
     free(tile_sums);
+  }
+
+ private:
+  void count(size_t k) {
+    launches += k;
+    if (total) *total += k;
   }
 };
 
