@@ -34,7 +34,8 @@
  * vdfgpu_running_finish may return before its fold has run and the next call may come from another stream or thread.
  * Device buffers the caller passes to "_dev" entry points are ordered by the caller's stream only: whatever writes
  * them on another stream must be made visible to it (an event) before the call.  A handle must not be destroyed while another thread uses it; a generator set or
- * shape held by a running instance cannot be destroyed (VDFGPU_ERR_STATE) until that instance is.
+ * shape held by a running instance (or a set in use by vdfgpu_ipa_prove[_dev]) cannot be destroyed (VDFGPU_ERR_STATE)
+ * until that instance is (that call has returned).
  *
  * Inputs: every 32-byte field element must be the canonical Montgomery image of a value < m, as pasta_curves'
  * from_repr guarantees on the Rust side.  The MinRoot verdict entry points check this themselves (a non-canonical
@@ -270,6 +271,30 @@ int vdfgpu_vec_lincomb(int field, const void* a_host, const void* b_host, size_t
 int vdfgpu_inner_product(int field, const void* a_host, const void* b_host, size_t n, void* out32_host);
 int vdfgpu_points_lincomb(int curve, const void* P_affine72_host, const void* Q_affine72_host, size_t n,
                           const void* w1_32_host, const void* w2_32_host, void* out_affine72_host);
+/* The whole inner-product argument (spartan_with_ipa_pc's polynomial-evaluation argument [R]) on a resident set g:
+ * n = 2^ell; a, b: n elements of the scalar field of g's curve (Montgomery); g holds at least n + 1 points, G_k is
+ * point k and U0 = G_n is nova's gens_c; U = u_scale U0 (nova scales gens_c by a transcript scalar before the rounds;
+ * a caller without that step passes u_scale = 1).  Round j = 0 .. ell-1, m = n / 2^j, h = m / 2:
+ *   c_L = <a[0,h), b[h,m)>, c_R = <a[h,m), b[0,h)>
+ *   L = <a[0,h), G'[h,m)> + c_L U,  R = <a[h,m), G'[0,h)> + c_R U
+ *   round_fn(user, j, L, R, r_out) -- the caller's transcript: absorbs L and R, writes the challenge r != 0
+ *   a <- r a_L + r^-1 a_R,  b <- r^-1 b_L + r b_R,  G' <- r^-1 G'_L + r G'_R
+ * a_hat = a[0] after ell rounds.  L and R are normalised as vdfgpu_msm returns them (identity = 96 zero bytes), for
+ * every set layout including VDFGPU_GENS_RAW_JACOBIAN.  round_fn runs on the calling thread, outside the library's
+ * lock; a non-zero return, r = 0 or a non-canonical r (>= the group order) ends the call with VDFGPU_ERR_STATE.  g
+ * stays referenced for the whole call: vdfgpu_gens_destroy from another thread meanwhile returns VDFGPU_ERR_STATE.  ell = 0: a_hat = a[0], round_fn is not called
+ * (and may be NULL).  The _dev form works on device vectors on the calling thread's stream and consumes them; the host
+ * form takes ell <= 30.
+ * ipa_gens_hat: the verifier's folded generator G_hat = <s, G[0,n)> from the ell challenges (g holds at least n
+ * points), s_k = prod_j (bit_j(k) ? r_j : r_j^-1) with bit_0 the most significant of the ell bits (nova's s); a
+ * challenge that is 0 or non-canonical is VDFGPU_ERR_ARG. */
+typedef int (*vdfgpu_ipa_round_fn)(void* user, size_t round, const void* L_point96, const void* R_point96,
+                                   void* r_out32);
+int vdfgpu_ipa_prove(vdfgpu_gens* g, const void* a_host, const void* b_host, size_t ell, const void* u_scale32_host,
+                     vdfgpu_ipa_round_fn round_fn, void* user, void* a_hat32_host);
+int vdfgpu_ipa_prove_dev(vdfgpu_gens* g, void* a_dev, void* b_dev, size_t ell, const void* u_scale32_host,
+                         vdfgpu_ipa_round_fn round_fn, void* user, void* a_hat32_host);
+int vdfgpu_ipa_gens_hat(vdfgpu_gens* g, const void* r_host, size_t ell, void* out_point96_host);
 
 /* ---- a8: batched MinRoot verification.  Replaces a loop of MinRootVDF::check (src/minroot.rs:369-371)
  * / Evaluation::verify (:424-426) over independent chains.  ok_out[k] = 1 iff

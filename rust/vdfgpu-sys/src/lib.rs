@@ -44,6 +44,12 @@ pub type vdfgpu_round_fn = Option<
     unsafe extern "C" fn(user: *mut c_void, round: size_t, evals_fe32: *const c_void, n_evals: size_t, r_out_fe32: *mut c_void) -> c_int,
 >;
 
+/// Per-round callback of the inner-product argument: receives the round's commitments L and R (96-byte normalised
+/// points, identity = 96 zero bytes), owns the transcript, writes the challenge r != 0 to `r_out32`, returns 0.
+pub type vdfgpu_ipa_round_fn = Option<
+    unsafe extern "C" fn(user: *mut c_void, round: size_t, l_point96: *const c_void, r_point96: *const c_void, r_out32: *mut c_void) -> c_int,
+>;
+
 extern "C" {
     // ---- context
     pub fn vdfgpu_init(device: c_int) -> c_int;
@@ -171,6 +177,13 @@ extern "C" {
                                 out32_host: *mut c_void) -> c_int;
     pub fn vdfgpu_points_lincomb(curve: c_int, p_affine72_host: *const c_void, q_affine72_host: *const c_void, n: size_t,
                                  w1_32_host: *const c_void, w2_32_host: *const c_void, out_affine72_host: *mut c_void) -> c_int;
+    pub fn vdfgpu_ipa_prove(g: *mut vdfgpu_gens, a_host: *const c_void, b_host: *const c_void, ell: size_t,
+                            u_scale32_host: *const c_void, round_fn: vdfgpu_ipa_round_fn, user: *mut c_void,
+                            a_hat32_host: *mut c_void) -> c_int;
+    pub fn vdfgpu_ipa_prove_dev(g: *mut vdfgpu_gens, a_dev: *mut c_void, b_dev: *mut c_void, ell: size_t,
+                                u_scale32_host: *const c_void, round_fn: vdfgpu_ipa_round_fn, user: *mut c_void,
+                                a_hat32_host: *mut c_void) -> c_int;
+    pub fn vdfgpu_ipa_gens_hat(g: *mut vdfgpu_gens, r_host: *const c_void, ell: size_t, out_point96_host: *mut c_void) -> c_int;
 
     // ---- a8: batched MinRoot verification
     pub fn vdfgpu_minroot_check_batch(field: c_int, results_state96_host: *const c_void,

@@ -88,6 +88,9 @@ PROTOTYPES = {
     "vdfgpu_vec_lincomb": (c_int, [c_int, c_void_p, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p]),
     "vdfgpu_inner_product": (c_int, [c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
     "vdfgpu_points_lincomb": (c_int, [c_int, c_void_p, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p]),
+    "vdfgpu_ipa_prove": (c_int, [c_void_p, c_void_p, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vdfgpu_ipa_prove_dev": (c_int, [c_void_p, c_void_p, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vdfgpu_ipa_gens_hat": (c_int, [c_void_p, c_void_p, c_size_t, c_void_p]),
     "vdfgpu_minroot_check_batch": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_uint64, c_size_t, c_void_p]),
     "vdfgpu_minroot_check_batch_dev": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_uint64, c_size_t, c_void_p]),
     "vdfgpu_minroot_inverse_eval_batch": (c_int, [c_int, c_void_p, c_uint64, c_size_t, c_void_p]),
@@ -99,6 +102,8 @@ PROTOTYPES = {
 
 # int (*vdfgpu_round_fn)(void* user, size_t round, const void* evals_fe32, size_t n_evals, void* r_out_fe32)
 ROUND_FN = ctypes.CFUNCTYPE(c_int, c_void_p, c_size_t, c_void_p, c_size_t, c_void_p)
+# int (*vdfgpu_ipa_round_fn)(void* user, size_t round, const void* L_point96, const void* R_point96, void* r_out32)
+IPA_ROUND_FN = ctypes.CFUNCTYPE(c_int, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p)
 
 
 def lib_path() -> Path:

@@ -132,6 +132,17 @@ static void normalise_batch(uint8_t* const* pts, size_t m, int curve) {
 }
 }  // namespace hostfield
 
+static fe host_inv_mod(const fe& a, const hostfield::Mod& f) {
+  uint64_t x[4], r[4];
+  std::memcpy(x, &a, 32);
+  hostfield::inv(r, x, f);
+  fe out;
+  std::memcpy(&out, r, 32);
+  return out;
+}
+fe host_inv(Fp, const fe& a) { return host_inv_mod(a, hostfield::FP_MOD); }
+fe host_inv(Fq, const fe& a) { return host_inv_mod(a, hostfield::FQ_MOD); }
+
 struct PendingNorm { void* p; size_t count; int curve; };
 struct PendingCopy { void* dst; const void* src; size_t bytes; };
 static thread_local std::vector<PendingNorm> t_norms;
@@ -980,7 +991,9 @@ uint32_t vdfgpu_gens_affine_rounds(const vdfgpu_gens* g, size_t n) {
 int vdfgpu_gens_destroy(vdfgpu_gens* g) {
   return guarded([&] {
     if (!g) return;
-    if (g->refs > 0) throw StateError("gens_destroy: a running instance still uses this generator set (destroy it first)");
+    if (g->refs > 0)
+      throw StateError("gens_destroy: a running instance or an inner-product argument in progress still uses this "
+                       "generator set");
     if (ctx().ready) {
       VDF_CUDA_CHECK(cudaSetDevice(ctx().device));
       cudaDeviceSynchronize();   // MSMs on any stream (asynchronous slots, other threads) may still read the points

@@ -172,6 +172,165 @@ static void poly_evaluate_enqueue(const fe* poly_dev, const void* r_host, size_t
   sync_after_unlock(st);
 }
 
+// ---- the inner-product argument (notation: sumcheck.cuh) -------------------------------------------------------
+// a challenge the round loop can use: canonical (< m, so r = m is not a disguised 0) and not 0, which has no inverse
+template <class F>
+static bool usable_challenge(const fe& r) {
+  return F::is_canonical(r) && !F::is_zero(r);
+}
+
+struct IpaScratch {   // per-call device scratch of the IPA round loop (stream-ordered pool allocations)
+  fe* a = nullptr;         // host form only: the uploaded a and b
+  fe* b = nullptr;
+  fe* coef[2] = {nullptr, nullptr};   // coef_j and coef_{j+1}, n entries each
+  fe* S[2] = {nullptr, nullptr};      // SL, SR: n + 1 entries each, the same pointers every round (graph replay)
+  fe* partial = nullptr;   // [grid][2]
+  fe* c = nullptr;         // [2] = (c_L, c_R)
+  jac_t* out = nullptr;    // [2] = (L, R), un-normalised
+  std::vector<void*> all() const { return {a, b, coef[0], coef[1], S[0], S[1], partial, c, out}; }
+};
+
+template <class T>
+static T* pool_alloc(size_t count, cudaStream_t st) {
+  void* p = nullptr;
+  VDF_CUDA_CHECK(cudaMallocAsync(&p, count * sizeof(T) + 16, st));
+  return reinterpret_cast<T*>(p);
+}
+
+// s = coef_0 = [1] into coef[0]
+template <class F>
+static void ipa_coef_init(fe* coef, cudaStream_t st) {
+  const fe one = F::one();
+  h2d(coef, &one, sizeof(fe), st);   // pageable source: staged before cudaMemcpyAsync returns
+}
+
+// Both forms of vdfgpu_ipa_prove.  Like sumcheck(): every guarded() section ends before the caller's round callback
+// runs; a round is (c_L, c_R), the expansion into SL / SR, ONE batched MSM with k = 2 and one 192-byte read-back into
+// pinned memory, normalised on the host after the wait (the transcript absorbs canonical points, whatever the set's
+// flags); the fold takes r and r^-1 by value.  The call holds a reference on g from its first guarded() section to its
+// last, so vdfgpu_gens_destroy from another thread between rounds is refused instead of freeing the points.
+static int ipa_prove(vdfgpu_gens* g, void* a_in, void* b_in, bool on_host, size_t ell, const void* u_scale_host,
+                     vdfgpu_ipa_round_fn fn, void* user, void* a_hat_host) {
+  IpaScratch s;
+  fe u_scale;
+  fe* a = reinterpret_cast<fe*>(a_in);
+  fe* b = reinterpret_cast<fe*>(b_in);
+  const size_t n = ell <= 40 ? (size_t)1 << ell : 0;
+  bool holds_g = false;
+  int rc = guarded([&] {
+    if (!g || !a_in || !b_in || !u_scale_host || !a_hat_host || (ell && !fn)) throw ArgError("ipa_prove: null pointer");
+    if (on_host && ell > 30) throw ArgError("ipa_prove: ell too large for the host-vector form");
+    if (ell > 40 || g->n < n + 1) throw ArgError("ipa_prove: the generator set needs at least 2^ell + 1 points");
+    std::memcpy(&u_scale, u_scale_host, sizeof(fe));
+    require_ready();
+    g->refs++;
+    holds_g = true;
+    cudaStream_t st = cur_stream();
+    if (on_host) {
+      a = s.a = pool_alloc<fe>(n, st);
+      b = s.b = pool_alloc<fe>(n, st);
+      h2d_scalars(a, a_in, n * sizeof(fe), st);
+      h2d_scalars(b, b_in, n * sizeof(fe), st);
+    }
+    for (int q = 0; q < 2; q++) {
+      s.coef[q] = pool_alloc<fe>(n, st);
+      s.S[q] = pool_alloc<fe>(n + 1, st);
+    }
+    s.partial = pool_alloc<fe>((size_t)sc_grid(n / 2) * 2, st);
+    s.c = pool_alloc<fe>(2, st);
+    s.out = pool_alloc<jac_t>(2, st);
+    with_curve(g->curve, "ipa_prove", [&](auto, auto, auto SF) { ipa_coef_init<decltype(SF)>(s.coef[0], st); });
+  });
+  int cur = 0;
+  for (size_t round = 0; rc == VDFGPU_OK && round < ell; round++) {
+    const size_t h = (n >> round) / 2, nc = (size_t)1 << round;
+    uint8_t LR[2][96];
+    fe r, r_inv;
+    rc = guarded([&] {
+      require_ready();
+      cudaStream_t st = cur_stream();
+      with_curve(g->curve, "ipa_prove", [&](auto, auto, auto SF) {
+        using F = decltype(SF);
+        const uint32_t grid = sc_grid(h);
+        sc_cross_dot_kernel<F><<<grid, SC_BLOCK, 0, st>>>(a, b, h, s.partial);
+        sc_final_kernel<F, 2><<<1, SC_BLOCK, 0, st>>>(s.partial, grid, s.c);
+        VDF_CUDA_CHECK(cudaGetLastError());
+        ctx().launches += 2;
+        CudaLaunch L = api_launch(st);
+        L.run<256>(n + 1, IpaExpandFn<F>{a, s.coef[cur], s.c, u_scale, (uint32_t)(ell - round), n, s.S[0], s.S[1]});
+      });
+      const fe* vecs[2] = {s.S[0], s.S[1]};
+      const size_t lens[2] = {n + 1, n + 1};
+      msm_batch_on_device(g, vecs, lens, 2, s.out, true);
+      fe* pin = pinned_evals();
+      d2h(pin, s.out, 2 * sizeof(jac_t), st);
+      sync_after_unlock(st);
+      copy_after_sync(LR, pin, sizeof(LR));
+      normalise_after_sync(LR, 2, g->curve);
+    });
+    if (rc != VDFGPU_OK) break;
+    if (fn(user, round, LR[0], LR[1], &r) != 0) {   // the caller's transcript: outside the lock
+      set_error("ipa_prove: the round callback failed");
+      rc = VDFGPU_ERR_STATE;
+      break;
+    }
+    if (!with_curve(g->curve, "ipa_prove", [&](auto, auto, auto SF) { return usable_challenge<decltype(SF)>(r); })) {
+      set_error("ipa_prove: the round callback returned 0 or a non-canonical challenge");
+      rc = VDFGPU_ERR_STATE;
+      break;
+    }
+    rc = guarded([&] {
+      require_ready();
+      CudaLaunch L = api_launch(cur_stream());
+      with_curve(g->curve, "ipa_prove", [&](auto, auto, auto SF) {
+        using F = decltype(SF);
+        r_inv = host_inv(SF, r);
+        L.run<256>(h > nc ? h : nc, IpaFoldFn<F>{a, b, h, s.coef[cur], s.coef[cur ^ 1], nc, r, r_inv});
+      });
+    });
+    cur ^= 1;
+  }
+  if (rc == VDFGPU_OK)
+    rc = guarded([&] {
+      require_ready();
+      cudaStream_t st = cur_stream();
+      fe* pin = pinned_evals();
+      d2h(pin, a, sizeof(fe), st);
+      sync_after_unlock(st);
+      copy_after_sync(a_hat_host, pin, sizeof(fe));
+    });
+  std::string keep = rc == VDFGPU_OK ? std::string() : std::string(vdfgpu_last_error());
+  guarded([&] {
+    if (holds_g) g->refs--;
+    if (!ctx().ready) return;
+    for (void* p : s.all())
+      if (p) cudaFreeAsync(p, cur_stream());
+  });
+  if (rc != VDFGPU_OK) set_error(keep);
+  return rc;
+}
+
+// G_hat = <s, G[0, 2^ell)>: the s table by ell doubling launches of IpaFoldFn, then one MSM, normalised on the host
+template <class F>
+static void ipa_gens_hat_enqueue(vdfgpu_gens* g, const fe* r, const fe* r_inv, size_t ell, void* out_host) {
+  cudaStream_t st = cur_stream();
+  CudaLaunch L = api_launch(st);
+  const size_t n = (size_t)1 << ell;
+  DevBuf<fe> t0(n, st), t1(n, st);
+  DevBuf<jac_t> out(1, st);
+  fe* coef[2] = {t0.p, t1.p};
+  ipa_coef_init<F>(coef[0], st);
+  for (size_t j = 0; j < ell; j++)
+    L.run<256>((size_t)1 << j, IpaFoldFn<F>{nullptr, nullptr, 0, coef[j & 1], coef[(j & 1) ^ 1], (size_t)1 << j, r[j],
+                                              r_inv[j]});
+  msm_on_device(g, 0, coef[ell & 1], n, out.p, true, st, true);
+  fe* pin = pinned_evals();
+  d2h(pin, out.p, sizeof(jac_t), st);
+  sync_after_unlock(st);
+  copy_after_sync(out_host, pin, sizeof(jac_t));
+  normalise_after_sync(out_host, 1, g->curve);
+}
+
 }  // namespace vdf
 
 using namespace vdf;
@@ -313,6 +472,34 @@ int vdfgpu_points_lincomb(int curve, const void* P_affine72_host, const void* Q_
       L.run<256>(n, UnpackFn{out.p, raw.p});
       d2h(out_affine72_host, raw.p, n * 72, st);
       sync_after_unlock(st);
+    });
+  });
+}
+
+// ---- the inner-product argument on a resident generator set ----------------------------------------------------
+int vdfgpu_ipa_prove(vdfgpu_gens* g, const void* a_host, const void* b_host, size_t ell, const void* u_scale32_host,
+                     vdfgpu_ipa_round_fn round_fn, void* user, void* a_hat32_host) {
+  return ipa_prove(g, const_cast<void*>(a_host), const_cast<void*>(b_host), true, ell, u_scale32_host, round_fn, user,
+                   a_hat32_host);
+}
+
+int vdfgpu_ipa_prove_dev(vdfgpu_gens* g, void* a_dev, void* b_dev, size_t ell, const void* u_scale32_host,
+                         vdfgpu_ipa_round_fn round_fn, void* user, void* a_hat32_host) {
+  return ipa_prove(g, a_dev, b_dev, false, ell, u_scale32_host, round_fn, user, a_hat32_host);
+}
+
+int vdfgpu_ipa_gens_hat(vdfgpu_gens* g, const void* r_host, size_t ell, void* out_point96_host) {
+  return guarded([&] {
+    if (!g || !out_point96_host || (ell && !r_host)) throw ArgError("ipa_gens_hat: null pointer");
+    if (ell > 40 || g->n < (size_t)1 << ell) throw ArgError("ipa_gens_hat: the generator set needs at least 2^ell points");
+    std::vector<fe> r(ell ? ell : 1), r_inv(ell ? ell : 1);
+    if (ell) std::memcpy(r.data(), r_host, ell * sizeof(fe));
+    with_curve(g->curve, "ipa_gens_hat", [&](auto, auto, auto SF) {
+      for (size_t j = 0; j < ell; j++)
+        if (!usable_challenge<decltype(SF)>(r[j])) throw ArgError("ipa_gens_hat: a challenge is 0 or non-canonical");
+      for (size_t j = 0; j < ell; j++) r_inv[j] = host_inv(SF, r[j]);
+      require_ready();
+      ipa_gens_hat_enqueue<decltype(SF)>(g, r.data(), r_inv.data(), ell, out_point96_host);
     });
   });
 }

@@ -226,7 +226,8 @@ struct vdfgpu_gens {
   uint32_t c = 0;          // window bits of the table (table mode)
   uint32_t W = 0;          // levels stored (1 in plain mode)
   vdf::affine_t* pts = nullptr;  // [W][n]
-  int refs = 0;            // running instances holding this set (vdfgpu_gens_destroy refuses while > 0)
+  int refs = 0;            // running instances and IPA calls in progress holding this set (vdfgpu_gens_destroy refuses
+                           // while > 0)
 };
 
 // internal cross-TU entry: MSM over device scalars into a device point, on the calling thread's stream
@@ -247,4 +248,7 @@ void normalise_after_sync(void* host_ptr, size_t count, int curve);
 // with ONE asynchronous copy and are handed to the caller's (usually pageable) pointers on the host
 void copy_after_sync(void* dst, const void* src, size_t bytes);
 bool host_normalise_wanted(const vdfgpu_gens* g);
+// a^-1 in Montgomery form, computed on the host (a != 0): the per-round challenge inverse of the IPA
+fe host_inv(Fp, const fe& a);
+fe host_inv(Fq, const fe& a);
 }

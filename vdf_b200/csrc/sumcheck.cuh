@@ -90,6 +90,67 @@ struct PointLinCombFn {
   }
 };
 
+// ---- the whole inner-product argument on a resident generator set (vdfgpu_ipa_prove, vdfgpu_ipa_gens_hat) ----------
+// n = 2^ell; a, b in the scalar field of g's curve (Montgomery); g holds at least n + 1 points, G_k = point k, and
+// U0 = G_n is nova's gens_c; U = u_scale U0 (nova scales gens_c by a transcript scalar first, gens_c.scale(&r) [R]).
+// Round j = 0 .. ell-1, m = n / 2^j, h = m / 2:
+//   c_L = <a[0,h), b[h,m)>,  c_R = <a[h,m), b[0,h)>
+//   L = <a[0,h), G'[h,m)> + c_L U,  R = <a[h,m), G'[0,h)> + c_R U;  the caller's transcript turns (L, R) into r != 0
+//   a <- r a_L + r^-1 a_R,  b <- r^-1 b_L + r b_R,  G' <- r^-1 G'_L + r G'_R;   a_hat = a[0] after ell rounds.
+// s_k = prod_j (bit_j(k) ? r_j : r_j^-1), bit_0 the most significant of the ell bits (nova's s), G_hat = <s, G[0,n)>.
+// The generators are never folded: G'_j[i] = sum_t coef_j[t] G[t m + i] with coef_0 = [1],
+// coef_{j+1}[2t + beta] = coef_j[t] (beta ? r_j : r_j^-1), so coef_ell = s, and L and R are ONE batched MSM over the
+// original resident set with the scalars IpaExpandFn writes.  Folding n points per round instead is a 256-bit
+// double-and-add per output (PointLinCombFn, ~4 500 multiplications each) plus a plain-layout MSM per round.
+
+// Round j's commitment scalars over G[0, n], k = t m + i (i < m, m = 2^log_m, h = m / 2), index space n + 1:
+//   SL[k] = a[i - h] coef[t] if i >= h else 0,  SR[k] = a[i + h] coef[t] if i < h else 0,
+//   SL[n] = c[0] u_scale,  SR[n] = c[1] u_scale       (c = (c_L, c_R), on the device)
+template <class F>
+struct IpaExpandFn {
+  const fe* a; const fe* coef; const fe* c;
+  fe u_scale;
+  uint32_t log_m;
+  size_t n;
+  fe* SL; fe* SR;
+  VDF_HD void operator()(size_t k) const {
+    if (k == n) {
+      fe_store(SL + n, F::mul(fe_load(c), u_scale));
+      fe_store(SR + n, F::mul(fe_load(c + 1), u_scale));
+      return;
+    }
+    const size_t h = (size_t)1 << (log_m - 1), i = k & ((h << 1) - 1);
+    const bool left = i < h;
+    const fe v = F::mul(fe_load(a + (left ? i + h : i - h)), fe_load(coef + (k >> log_m)));
+    fe_store(SL + k, left ? F::zero() : v);
+    fe_store(SR + k, left ? v : F::zero());
+  }
+};
+
+// The fold of one round, index space max(h, nc):
+//   a[i] <- r a[i] + r^-1 a[h + i],  b[i] <- r^-1 b[i] + r b[h + i]        for i < h (in place)
+//   coef_out[2t] = coef_in[t] r^-1,  coef_out[2t + 1] = coef_in[t] r      for t < nc
+// With h = 0 it only doubles coef (the s table of vdfgpu_ipa_gens_hat).
+template <class F>
+struct IpaFoldFn {
+  fe* a; fe* b;
+  size_t h;
+  const fe* coef_in; fe* coef_out;
+  size_t nc;
+  fe r, r_inv;
+  VDF_HD void operator()(size_t i) const {
+    if (i < h) {
+      fe_store(a + i, F::add(F::mul(r, fe_load(a + i)), F::mul(r_inv, fe_load(a + h + i))));
+      fe_store(b + i, F::add(F::mul(r_inv, fe_load(b + i)), F::mul(r, fe_load(b + h + i))));
+    }
+    if (i < nc) {
+      const fe c = fe_load(coef_in + i);
+      fe_store(coef_out + 2 * i, F::mul(c, r_inv));
+      fe_store(coef_out + 2 * i + 1, F::mul(c, r));
+    }
+  }
+};
+
 constexpr int SC_BLOCK = 256;
 constexpr int SC_MAX_POLYS = 4;
 
@@ -227,6 +288,17 @@ __global__ void __launch_bounds__(SC_BLOCK) sc_dot_kernel(const fe* A, const fe*
   for (size_t i = (size_t)blockIdx.x * SC_BLOCK + threadIdx.x; i < n; i += (size_t)gridDim.x * SC_BLOCK)
     acc[0] = F::add(acc[0], F::mul(fe_load(A + i), fe_load(B + i)));
   block_sum_store<F, 1>(acc, partial);
+}
+
+// (<A[0,h), B[h,2h)>, <A[h,2h), B[0,h)>), the IPA's (c_L, c_R): per-block partials
+template <class F>
+__global__ void __launch_bounds__(SC_BLOCK) sc_cross_dot_kernel(const fe* A, const fe* B, size_t half, fe* partial) {
+  fe acc[2] = {F::zero(), F::zero()};
+  for (size_t i = (size_t)blockIdx.x * SC_BLOCK + threadIdx.x; i < half; i += (size_t)gridDim.x * SC_BLOCK) {
+    acc[0] = F::add(acc[0], F::mul(fe_load(A + i), fe_load(B + half + i)));
+    acc[1] = F::add(acc[1], F::mul(fe_load(A + half + i), fe_load(B + i)));
+  }
+  block_sum_store<F, 2>(acc, partial);
 }
 
 // second stage: out[a] = sum over blocks of partial[block * NACC + a]; one block

@@ -99,3 +99,66 @@ def points_lincomb(curve: int, P: bytes, Q: bytes, w1: int, w2: int) -> bytes:
                                                  _lib.as_ptr(fe_to_bytes(w1, order)), _lib.as_ptr(fe_to_bytes(w2, order)), _lib.as_ptr(out)))
     return bytes(out)
 
+
+
+# ---- the whole inner-product argument on a resident generator set -----------------------------------------------
+IpaChallenge = Callable[[int, bytes, bytes], int]
+
+
+def _ipa_trampoline(order: int, challenge: IpaChallenge, log: list):
+    def fn(_user, rnd, L_ptr, R_ptr, r_out):
+        try:
+            L, R = ctypes.string_at(L_ptr, 96), ctypes.string_at(R_ptr, 96)
+            r = challenge(int(rnd), L, R) % order
+            log.append((L, R, r))
+            ctypes.memmove(r_out, fe_to_bytes(r, order), 32)
+            return 0
+        except Exception:   # surfaces as VDFGPU_ERR_STATE
+            return 1
+    return _lib.IPA_ROUND_FN(fn)
+
+
+def _ipa_call(gens, fn_name: str, a_arg, b_arg, ell: int, u_scale: int, challenge: IpaChallenge):
+    from .encoding import CURVE_ORDER
+    order = CURVE_ORDER[gens.curve]
+    log: list = []
+    cb = _ipa_trampoline(order, challenge, log)
+    a_hat = bytearray(32)
+    _lib.check(getattr(_lib.load(), fn_name)(gens._h, a_arg, b_arg, ell, _lib.as_ptr(fe_to_bytes(u_scale, order)),
+                                             ctypes.cast(cb, ctypes.c_void_p), None, _lib.as_ptr(a_hat)))
+    return [L for L, _, _ in log], [R for _, R, _ in log], [r for _, _, r in log], fe_from_bytes(bytes(a_hat), order)
+
+
+def ipa_prove(gens, a: Sequence[int], b: Sequence[int], u_scale: int, challenge: IpaChallenge):
+    """The inner-product argument over 2^ell-entry vectors a, b on the resident set `gens` (at least 2^ell + 1 points;
+    U = u_scale * gens[2^ell]).  challenge(round, L, R) is the caller's transcript: it receives the round's commitments
+    as 96-byte normalised points and returns r != 0.  Returns (L list, R list, challenges, a_hat)."""
+    from .encoding import CURVE_ORDER
+    order = CURVE_ORDER[gens.curve]
+    n = len(a)
+    ell = n.bit_length() - 1
+    if n != 1 << ell or len(b) != n:
+        raise ValueError("ipa_prove: a and b need the same power-of-two length")
+    return _ipa_call(gens, "vdfgpu_ipa_prove", _lib.as_ptr(fes_to_bytes(a, order)), _lib.as_ptr(fes_to_bytes(b, order)),
+                     ell, u_scale, challenge)
+
+
+def ipa_prove_dev(gens, a_dev, b_dev, u_scale: int, challenge: IpaChallenge):
+    """ipa_prove on device vectors (CUDA tensors of 32-byte Montgomery elements, consumed) on the calling thread's
+    stream."""
+    nbytes = a_dev.numel() * a_dev.element_size()
+    n = nbytes // 32
+    ell = n.bit_length() - 1
+    if nbytes % 32 or n != 1 << ell or b_dev.numel() * b_dev.element_size() != nbytes:
+        raise ValueError("ipa_prove_dev: a and b need the same power-of-two number of elements")
+    return _ipa_call(gens, "vdfgpu_ipa_prove_dev", a_dev.data_ptr(), b_dev.data_ptr(), ell, u_scale, challenge)
+
+
+def ipa_gens_hat(gens, r: Sequence[int]) -> bytes:
+    """The verifier's folded generator G_hat = <s, gens[0, 2^len(r))> as a 96-byte normalised point."""
+    from .encoding import CURVE_ORDER
+    order = CURVE_ORDER[gens.curve]
+    out = bytearray(96)
+    _lib.check(_lib.load().vdfgpu_ipa_gens_hat(gens._h, _lib.as_ptr(fes_to_bytes(r, order) or bytes(32)), len(r),
+                                               _lib.as_ptr(out)))
+    return bytes(out)
