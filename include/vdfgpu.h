@@ -39,7 +39,7 @@
  *
  * Inputs: every 32-byte field element must be the canonical Montgomery image of a value < m, as pasta_curves'
  * from_repr guarantees on the Rust side.  The MinRoot verdict entry points check this themselves (a non-canonical
- * State gives ok = 0); the other entry points do not.
+ * State gives ok = 0), and so does vdfgpu_ipa_verify_batch for its proofs; the other entry points do not.
  *
  * Limits: point references are 31 bits, so windows * points of one generator set must stay below 2^31 (a table
  * set of 2^26 points x 13 levels uses 41 %); shard larger sets by point range (vdfgpu_msm_range_dev / one set per
@@ -295,6 +295,32 @@ int vdfgpu_ipa_prove(vdfgpu_gens* g, const void* a_host, const void* b_host, siz
 int vdfgpu_ipa_prove_dev(vdfgpu_gens* g, void* a_dev, void* b_dev, size_t ell, const void* u_scale32_host,
                          vdfgpu_ipa_round_fn round_fn, void* user, void* a_hat32_host);
 int vdfgpu_ipa_gens_hat(vdfgpu_gens* g, const void* r_host, size_t ell, void* out_point96_host);
+/* ipa_verify_batch: verifies k inner-product arguments over the same set g (at least 2^ell + 1 points, U0 = G_n) in
+ * one call.  Proof q: comm_a[q] (the commitment to a), L[q][j] and R[q][j] (j < ell, proof-major), a_hat[q]; its
+ * instance: c[q] = <a, b>, b_hat[q] = <b, s_q>, u_scale[q] (U = u_scale U0); r[q][j]: the challenges the caller's
+ * transcript derived from L and R.  Proof q is valid iff
+ *   a_hat G_hat + u_scale (a_hat b_hat - c) U0 - comm_a - sum_j (r_j^2 L_j + r_j^-2 R_j) = O,   G_hat = <s_q, G[0,n)>
+ * (nova's InnerProductArgument::verify with P = comm_a + c U), s_q as for ipa_gens_hat.  b_hat is an input because b
+ * is the caller's: for b = eq(x), b_hat = prod_j ((1 - x_j) r_j^-1 + x_j r_j); for b = sum_i rho_i eq(x_i) (two
+ * evaluation claims folded into one) the sum of those terms; a table shorter than 2^ell, zero-padded at the top, is
+ * eq over x with leading zero coordinates.  Points are 96-byte Jacobian (X, Y, Z), normalised or not; the identity is
+ * Z = 0 (96 zero bytes, as vdfgpu_msm returns it).  Scalars are 32-byte Montgomery in g's scalar field.
+ * The k equations are checked as ONE weighted sum, sum_q w_q (equation q) = O: one MSM over G[0, n] and one over the
+ * k (2 ell + 1) caller points.  If that sum is not O, each proof is checked alone (MSMs in batches of four: about k/4
+ * extra MSM passes over the set, paid only by a failing batch).  ok_out[q] = 1 iff proof q is valid; the verdicts
+ * fail closed: whenever the call returns an error, every ok_out[q] it could write is 0.
+ * Verdicts and errors: a malformed proof is a verdict, not an error -- a point with a coordinate >= p or off
+ * y^2 = x^3 + 5, or a non-canonical a_hat, c, b_hat or u_scale gives ok_out[q] = 0 for that proof only and leaves it
+ * out of the weighted sum.  VDFGPU_ERR_ARG, before any device work: a null pointer, k = 0, ell > 40, fewer than
+ * 2^ell + 1 points in g, a challenge that is 0 or >= the group order, a weight that is 0 or >= the group order.
+ * Soundness: the weights must be uniform and unpredictable to whoever produced the proofs (the OS CSPRNG, e.g.
+ * OsRng); a batch that contains an invalid proof then passes with probability at most 1 / order.  Weights the prover
+ * can predict let two invalid proofs cancel.  The library never generates weights.  g stays referenced for the call,
+ * which runs on the calling thread's stream. */
+int vdfgpu_ipa_verify_batch(vdfgpu_gens* g, size_t ell, size_t k, const void* comm_a96_host, const void* L96_host,
+                            const void* R96_host, const void* r32_host, const void* a_hat32_host, const void* c32_host,
+                            const void* b_hat32_host, const void* u_scale32_host, const void* w32_host,
+                            uint8_t* ok_out_host);
 
 /* ---- a8: batched MinRoot verification.  Replaces a loop of MinRootVDF::check (src/minroot.rs:369-371)
  * / Evaluation::verify (:424-426) over independent chains.  ok_out[k] = 1 iff

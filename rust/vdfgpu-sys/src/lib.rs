@@ -184,6 +184,10 @@ extern "C" {
                                 u_scale32_host: *const c_void, round_fn: vdfgpu_ipa_round_fn, user: *mut c_void,
                                 a_hat32_host: *mut c_void) -> c_int;
     pub fn vdfgpu_ipa_gens_hat(g: *mut vdfgpu_gens, r_host: *const c_void, ell: size_t, out_point96_host: *mut c_void) -> c_int;
+    pub fn vdfgpu_ipa_verify_batch(g: *mut vdfgpu_gens, ell: size_t, k: size_t, comm_a96_host: *const c_void,
+                                   l96_host: *const c_void, r96_host: *const c_void, r32_host: *const c_void,
+                                   a_hat32_host: *const c_void, c32_host: *const c_void, b_hat32_host: *const c_void,
+                                   u_scale32_host: *const c_void, w32_host: *const c_void, ok_out_host: *mut u8) -> c_int;
 
     // ---- a8: batched MinRoot verification
     pub fn vdfgpu_minroot_check_batch(field: c_int, results_state96_host: *const c_void,

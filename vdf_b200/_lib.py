@@ -91,6 +91,7 @@ PROTOTYPES = {
     "vdfgpu_ipa_prove": (c_int, [c_void_p, c_void_p, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_void_p]),
     "vdfgpu_ipa_prove_dev": (c_int, [c_void_p, c_void_p, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_void_p]),
     "vdfgpu_ipa_gens_hat": (c_int, [c_void_p, c_void_p, c_size_t, c_void_p]),
+    "vdfgpu_ipa_verify_batch": (c_int, [c_void_p, c_size_t, c_size_t] + [c_void_p] * 10),
     "vdfgpu_minroot_check_batch": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_uint64, c_size_t, c_void_p]),
     "vdfgpu_minroot_check_batch_dev": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_uint64, c_size_t, c_void_p]),
     "vdfgpu_minroot_inverse_eval_batch": (c_int, [c_int, c_void_p, c_uint64, c_size_t, c_void_p]),

@@ -507,10 +507,10 @@ static uint64_t mix64(uint64_t h, uint64_t v) {
 // runs `enqueue(L)` either directly or, for small plans on an arena, as a cached CUDA graph
 template <class Enqueue>
 static void msm_dispatch(vdfgpu_gens* g, const MsmPlan& p, Workspace* w, cudaStream_t st, const ScalarSet& ss,
-                         const void* pts, const void* d_out, Enqueue enqueue) {
+                         const void* pts, const void* d_out, bool replay, Enqueue enqueue) {
   Context& c = ctx();
   const size_t E = (size_t)p.n * p.W * p.batch;
-  if (!w || !graphs_enabled() || c.prof.enabled || E > GRAPH_MAX_ENTRIES) {
+  if (!replay || !w || !graphs_enabled() || c.prof.enabled || E > GRAPH_MAX_ENTRIES) {
     CudaLaunch L = api_launch(st, &c.prof, w ? &w->arena : nullptr);
     enqueue(L);
     return;
@@ -570,7 +570,7 @@ static void msm_dispatch(vdfgpu_gens* g, const MsmPlan& p, Workspace* w, cudaStr
 }
 
 void msm_on_device(vdfgpu_gens* g, size_t first, const fe* d_scalars, size_t n, jac_t* d_out, bool is_mont,
-                   cudaStream_t stream, bool raw) {
+                   cudaStream_t stream, bool raw, bool replay) {
   if (first + n > g->n) throw ArgError("msm: more scalars than generators");
   Context& c = ctx();
   cudaStream_t st = stream ? stream : cur_stream();
@@ -581,7 +581,7 @@ void msm_on_device(vdfgpu_gens* g, size_t first, const fe* d_scalars, size_t n, 
   Workspace* w = n ? plan_workspace(g->curve, p, st) : nullptr;
   const affine_t* pts = g->pts + first;
   ScalarSet ss{{d_scalars, nullptr, nullptr, nullptr}};
-  msm_dispatch(g, p, w, st, ss, pts, d_out, [&](CudaLaunch& L) {
+  msm_dispatch(g, p, w, st, ss, pts, d_out, replay, [&](CudaLaunch& L) {
     with_curve(g->curve, "msm", [&](auto C, auto, auto SF) {
       msm_run<CudaLaunch, decltype(C), decltype(SF)>(L, p, pts, ss, d_out);
     });
@@ -634,7 +634,7 @@ void msm_host_chunked(vdfgpu_gens* g, const void* h_scalars, size_t n, jac_t* d_
 // k scalar vectors over the same generators in ONE pass of the pipeline (one bucket set per vector):
 // the latency of one MSM for k commitments.  d_out receives k points.
 void msm_batch_on_device(vdfgpu_gens* g, const fe* const* d_scalars, const size_t* lens, uint32_t k, jac_t* d_out,
-                         bool raw) {
+                         bool raw, bool replay) {
   if (k == 0 || k > MSM_MAX_BATCH) throw ArgError("msm_batch: batch size must be 1..4");
   size_t n = 0;
   for (uint32_t j = 0; j < k; j++) {
@@ -654,7 +654,7 @@ void msm_batch_on_device(vdfgpu_gens* g, const fe* const* d_scalars, const size_
   }
   Workspace* w = n ? plan_workspace(g->curve, p, st) : nullptr;
   const affine_t* pts = g->pts;
-  msm_dispatch(g, p, w, st, ss, pts, d_out, [&](CudaLaunch& L) {
+  msm_dispatch(g, p, w, st, ss, pts, d_out, replay, [&](CudaLaunch& L) {
     with_curve(g->curve, "msm", [&](auto C, auto, auto SF) {
       msm_run<CudaLaunch, decltype(C), decltype(SF)>(L, p, pts, ss, d_out);
     });

@@ -2,6 +2,7 @@
 // src/nova/proof.rs:360-368 -> nova-snark 0.8 spartan_with_ipa_pc [R]).  Contract: include/vdfgpu.h.
 // The interactive part of a sum-check (absorb the round polynomial into the transcript, squeeze the challenge) is
 // host work that belongs to the caller: it is a callback invoked once per round, outside the library's lock.
+#include <algorithm>
 #include <cstring>
 #include <vector>
 
@@ -31,10 +32,11 @@ struct ScScratch {   // per-call device scratch of the round loop (stream-ordere
 
 // Pinned landing zone of the per-round read-backs, one per calling thread: at Nova sizes a round is two small kernels,
 // so what a round costs is the round trip to the caller's transcript -- a pageable 96-byte copy is staged by the driver
-// (about 10 us), a pinned one is a plain DMA.
+// (about 10 us), a pinned one is a plain DMA.  24 elements: the eight points a chunk of vdfgpu_ipa_verify_batch's
+// single-proof checks reads back.
 static fe* pinned_evals() {
   static thread_local fe* p = nullptr;
-  if (!p) VDF_CUDA_CHECK(cudaHostAlloc((void**)&p, 8 * sizeof(fe), cudaHostAllocDefault));
+  if (!p) VDF_CUDA_CHECK(cudaHostAlloc((void**)&p, 24 * sizeof(fe), cudaHostAllocDefault));
   return p;
 }
 
@@ -331,6 +333,291 @@ static void ipa_gens_hat_enqueue(vdfgpu_gens* g, const fe* r, const fe* r_inv, s
   normalise_after_sync(out_host, 1, g->curve);
 }
 
+// ---- batch verification of inner-product arguments (notation: sumcheck.cuh) ---------------------------------------
+struct IpaVerifyArgs {   // the caller's arrays, as vdfgpu_ipa_verify_batch takes them
+  const uint8_t* comm; const uint8_t* L; const uint8_t* R;   // 96-byte Jacobian points
+  const fe* r; const fe* a_hat; const fe* c; const fe* b_hat; const fe* u_scale; const fe* w;
+};
+
+// What the host derives from the well-formed proofs ("active", in order, ka of them; per = 2 ell + 1 points each)
+struct IpaVerifyPlan {
+  std::vector<size_t> active;
+  std::vector<fe> rr;             // r [ka][ell], then r^-1 [ka][ell], then w a_hat [ka]: the IpaHalfTablesFn inputs
+  std::vector<fe> last;           // [ka] w u_scale (a_hat b_hat - c): S[n] of proof q alone; the batch's is their sum
+  std::vector<uint8_t> pts72;     // [ka][per] comm_a, L_0 .. L_{ell-1}, R_0 .. R_{ell-1} as 72-byte affine records
+  std::vector<fe> small;          // [ka][per] their scalars -w, -w r_j^2, -w r_j^-2
+};
+
+struct IpaVerifyScratch {   // device buffers of one call, kept for the single-proof checks of a failing batch
+  fe* rr = nullptr;
+  fe* tables = nullptr;     // all Hi tables, then all Lo tables
+  fe* S = nullptr;          // n + 1: the batch
+  fe* small = nullptr;      // ka per: the batch
+  uint8_t* raw = nullptr;   // the 72-byte records, repacked into pts
+  affine_t* pts = nullptr;
+  jac_t* out = nullptr;     // [2 MSM_MAX_BATCH + 1]
+  fe* S4 = nullptr;         // MSM_MAX_BATCH (n + 1), MSM_MAX_BATCH ka per: the single-proof checks, allocated only
+  fe* small4 = nullptr;     // when the batch fails
+  std::vector<void*> all() const { return {rr, tables, S, small, raw, pts, out, S4, small4}; }
+};
+
+// v[i] <- v[i]^-1 for non-zero v with ONE inversion (Montgomery's trick)
+template <class F>
+static void batch_invert(std::vector<fe>& v) {
+  if (v.empty()) return;
+  std::vector<fe> pre(v.size());
+  fe acc = F::one();
+  for (size_t i = 0; i < v.size(); i++) {
+    pre[i] = acc;
+    acc = F::mul(acc, v[i]);
+  }
+  fe inv = host_inv(F{}, acc);
+  for (size_t i = v.size(); i-- > 0;) {
+    const fe vi = v[i];
+    v[i] = F::mul(inv, pre[i]);
+    inv = F::mul(inv, vi);
+  }
+}
+
+// The host half of the call: the well-formed proofs (the others keep verdict 0), their points checked on the curve and
+// written as affine records (one batched inversion for every Z other than 0 and 1; L and R from vdfgpu_ipa_prove have
+// Z = 1), r^-1 by one batched inversion, and the scalars of both MSMs.  Challenges and weights were checked by the
+// caller.
+template <class BF, class SF>
+static IpaVerifyPlan ipa_verify_prepare(size_t ell, size_t k, const IpaVerifyArgs& a) {
+  std::vector<uint8_t> good(k);   // well-formed so far
+  const size_t per = 2 * ell + 1;
+  const fe one = BF::one(), b = BF::add(BF::add(BF::add(one, one), BF::add(one, one)), one);   // y^2 = x^3 + 5
+  auto point = [&](size_t q, size_t i) -> const uint8_t* {
+    return i == 0 ? a.comm + 96 * q : i <= ell ? a.L + 96 * (q * ell + i - 1) : a.R + 96 * (q * ell + i - 1 - ell);
+  };
+  std::vector<fe> X(k * per), Y(k * per), Z(k * per), zi;
+  std::vector<size_t> zi_at;
+  for (size_t q = 0; q < k; q++) {
+    good[q] = SF::is_canonical(a.a_hat[q]) && SF::is_canonical(a.c[q]) && SF::is_canonical(a.b_hat[q]) &&
+            SF::is_canonical(a.u_scale[q]);
+    for (size_t i = 0; good[q] && i < per; i++) {
+      const size_t at = q * per + i;
+      std::memcpy(&X[at], point(q, i), 32);
+      std::memcpy(&Y[at], point(q, i) + 32, 32);
+      std::memcpy(&Z[at], point(q, i) + 64, 32);
+      good[q] = BF::is_canonical(X[at]) && BF::is_canonical(Y[at]) && BF::is_canonical(Z[at]);
+      if (good[q] && !BF::is_zero(Z[at]) && !BF::eq(Z[at], one)) {
+        zi.push_back(Z[at]);
+        zi_at.push_back(at);
+      }
+    }
+  }
+  batch_invert<BF>(zi);
+  for (size_t m = 0; m < zi.size(); m++) {   // x = X / Z^2, y = Y / Z^3
+    const size_t at = zi_at[m];
+    const fe z2 = BF::mul(zi[m], zi[m]);
+    X[at] = BF::mul(X[at], z2);
+    Y[at] = BF::mul(Y[at], BF::mul(z2, zi[m]));
+  }
+  IpaVerifyPlan p;
+  for (size_t q = 0; q < k; q++) {
+    for (size_t i = 0; good[q] && i < per; i++) {
+      const size_t at = q * per + i;
+      if (!BF::is_zero(Z[at]))
+        good[q] = BF::eq(BF::mul(Y[at], Y[at]), BF::add(BF::mul(BF::mul(X[at], X[at]), X[at]), b));
+    }
+    if (good[q]) p.active.push_back(q);
+  }
+  const size_t ka = p.active.size();
+  p.rr.resize(ka * (2 * ell + 1));
+  p.last.resize(ka);
+  p.pts72.assign(ka * per * 72, 0);
+  p.small.resize(ka * per);
+  fe* r = p.rr.data();
+  fe* r_inv = r + ka * ell;
+  fe* scale = r_inv + ka * ell;
+  for (size_t x = 0; x < ka && ell; x++) std::memcpy(r + x * ell, a.r + p.active[x] * ell, ell * sizeof(fe));
+  std::vector<fe> inv(r, r + ka * ell);
+  batch_invert<SF>(inv);
+  std::copy(inv.begin(), inv.end(), r_inv);
+  for (size_t x = 0; x < ka; x++) {
+    const size_t q = p.active[x];
+    const fe w = a.w[q], nw = SF::neg(w);
+    scale[x] = SF::mul(w, a.a_hat[q]);
+    p.last[x] = SF::mul(SF::mul(w, a.u_scale[q]), SF::sub(SF::mul(a.a_hat[q], a.b_hat[q]), a.c[q]));
+    fe* sm = p.small.data() + x * per;
+    sm[0] = nw;
+    for (size_t j = 0; j < ell; j++) {
+      sm[1 + j] = SF::mul(nw, SF::mul(r[x * ell + j], r[x * ell + j]));
+      sm[1 + ell + j] = SF::mul(nw, SF::mul(r_inv[x * ell + j], r_inv[x * ell + j]));
+    }
+    for (size_t i = 0; i < per; i++) {
+      const size_t at = q * per + i;
+      uint8_t* rec = p.pts72.data() + (x * per + i) * 72;
+      if (BF::is_zero(Z[at])) {
+        rec[64] = 1;   // the infinity flag
+      } else {
+        std::memcpy(rec, &X[at], 32);
+        std::memcpy(rec + 32, &Y[at], 32);
+      }
+    }
+  }
+  return p;
+}
+
+// the proofs' own points as a transient plain-layout set (the layout vdfgpu_gens_create makes without flags)
+static vdfgpu_gens ipa_small_set(int curve, affine_t* pts, size_t count) {
+  vdfgpu_gens gs;
+  gs.curve = curve;
+  gs.n = count;
+  gs.W = 1;
+  gs.pts = pts;
+  return gs;
+}
+
+// The weighted sum of all active proofs: Hi / Lo tables, S, the MSM over g, the proofs' points uploaded and
+// repacked, the MSM over them, the sum of the two results; one 96-byte read-back into sum_host (normalised on the
+// device: the identity is 96 zero bytes)
+template <class C, class SF>
+static void ipa_verify_batch_enqueue(vdfgpu_gens* g, size_t ell, const IpaVerifyPlan& p, IpaVerifyScratch& s,
+                                     void* sum_host) {
+  cudaStream_t st = cur_stream();
+  CudaLaunch L = api_launch(st);
+  const size_t ka = p.active.size(), n = (size_t)1 << ell, ns = p.small.size();
+  const uint32_t lo_bits = (uint32_t)(ell / 2), hi_bits = (uint32_t)ell - lo_bits;
+  const size_t hi_len = ka << hi_bits, lo_len = ka << lo_bits;
+  s.rr = pool_alloc<fe>(p.rr.size(), st);
+  s.tables = pool_alloc<fe>(hi_len + lo_len, st);
+  s.S = pool_alloc<fe>(n + 1, st);
+  s.small = pool_alloc<fe>(ns, st);
+  s.raw = pool_alloc<uint8_t>(p.pts72.size(), st);
+  s.pts = pool_alloc<affine_t>(ns, st);
+  s.out = pool_alloc<jac_t>(2 * MSM_MAX_BATCH + 1, st);
+  h2d(s.rr, p.rr.data(), p.rr.size() * sizeof(fe), st);   // pageable sources: staged before cudaMemcpyAsync returns
+  h2d(s.small, p.small.data(), ns * sizeof(fe), st);
+  h2d(s.raw, p.pts72.data(), p.pts72.size(), st);
+  fe last = SF::zero();
+  for (const fe& x : p.last) last = SF::add(last, x);
+  L.run<256>(hi_len + lo_len, IpaHalfTablesFn<SF>{s.rr, s.rr + ka * ell, s.rr + 2 * ka * ell, (uint32_t)ell, lo_bits,
+                                                  ka, s.tables, s.tables + hi_len});
+  L.run<256>(n + 1, IpaBatchScalarsFn<SF>{s.tables, s.tables + hi_len, hi_bits, lo_bits, ka, last, s.S});
+  msm_on_device(g, 0, s.S, n + 1, s.out, true, st, true);
+  L.run<256>(ns, RepackFn{s.raw, s.pts});
+  vdfgpu_gens gs = ipa_small_set(g->curve, s.pts, ns);
+  msm_on_device(&gs, 0, s.small, ns, s.out + 1, true, st, true, false);
+  L.run<32>(32, JacSumFn<C>{s.out, 2, s.out + 2});
+  fe* pin = pinned_evals();
+  d2h(pin, s.out + 2, sizeof(jac_t), st);
+  sync_after_unlock(st);
+  copy_after_sync(sum_host, pin, sizeof(jac_t));
+}
+
+// Active proofs [first, first + kc), kc <= MSM_MAX_BATCH, each alone: proof q's share of the batch (its S from its
+// own Hi / Lo tables, its slice of the small scalars) as kc vectors of one batched MSM over g and one over the small
+// set.  out_host receives the kc results over g, then at 4 * 96 bytes the kc over the small set, normalised.
+template <class SF>
+static void ipa_verify_chunk_enqueue(vdfgpu_gens* g, size_t ell, const IpaVerifyPlan& p, IpaVerifyScratch& s,
+                                     size_t first, uint32_t kc, void* out_host) {
+  cudaStream_t st = cur_stream();
+  CudaLaunch L = api_launch(st);
+  const size_t ka = p.active.size(), n = (size_t)1 << ell, ns = p.small.size(), per = 2 * ell + 1;
+  const uint32_t lo_bits = (uint32_t)(ell / 2), hi_bits = (uint32_t)ell - lo_bits;
+  if (!s.S4) {
+    s.S4 = pool_alloc<fe>(MSM_MAX_BATCH * (n + 1), st);
+    s.small4 = pool_alloc<fe>(MSM_MAX_BATCH * ns, st);
+  }
+  std::vector<fe> sm((size_t)kc * ns, SF::zero());
+  const fe* vg[MSM_MAX_BATCH];
+  const fe* vs[MSM_MAX_BATCH];
+  size_t lg[MSM_MAX_BATCH], ls[MSM_MAX_BATCH];
+  for (uint32_t j = 0; j < kc; j++) {
+    const size_t x = first + j;
+    fe* S = s.S4 + j * (n + 1);
+    L.run<256>(n + 1, IpaBatchScalarsFn<SF>{s.tables + (x << hi_bits), s.tables + (ka << hi_bits) + (x << lo_bits),
+                                            hi_bits, lo_bits, 1, p.last[x], S});
+    std::copy(p.small.begin() + x * per, p.small.begin() + (x + 1) * per, sm.begin() + j * ns + x * per);
+    vg[j] = S;
+    lg[j] = n + 1;
+    vs[j] = s.small4 + j * ns;
+    ls[j] = ns;
+  }
+  h2d(s.small4, sm.data(), sm.size() * sizeof(fe), st);
+  msm_batch_on_device(g, vg, lg, kc, s.out, true);
+  vdfgpu_gens gs = ipa_small_set(g->curve, s.pts, ns);
+  msm_batch_on_device(&gs, vs, ls, kc, s.out + MSM_MAX_BATCH, true, false);
+  fe* pin = pinned_evals();
+  d2h(pin, s.out, kc * sizeof(jac_t), st);
+  d2h(pin + 3 * MSM_MAX_BATCH, s.out + MSM_MAX_BATCH, kc * sizeof(jac_t), st);
+  sync_after_unlock(st);
+  copy_after_sync(out_host, pin, 2 * MSM_MAX_BATCH * sizeof(jac_t));
+  normalise_after_sync(out_host, kc, g->curve);
+  normalise_after_sync(reinterpret_cast<uint8_t*>(out_host) + MSM_MAX_BATCH * sizeof(jac_t), kc, g->curve);
+}
+
+// vdfgpu_ipa_verify_batch.  Like ipa_prove, the call holds a reference on g from its first guarded() section to its
+// last; the batch is one section, each chunk of single-proof checks of a failing batch one more.  The verdicts fail
+// closed: ok is zeroed first, and a 1 reaches it only when the whole call succeeded and that proof's check passed.
+static int ipa_verify_batch(vdfgpu_gens* g, size_t ell, size_t k, const IpaVerifyArgs& a, uint8_t* ok) {
+  IpaVerifyPlan p;
+  IpaVerifyScratch s;
+  bool holds_g = false;
+  uint8_t sum[96];
+  std::vector<uint8_t> verdict(k, 0);
+  int rc = guarded([&] {
+    if (!g || !a.comm || !a.a_hat || !a.c || !a.b_hat || !a.u_scale || !a.w || !ok || (ell && (!a.L || !a.R || !a.r)))
+      throw ArgError("ipa_verify_batch: null pointer");   // L, R and r may be NULL at ell = 0
+    if (k == 0) throw ArgError("ipa_verify_batch: no proofs");
+    std::memset(ok, 0, k);
+    if (ell > 40 || g->n < ((size_t)1 << ell) + 1)
+      throw ArgError("ipa_verify_batch: the generator set needs at least 2^ell + 1 points");
+    with_curve(g->curve, "ipa_verify_batch", [&](auto C, auto BF, auto SF) {
+      using F = decltype(SF);
+      for (size_t i = 0; i < k * ell; i++)
+        if (!usable_challenge<F>(a.r[i])) throw ArgError("ipa_verify_batch: a challenge is 0 or non-canonical");
+      for (size_t q = 0; q < k; q++)
+        if (!usable_challenge<F>(a.w[q])) throw ArgError("ipa_verify_batch: a weight is 0 or non-canonical");
+      p = ipa_verify_prepare<decltype(BF), F>(ell, k, a);
+      if (p.active.empty()) return;
+      require_ready();
+      g->refs++;
+      holds_g = true;
+      ipa_verify_batch_enqueue<decltype(C), F>(g, ell, p, s, sum);
+    });
+  });
+  const bool passed = rc == VDFGPU_OK && holds_g && std::all_of(sum + 64, sum + 96, [](uint8_t v) { return v == 0; });
+  if (rc == VDFGPU_OK && holds_g && !passed) {
+    for (size_t first = 0; rc == VDFGPU_OK && first < p.active.size(); first += MSM_MAX_BATCH) {
+      const uint32_t kc = (uint32_t)std::min<size_t>(MSM_MAX_BATCH, p.active.size() - first);
+      uint8_t res[2 * MSM_MAX_BATCH][96];
+      rc = guarded([&] {
+        require_ready();
+        with_curve(g->curve, "ipa_verify_batch", [&](auto, auto, auto SF) {
+          ipa_verify_chunk_enqueue<decltype(SF)>(g, ell, p, s, first, kc, res);
+        });
+      });
+      if (rc != VDFGPU_OK) break;
+      // proof valid iff (its share over g) = -(its share over its own points): both normalised, identity all zero
+      with_curve(g->curve, "ipa_verify_batch", [&](auto, auto BF, auto) {
+        using F = decltype(BF);
+        for (uint32_t j = 0; j < kc; j++) {
+          fe P[3], Q[3];
+          std::memcpy(P, res[j], 96);
+          std::memcpy(Q, res[MSM_MAX_BATCH + j], 96);
+          verdict[p.active[first + j]] = F::eq(P[0], Q[0]) && F::eq(P[1], F::neg(Q[1])) && F::eq(P[2], Q[2]);
+        }
+      });
+    }
+  } else if (passed) {
+    for (size_t q : p.active) verdict[q] = 1;
+  }
+  if (rc == VDFGPU_OK) std::memcpy(ok, verdict.data(), k);
+  std::string keep = rc == VDFGPU_OK ? std::string() : std::string(vdfgpu_last_error());
+  guarded([&] {
+    if (holds_g) g->refs--;
+    if (!ctx().ready) return;
+    for (void* ptr : s.all())
+      if (ptr) cudaFreeAsync(ptr, cur_stream());
+  });
+  if (rc != VDFGPU_OK) set_error(keep);
+  return rc;
+}
+
 }  // namespace vdf
 
 using namespace vdf;
@@ -502,6 +789,17 @@ int vdfgpu_ipa_gens_hat(vdfgpu_gens* g, const void* r_host, size_t ell, void* ou
       ipa_gens_hat_enqueue<decltype(SF)>(g, r.data(), r_inv.data(), ell, out_point96_host);
     });
   });
+}
+
+int vdfgpu_ipa_verify_batch(vdfgpu_gens* g, size_t ell, size_t k, const void* comm_a96_host, const void* L96_host,
+                            const void* R96_host, const void* r32_host, const void* a_hat32_host, const void* c32_host,
+                            const void* b_hat32_host, const void* u_scale32_host, const void* w32_host,
+                            uint8_t* ok_out_host) {
+  auto fes = [](const void* p) { return reinterpret_cast<const fe*>(p); };
+  const IpaVerifyArgs a{reinterpret_cast<const uint8_t*>(comm_a96_host), reinterpret_cast<const uint8_t*>(L96_host),
+                        reinterpret_cast<const uint8_t*>(R96_host), fes(r32_host), fes(a_hat32_host), fes(c32_host),
+                        fes(b_hat32_host), fes(u_scale32_host), fes(w32_host)};
+  return ipa_verify_batch(g, ell, k, a, ok_out_host);
 }
 
 #pragma GCC visibility pop

@@ -233,11 +233,12 @@ struct vdfgpu_gens {
 // internal cross-TU entry: MSM over device scalars into a device point, on the calling thread's stream
 namespace vdf {
 // raw = true: the result is written as an un-normalised Jacobian point whatever the set's flags say (the host entry
-// points then normalise it on the host, see normalise_after_sync)
+// points then normalise it on the host, see normalise_after_sync).  replay = false: never run as a cached graph -- for
+// points in a transient buffer, whose address keys a graph nothing will replay, and which would evict useful ones
 void msm_on_device(vdfgpu_gens* g, size_t first, const fe* d_scalars, size_t n, jac_t* d_out, bool is_mont,
-                   cudaStream_t stream = nullptr, bool raw = false);
+                   cudaStream_t stream = nullptr, bool raw = false, bool replay = true);
 void msm_batch_on_device(vdfgpu_gens* g, const fe* const* d_scalars, const size_t* lens, uint32_t k, jac_t* d_out,
-                         bool raw = false);
+                         bool raw = false, bool replay = true);
 // Host entry points that return a point to HOST memory let the device write the un-normalised Jacobian result and
 // divide by Z on the host once the copy has landed: one field inversion is a strictly sequential chain of ~335
 // multiplications -- 0.12 ms in a single GPU thread, ~15 us on a CPU core -- and the bytes are identical.  (Same

@@ -151,6 +151,74 @@ struct IpaFoldFn {
   }
 };
 
+// ---- batch verification of inner-product arguments (vdfgpu_ipa_verify_batch) -------------------------------------
+// Proof q (of k) over the same set is valid iff
+//   a_hat G_hat + u_scale (a_hat b_hat - c) U0 - comm_a - sum_j (r_j^2 L_j + r_j^-2 R_j) = O,   G_hat = <s_q, G[0,n)>
+// (ipa_ref.verify with P = comm_a + c U).  The equation is linear in the points, so with weights w_q != 0 the batch
+// checks the weighted sum of the k left-hand sides with two MSMs:
+//   over G[0, n]:            S[i] = sum_q w_q a_hat_q s_q[i]  (i < n),   S[n] = sum_q w_q u_scale_q (a_hat_q b_hat_q - c_q)
+//   over the proofs' points: -w_q for comm_a_q, -w_q r_qj^2 for L_qj, -w_q r_qj^-2 for R_qj.
+// S is built without k s tables: with ell_h = ceil(ell / 2) high bits and ell_l = floor(ell / 2) low bits of the index,
+// s_q[t 2^ell_l + u] = Hi_q[t] Lo_q[u] (Hi over r_0 .. r_{ell_h - 1}, Lo over the rest), so S = sum_q Hi_q[t] Lo_q[u]
+// is a field "matrix product" with inner dimension k: k multiplications per entry, from two tables of k 2^ell_h
+// entries each at most (4 MB at k = 64, ell = 20), which stay in L2.
+
+// All k Hi tables, then all k Lo tables, index space k (2^hi_bits + 2^lo_bits), hi_bits = ell - lo_bits:
+//   hi[q 2^hi_bits + t] = scale[q] prod_{j < hi_bits} (bit_j(t) ? r[q][j] : r_inv[q][j])
+//   lo[q 2^lo_bits + u] =          prod_{j < lo_bits} (bit_j(u) ? r[q][hi_bits + j] : r_inv[q][hi_bits + j])
+// bit_0 the most significant; r and r_inv are [k][ell], proof-major.  scale = w a_hat (batch) or a_hat (one proof).
+template <class F>
+struct IpaHalfTablesFn {
+  const fe* r; const fe* r_inv; const fe* scale;
+  uint32_t ell, lo_bits;
+  size_t k;
+  fe* hi; fe* lo;
+  VDF_HD void operator()(size_t idx) const {
+    const uint32_t hi_bits = ell - lo_bits;
+    const size_t hi_len = k << hi_bits;
+    const bool is_hi = idx < hi_len;
+    const size_t e = is_hi ? idx : idx - hi_len;
+    const uint32_t nbits = is_hi ? hi_bits : lo_bits, first = is_hi ? 0u : hi_bits;
+    const size_t q = e >> nbits, t = e & (((size_t)1 << nbits) - 1);
+    fe acc = is_hi ? fe_load(scale + q) : F::one();
+    const fe* rq = r + q * ell + first;
+    const fe* riq = r_inv + q * ell + first;
+#pragma unroll 1
+    for (uint32_t j = 0; j < nbits; j++)
+      acc = F::mul(acc, fe_load(((t >> (nbits - 1 - j)) & 1u) ? rq + j : riq + j));
+    fe_store((is_hi ? hi : lo) + e, acc);
+  }
+};
+
+// S[t 2^lo_bits + u] = sum_{q < k} hi[q 2^hi_bits + t] lo[q 2^lo_bits + u], S[n] = last (n = 2^(hi_bits + lo_bits)),
+// index space n + 1.  Adjacent threads take adjacent u: the warp reads lo coalesced and hi as a broadcast.
+template <class F>
+struct IpaBatchScalarsFn {
+  const fe* hi; const fe* lo;
+  uint32_t hi_bits, lo_bits;
+  size_t k;
+  fe last;
+  fe* S;
+  VDF_HD void operator()(size_t i) const {
+    const size_t n = (size_t)1 << (hi_bits + lo_bits);
+    if (i == n) {
+      fe_store(S + n, last);
+      return;
+    }
+    const size_t t = i >> lo_bits, u = i & (((size_t)1 << lo_bits) - 1);
+    const fe* h = hi + t;
+    const fe* l = lo + u;
+    fe acc = F::mul(fe_load(h), fe_load(l));
+#pragma unroll 1
+    for (size_t q = 1; q < k; q++) {
+      h += (size_t)1 << hi_bits;
+      l += (size_t)1 << lo_bits;
+      acc = F::add(acc, F::mul(fe_load(h), fe_load(l)));
+    }
+    fe_store(S + i, acc);
+  }
+};
+
 constexpr int SC_BLOCK = 256;
 constexpr int SC_MAX_POLYS = 4;
 

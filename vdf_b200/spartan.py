@@ -162,3 +162,60 @@ def ipa_gens_hat(gens, r: Sequence[int]) -> bytes:
     _lib.check(_lib.load().vdfgpu_ipa_gens_hat(gens._h, _lib.as_ptr(fes_to_bytes(r, order) or bytes(32)), len(r),
                                                _lib.as_ptr(out)))
     return bytes(out)
+
+
+# ---- verification of inner-product arguments ---------------------------------------------------------------------
+# A proof as the verifier receives it: what ipa_prove returns (L list, R list, challenges, a_hat) and the instance
+# (comm_a as a 96-byte point, c = <a, b>, b_hat = <b, s>, u_scale).
+IpaProof = Tuple[Sequence[bytes], Sequence[bytes], Sequence[int], int, bytes, int, int, int]
+
+
+def ipa_b_hat(field_id: int, rs: Sequence[int], terms: Sequence[Tuple[int, Sequence[int]]]) -> int:
+    """b_hat = <b, s> for b = sum_i rho_i eq(x_i), terms = [(rho_i, x_i)], in closed form: <eq(x), s> =
+    prod_j ((1 - x_j) r_j^-1 + x_j r_j).  An x shorter than rs stands for an eq table zero-padded at the top (eq over
+    x with leading zero coordinates)."""
+    m = MODULUS[field_id]
+    inv = [pow(r, -1, m) for r in rs]
+    out = 0
+    for rho, x in terms:
+        if len(x) > len(rs):
+            raise ValueError("ipa_b_hat: a point has more coordinates than there are challenges")
+        x = [0] * (len(rs) - len(x)) + list(x)
+        v = rho % m
+        for xj, r, ri in zip(x, rs, inv):
+            v = v * ((1 - xj) * ri + xj * r) % m
+        out = (out + v) % m
+    return out
+
+
+def ipa_verify_batch(gens, proofs: Sequence[IpaProof], weights: Sequence[int] | None = None) -> List[bool]:
+    """Verifies inner-product arguments over the resident set `gens` (at least 2^ell + 1 points) in one call, one
+    verdict per proof.  All proofs need the same ell.  weights: one non-zero weight per proof for the random linear
+    combination; None draws them with `secrets`.  A caller that passes its own must draw them uniformly and out of
+    the provers' sight: predictable weights let two invalid proofs cancel."""
+    import secrets
+
+    from .encoding import CURVE_ORDER
+    order = CURVE_ORDER[gens.curve]
+    k = len(proofs)
+    if k == 0:
+        return []
+    ell = len(proofs[0][2])
+    if any(len(p[0]) != ell or len(p[1]) != ell or len(p[2]) != ell for p in proofs):
+        raise ValueError("ipa_verify_batch: every proof needs ell L, R and challenges, the same ell for all")
+    if any(len(x) != 96 for p in proofs for x in (p[4], *p[0], *p[1])):
+        raise ValueError("ipa_verify_batch: comm_a, L and R must be 96-byte Jacobian points")
+    if weights is None:
+        weights = [1 + secrets.randbelow(order - 1) for _ in range(k)]
+    if len(weights) != k:
+        raise ValueError("ipa_verify_batch: one weight per proof")
+    comm = b"".join(p[4] for p in proofs)
+    Ls = b"".join(x for p in proofs for x in p[0]) or bytes(96)
+    Rs = b"".join(x for p in proofs for x in p[1]) or bytes(96)
+    rs = fes_to_bytes([r for p in proofs for r in p[2]], order) or bytes(32)
+    col = lambda i: _lib.as_ptr(fes_to_bytes([p[i] for p in proofs], order))  # noqa: E731
+    ok = bytearray(k)
+    _lib.check(_lib.load().vdfgpu_ipa_verify_batch(gens._h, ell, k, _lib.as_ptr(comm), _lib.as_ptr(Ls), _lib.as_ptr(Rs),
+                                                   _lib.as_ptr(rs), col(3), col(5), col(6), col(7),
+                                                   _lib.as_ptr(fes_to_bytes(weights, order)), _lib.as_ptr(ok)))
+    return [bool(v) for v in ok]
