@@ -190,7 +190,9 @@ int vdfgpu_running_create(const vdfgpu_r1cs* s, vdfgpu_gens* gens, vdfgpu_runnin
 int vdfgpu_running_destroy(vdfgpu_running* f);
 int vdfgpu_running_set(vdfgpu_running* f, const void* W_host, const void* E_host, const void* u_host,
                             const void* X_host);
-int vdfgpu_running_get(const vdfgpu_running* f, void* W_host, void* E_host, void* u_host, void* X_host);   /* CompressedSNARK::prove's input */
+int vdfgpu_running_get(const vdfgpu_running* f, void* W_host, void* E_host, void* u_host, void* X_host);
+/* CompressedSNARK::prove of the running instance without reading it back: vdfgpu_running_spartan_prove, after the
+ * sum-check and IPA callback types below */
 /* upload fresh witness, commit to it, compute T and comm_T; W2/T stay on the device for running_finish */
 int vdfgpu_running_commit(vdfgpu_running* f, const void* W2_host, const void* X2_host,
                        void* comm_W2_point96_host, void* comm_T_point96_host);
@@ -321,6 +323,42 @@ int vdfgpu_ipa_verify_batch(vdfgpu_gens* g, size_t ell, size_t k, const void* co
                             const void* R96_host, const void* r32_host, const void* a_hat32_host, const void* c32_host,
                             const void* b_hat32_host, const void* u_scale32_host, const void* w32_host,
                             uint8_t* ok_out_host);
+
+/* RelaxedR1CSSNARK::prove of the running instance (CompressedSNARK::prove, src/nova/proof.rs:363 -> nova-snark 0.8
+ * spartan_with_ipa_pc [R]; the math is restated in vdf_b200/csrc/sumcheck.cuh) in ONE call, the transcript left to the
+ * caller's callbacks.  Padded layout (nova's R1CSShape::pad [R]): m = the next power of two >= max(num_vars, num_cons);
+ * column c of the shape is column c if c < num_vars, else c + (m - num_vars), so z = [W | 0 | u | X | 0] has 2m entries;
+ * ell_x = log2 m, ell_y = ell_x + 1; 1 + num_io <= m is required.  In order:
+ *   1. snapshot: W and E (zero-padded to m) and u, X are copied on the device behind the instance's previous call; the
+ *      proof reads only the snapshot (a later running_commit / running_finish cannot change it).
+ *   2. outer sum-check of sum_x eq(tau, x) (Az Bz - (u Cz + E))(x) = 0, ell_x rounds: sc_round(user, j, (e0, e2, e3),
+ *      3, r_out) -> r_x.  claim_Az, claim_Bz: the bound tables; claim_Cz = Cz(r_x), eval_E = E(r_x).
+ *      claims(user, VDFGPU_SPARTAN_OUTER, (claim_Az, claim_Bz, claim_Cz, eval_E), 4, (r_A, r_B, r_C), 3).
+ *   3. inner sum-check of sum_y M(y) z(y) with M(y) = sum_x eq(r_x, x) (r_A A + r_B B + r_C C)[x, y], ell_y rounds:
+ *      sc_round(user, j, (e0, e2), 2, r_out) -> r_y (round indices restart at 0).  r_y' = r_y[1..].
+ *   4. eval_W = W(r_y'), T = <E, eq(r_y')> + <W, eq(r_x)>: claims(user, VDFGPU_SPARTAN_EVAL, (eval_W, T), 2, rho, 1).
+ *   5. the two claims E(r_x) = eval_E, W(r_y') = eval_W folded into one (nova's fold of two inner-product instances
+ *      [R]): a = E + rho W, b = eq(r_x) + rho eq(r_y'), c = eval_E + rho T + rho^2 eval_W; the caller forms
+ *      comm_a = comm_E + rho comm_W.  claims(user, VDFGPU_SPARTAN_IPA, c, 1, u_scale, 1).
+ *   6. vdfgpu_ipa_prove of (a, b) over ipa_gens with u_scale: ipa_round as there; a_hat into a_hat32_host.
+ * All values are 32-byte Montgomery elements of the shape's field.  ipa_gens: the curve whose scalar field is the
+ * shape's, at least m + 1 points (U0 = G_m); its first m points must be the instance's commitment generators (it may be
+ * the instance's own set when that holds m + 1 points).  tau: ell_x elements.  Callbacks run on the calling thread,
+ * outside the library's lock; a non-zero return, a non-canonical value returned, or an IPA challenge of 0 ends the call
+ * with VDFGPU_ERR_STATE.  VDFGPU_ERR_ARG before any device work: a null pointer, ipa_gens of the wrong curve or with
+ * fewer than m + 1 points, 1 + num_io > m.  Before vdfgpu_running_set: VDFGPU_ERR_STATE.  The shape, ipa_gens and f
+ * stay referenced for the whole call: destroying any of them meanwhile returns VDFGPU_ERR_STATE.  The instance itself
+ * is left unchanged. */
+typedef int (*vdfgpu_spartan_claims_fn)(void* user, int stage, const void* in_fe32, size_t n_in, void* out_fe32,
+                                        size_t n_out);
+enum { VDFGPU_SPARTAN_OUTER = 0, VDFGPU_SPARTAN_EVAL = 1, VDFGPU_SPARTAN_IPA = 2 };
+int vdfgpu_running_spartan_prove(vdfgpu_running* f, vdfgpu_gens* ipa_gens, const void* tau_host,
+                                 vdfgpu_round_fn sc_round, vdfgpu_spartan_claims_fn claims,
+                                 vdfgpu_ipa_round_fn ipa_round, void* user, void* a_hat32_host);
+/* The sparse part of RelaxedR1CSSNARK::verify [R]: out = (A(r_x, r_y), B(r_x, r_y), C(r_x, r_y)) over the padded layout
+ * above, A(r_x, r_y) = sum over entries (x, c, v) of v eq(r_x, x) eq(r_y, col(c)); r_x: ell_x elements, r_y: ell_x + 1
+ * (most significant variable first).  1 + num_io > m: VDFGPU_ERR_ARG. */
+int vdfgpu_r1cs_evaluate(const vdfgpu_r1cs* s, const void* rx_host, const void* ry_host, void* out3_host);
 
 /* ---- a8: batched MinRoot verification.  Replaces a loop of MinRootVDF::check (src/minroot.rs:369-371)
  * / Evaluation::verify (:424-426) over independent chains.  ok_out[k] = 1 iff

@@ -310,7 +310,53 @@ impl<'a, G: GpuCurve> GpuRunning<'a, G> {
     pub fn fold(&mut self, r: &G::Scalar) -> Result<(), GpuError> {
         check(unsafe { sys::vdfgpu_running_finish(self.h, (r as *const G::Scalar).cast()) })
     }
-    /// Read the running witness back (needed by `CompressedSNARK::prove` only; `check` verifies it in place).
+    /// `RelaxedR1CSSNARK::prove` of this running instance in one call [R: nova-snark 0.8 spartan_with_ipa_pc]: W, E, u
+    /// and X are not read back.  `ipa_gens` holds the commitment generators G_0 .. G_{m-1} followed by gens_c (m + 1
+    /// points, m = the padded size).  The arithmetic is the library's; the order in which nova's transcript absorbs and
+    /// squeezes is the caller's, recalled here [R] and unpinned like the rest of this module:
+    ///   outer rounds  absorb the round polynomial [e0, claim - e0, e2, e3], squeeze r_j (`sumcheck_round`)
+    ///   OUTER         absorb (claim_Az, claim_Bz, claim_Cz, eval_E), squeeze r; (r_A, r_B, r_C) = (1, r, r^2)
+    ///   inner rounds  absorb [e0, claim - e0, e2], squeeze r_j
+    ///   EVAL          absorb eval_W; the fold of the two inner-product instances (comm_E, eq(r_x), eval_E) and
+    ///                 (comm_W, eq(r_y'), eval_W): absorb both instances and T, squeeze rho
+    ///   IPA           absorb the folded instance (comm_E + rho comm_W, c), squeeze the scale of gens_c
+    ///   IPA rounds    absorb L and R, squeeze r_j
+    /// The proof nova serialises is assembled by the transcript from what it is handed; a_hat is returned.
+    pub fn spartan_prove<T: SpartanTranscript<G>>(&self, ipa_gens: &GpuGens<G>, tau: &[G::Scalar], transcript: &mut T)
+                                                  -> Result<G::Scalar, GpuError> {
+        unsafe extern "C" fn sc<G: GpuCurve, T: SpartanTranscript<G>>(user: *mut libc::c_void, round: libc::size_t,
+                                                                     evals: *const libc::c_void, n: libc::size_t,
+                                                                     r_out: *mut libc::c_void) -> libc::c_int {
+            let t = &mut *(user as *mut T);
+            let e = std::slice::from_raw_parts(evals as *const G::Scalar, n);
+            *(r_out as *mut G::Scalar) = t.sumcheck_round(round, e);
+            0
+        }
+        unsafe extern "C" fn claims<G: GpuCurve, T: SpartanTranscript<G>>(user: *mut libc::c_void, stage: libc::c_int,
+                                                                         vals: *const libc::c_void, n_in: libc::size_t,
+                                                                         out: *mut libc::c_void,
+                                                                         n_out: libc::size_t) -> libc::c_int {
+            let t = &mut *(user as *mut T);
+            t.claims(stage, std::slice::from_raw_parts(vals as *const G::Scalar, n_in),
+                     std::slice::from_raw_parts_mut(out as *mut G::Scalar, n_out));
+            0
+        }
+        unsafe extern "C" fn ipa<G: GpuCurve, T: SpartanTranscript<G>>(user: *mut libc::c_void, round: libc::size_t,
+                                                                      l: *const libc::c_void, r: *const libc::c_void,
+                                                                      r_out: *mut libc::c_void) -> libc::c_int {
+            let t = &mut *(user as *mut T);
+            *(r_out as *mut G::Scalar) = t.ipa_round(round, &*(l as *const G::Point), &*(r as *const G::Point));
+            0
+        }
+        let mut a_hat = <G::Scalar as ff::Field>::zero();
+        check(unsafe {
+            sys::vdfgpu_running_spartan_prove(self.h, ipa_gens.h, tau.as_ptr().cast(), Some(sc::<G, T>),
+                                              Some(claims::<G, T>), Some(ipa::<G, T>),
+                                              (transcript as *mut T).cast(), (&mut a_hat as *mut G::Scalar).cast())
+        })?;
+        Ok(a_hat)
+    }
+    /// Read the running witness back (`spartan_prove` proves it in place; `check` verifies it in place).
     pub fn get(&self) -> Result<(Vec<G::Scalar>, Vec<G::Scalar>, G::Scalar, Vec<G::Scalar>), GpuError> {
         let zero = <G::Scalar as ff::Field>::zero();
         let (mut w, mut e, mut u, mut x) =
@@ -334,6 +380,16 @@ impl<'a, G: GpuCurve> Drop for GpuRunning<'a, G> {
     fn drop(&mut self) {
         unsafe { sys::vdfgpu_running_destroy(self.h) };
     }
+}
+
+/// The transcript side of `GpuRunning::spartan_prove` [R]: nova's Poseidon transcript and proof assembly.
+pub trait SpartanTranscript<G: GpuCurve> {
+    /// the round's evaluations ((e0, e2, e3) outer, (e0, e2) inner; `round` restarts at 0 for each) -> r_j
+    fn sumcheck_round(&mut self, round: usize, evals: &[G::Scalar]) -> G::Scalar;
+    /// stage sys::VDFGPU_SPARTAN_OUTER / _EVAL / _IPA: the stage's values in, its challenges into `out`
+    fn claims(&mut self, stage: i32, values: &[G::Scalar], out: &mut [G::Scalar]);
+    /// the IPA round's L and R (normalised) -> r_j != 0
+    fn ipa_round(&mut self, round: usize, l: &G::Point, r: &G::Point) -> G::Scalar;
 }
 
 /// One `NIFS::prove` with the running witness on the device [R: nova-snark 0.8 nifs.rs].  `ro_challenge` is nova's

@@ -50,6 +50,16 @@ pub type vdfgpu_ipa_round_fn = Option<
     unsafe extern "C" fn(user: *mut c_void, round: size_t, l_point96: *const c_void, r_point96: *const c_void, r_out32: *mut c_void) -> c_int,
 >;
 
+/// Claims callback of `vdfgpu_running_spartan_prove`: at stage OUTER receives (claim_Az, claim_Bz, claim_Cz, eval_E) and
+/// writes (r_A, r_B, r_C); at EVAL receives (eval_W, T) and writes rho; at IPA receives c and writes u_scale; returns 0.
+pub type vdfgpu_spartan_claims_fn = Option<
+    unsafe extern "C" fn(user: *mut c_void, stage: c_int, in_fe32: *const c_void, n_in: size_t, out_fe32: *mut c_void,
+                         n_out: size_t) -> c_int,
+>;
+pub const VDFGPU_SPARTAN_OUTER: c_int = 0;
+pub const VDFGPU_SPARTAN_EVAL: c_int = 1;
+pub const VDFGPU_SPARTAN_IPA: c_int = 2;
+
 extern "C" {
     // ---- context
     pub fn vdfgpu_init(device: c_int) -> c_int;
@@ -188,6 +198,14 @@ extern "C" {
                                    l96_host: *const c_void, r96_host: *const c_void, r32_host: *const c_void,
                                    a_hat32_host: *const c_void, c32_host: *const c_void, b_hat32_host: *const c_void,
                                    u_scale32_host: *const c_void, w32_host: *const c_void, ok_out_host: *mut u8) -> c_int;
+
+    // ---- RelaxedR1CSSNARK::prove of the running instance in one call, and the verifier's sparse evaluation
+    pub fn vdfgpu_running_spartan_prove(f: *mut vdfgpu_running, ipa_gens: *mut vdfgpu_gens, tau_host: *const c_void,
+                                        sc_round: vdfgpu_round_fn, claims: vdfgpu_spartan_claims_fn,
+                                        ipa_round: vdfgpu_ipa_round_fn, user: *mut c_void,
+                                        a_hat32_host: *mut c_void) -> c_int;
+    pub fn vdfgpu_r1cs_evaluate(s: *const vdfgpu_r1cs, rx_host: *const c_void, ry_host: *const c_void,
+                                out3_host: *mut c_void) -> c_int;
 
     // ---- a8: batched MinRoot verification
     pub fn vdfgpu_minroot_check_batch(field: c_int, results_state96_host: *const c_void,

@@ -77,6 +77,8 @@ PROTOTYPES = {
                                            POINTER(c_uint64)]),
     "vdfgpu_r1cs_is_sat_relaxed_dev": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "vdfgpu_running_check": (c_int, [c_void_p, c_void_p, c_void_p, POINTER(c_uint64)]),
+    "vdfgpu_running_spartan_prove": (c_int, [c_void_p] * 8),
+    "vdfgpu_r1cs_evaluate": (c_int, [c_void_p] * 4),
     "vdfgpu_eq_evals": (c_int, [c_int, c_void_p, c_size_t, c_void_p]),
     "vdfgpu_eq_evals_dev": (c_int, [c_int, c_void_p, c_size_t, c_void_p]),
     "vdfgpu_sumcheck_cubic": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p]),
@@ -105,6 +107,8 @@ PROTOTYPES = {
 ROUND_FN = ctypes.CFUNCTYPE(c_int, c_void_p, c_size_t, c_void_p, c_size_t, c_void_p)
 # int (*vdfgpu_ipa_round_fn)(void* user, size_t round, const void* L_point96, const void* R_point96, void* r_out32)
 IPA_ROUND_FN = ctypes.CFUNCTYPE(c_int, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p)
+# int (*vdfgpu_spartan_claims_fn)(void* user, int stage, const void* in_fe32, size_t n_in, void* out_fe32, size_t n_out)
+CLAIMS_FN = ctypes.CFUNCTYPE(c_int, c_void_p, c_int, c_void_p, c_size_t, c_void_p, c_size_t)
 
 
 def lib_path() -> Path:

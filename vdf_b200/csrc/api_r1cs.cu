@@ -9,6 +9,7 @@
 #include "minroot.cuh"
 #include "r1cs.cuh"
 #include "r1cs_host.hpp"
+#include "sumcheck.cuh"
 
 struct vdfgpu_r1cs {
   int field = 0;
@@ -22,7 +23,8 @@ struct vdfgpu_r1cs {
   vdf::fe* csc_val = nullptr;     // [nnz]
   uint32_t* heavy = nullptr;      // [n_heavy]
   uint32_t n_heavy = 0;
-  mutable int refs = 0;   // running instances holding this shape (vdfgpu_r1cs_destroy refuses while > 0)
+  mutable int refs = 0;   // running instances and Spartan proofs in progress holding this shape (vdfgpu_r1cs_destroy
+                          // refuses while > 0)
   vdf::CsrView view() const { return vdf::CsrView{row_ptr, col, val, cons, vars, io}; }
   vdf::CscView col_view() const { return vdf::CscView{col_ptr, csc_row, csc_val, heavy, vdf::HostCsc::HEAVY}; }
   ~vdfgpu_r1cs() {   // the one release path: failed create, vdfgpu_r1cs_destroy
@@ -47,6 +49,7 @@ struct vdfgpu_running {
   // stream or thread (vdfgpu_running_finish returns before its fold has run) is ordered behind the previous one
   cudaEvent_t done = nullptr;
   bool have_running = false, have_fresh = false;
+  int refs = 0;   // Spartan proofs in progress on this instance (vdfgpu_running_destroy refuses while > 0)
   ~vdfgpu_running() {   // the one release path: failed create, vdfgpu_running_destroy
     if (bounce) cudaFreeHost(bounce);
     if (done) cudaEventDestroy(done);
@@ -93,11 +96,11 @@ static void launch_fold(CudaLaunch& L, fe* W1, const fe* W2, size_t nW, fe* E1, 
 }
 
 // the scalar field of the commitment curve must be the R1CS field
-static void check_gens_field(const vdfgpu_r1cs* s, const vdfgpu_gens* g) {
+static void check_gens_field(const vdfgpu_r1cs* s, const vdfgpu_gens* g, const std::string& who = "") {
   const bool same = with_curve(g->curve, "gens", [&](auto, auto, auto SF) {
     return with_field(s->field, "r1cs", [](auto f) { return std::is_same<decltype(f), decltype(SF)>::value; });
   });
-  if (!same) throw ArgError("generator curve's scalar field differs from the R1CS field");
+  if (!same) throw ArgError(who + "generator curve's scalar field differs from the R1CS field");
 }
 
 void upload_constants_r1cs() { VDF_CUDA_CHECK(upload_field_constants()); }
@@ -476,6 +479,7 @@ int vdfgpu_running_create(const vdfgpu_r1cs* s, vdfgpu_gens* gens, vdfgpu_runnin
 int vdfgpu_running_destroy(vdfgpu_running* f) {
   return guarded([&] {
     if (!f) return;
+    if (f->refs > 0) throw StateError("running_destroy: a Spartan proof of this instance is in progress");
     if (ctx().ready) {
       VDF_CUDA_CHECK(cudaSetDevice(ctx().device));
       cudaDeviceSynchronize();
@@ -694,6 +698,289 @@ int vdfgpu_running_finish(vdfgpu_running* f, const void* r32_host) {
     if (cudaPointerGetAttributes(&at, r32_host) == cudaSuccess && at.type == cudaMemoryTypeHost) sync_after_unlock(st);
     else cudaGetLastError();
     f->have_fresh = false;
+  });
+}
+
+#pragma GCC visibility pop
+}  // extern "C"
+
+// ---- Spartan of the running instance: RelaxedR1CSSNARK::prove [R] (notation: sumcheck.cuh) and the sparse evaluation
+// of its verifier --------------------------------------------------------------------------------------------------
+namespace vdf {
+
+// the caller's round callback behind sumcheck(): it keeps the challenges of the phase (r_x, then r_y) and rejects a
+// non-canonical one, which sumcheck() itself would bind
+struct SpartanRounds {
+  vdfgpu_round_fn fn;
+  void* user;
+  int field;
+  std::vector<fe> r;
+  bool non_canonical = false;
+};
+
+template <class F>
+static bool canonical_all(const fe* v, size_t n) {
+  for (size_t i = 0; i < n; i++)
+    if (!F::is_canonical(v[i])) return false;
+  return true;
+}
+
+static int spartan_round(void* p, size_t round, const void* evals, size_t n_evals, void* r_out) {
+  SpartanRounds& s = *static_cast<SpartanRounds*>(p);
+  if (s.fn(s.user, round, evals, n_evals, r_out) != 0) return 1;
+  fe r;
+  std::memcpy(&r, r_out, sizeof(fe));
+  s.non_canonical = !(s.field == VDFGPU_FP ? canonical_all<Fp>(&r, 1) : canonical_all<Fq>(&r, 1));
+  if (s.non_canonical) return 1;
+  s.r.push_back(r);
+  return 0;
+}
+
+// sumcheck() over the running instance's tables with the caller's callback; the challenges land in rounds.r
+static int spartan_sumcheck(SpartanRounds& rounds, fe* const* tables, int n_polys, size_t ell, fe* final_evals) {
+  rounds.r.clear();
+  const void* t[4] = {tables[0], tables[1], n_polys == 4 ? tables[2] : nullptr, n_polys == 4 ? tables[3] : nullptr};
+  const int rc = sumcheck(rounds.field, t, n_polys, false, ell, spartan_round, &rounds, final_evals);
+  if (rc != VDFGPU_OK && rounds.non_canonical) set_error("running_spartan_prove: the round callback returned a non-canonical challenge");
+  else if (rc != VDFGPU_OK) set_error(std::string("running_spartan_prove: ") + vdfgpu_last_error());
+  return rc;
+}
+
+static const char* const SPARTAN_STAGE[3] = {"OUTER", "EVAL", "IPA"};
+
+// one claims callback, outside the lock: every value it returns must be canonical
+static int spartan_claims(int field, vdfgpu_spartan_claims_fn fn, void* user, int stage, const fe* in, size_t n_in,
+                          fe* out, size_t n_out) {
+  if (fn(user, stage, in, n_in, out, n_out) != 0) {
+    set_error(std::string("running_spartan_prove: the claims callback failed at stage ") + SPARTAN_STAGE[stage]);
+    return VDFGPU_ERR_STATE;
+  }
+  if (!(field == VDFGPU_FP ? canonical_all<Fp>(out, n_out) : canonical_all<Fq>(out, n_out))) {
+    set_error(std::string("running_spartan_prove: the claims callback returned a non-canonical value at stage ") +
+              SPARTAN_STAGE[stage]);
+    return VDFGPU_ERR_STATE;
+  }
+  return VDFGPU_OK;
+}
+
+// The call's device buffers, carved from one stream-ordered allocation.  Az..D are contiguous: once the outer claims
+// are out they hold the inner tables (Mp over Az, Bz; zp over Cz, D), and eqt then holds eq(r_y').
+struct SpartanBufs {
+  fe* block = nullptr;
+  fe *W, *E, *uX, *Az, *Bz, *Cz, *D, *eqt, *eqx, *r, *eq3, *Mc, *coef, *partial, *res;
+  void carve(const vdfgpu_r1cs* s, const PaddedLayout& pad, cudaStream_t st) {
+    const size_t m = pad.m, ncols = (size_t)s->vars + 1 + s->io, npart = (size_t)148 * 8 * 3;
+    const size_t total = 9 * m + (1 + s->io) + (pad.ell_x + 1) + 3 * (size_t)s->cons + ncols + 3 + npart + 3;
+    VDF_CUDA_CHECK(cudaMallocAsync((void**)&block, total * sizeof(fe), st));
+    fe* p = block;
+    for (fe** q : {&W, &E, &Az, &Bz, &Cz, &D, &eqt, &eqx}) { *q = p; p += m; }
+    uX = p; p += 1 + s->io;
+    r = p; p += pad.ell_x + 1;
+    eq3 = p; p += 3 * (size_t)s->cons;
+    Mc = p; p += ncols;
+    coef = p; p += 3;
+    partial = p; p += npart;
+    res = p;
+  }
+};
+
+// the m-entry zero-padded copy of n elements at src
+static void padded_copy(fe* dst, const fe* src, size_t n, size_t m, cudaStream_t st) {
+  d2d(dst, src, n * sizeof(fe), st);
+  if (m > n) VDF_CUDA_CHECK(cudaMemsetAsync(dst + n, 0, (m - n) * sizeof(fe), st));
+}
+
+// K inner products on the device, read back into out_host after the wait
+template <class F, int K>
+static void spartan_dots(const MultiDot<K>& d, size_t n, const SpartanBufs& b, fe* out_host, cudaStream_t st) {
+  multi_dot_enqueue<F, K>(st, d, n, b.partial, b.res);
+  fe* pin = pinned_evals();
+  d2h(pin, b.res, K * sizeof(fe), st);
+  sync_after_unlock(st);
+  copy_after_sync(out_host, pin, K * sizeof(fe));
+}
+
+// vdfgpu_running_spartan_prove.  Like ipa_prove, a sequence of guarded() sections with the caller's callbacks between
+// them; the two sum-checks and the opening are sumcheck() and ipa_prove() themselves.  The shape, the IPA set and the
+// instance stay referenced from the first section to the last, so destroying any of them meanwhile is refused.
+static int running_spartan_prove(vdfgpu_running* f, vdfgpu_gens* g, const void* tau_host, vdfgpu_round_fn sc_round,
+                                 vdfgpu_spartan_claims_fn claims, vdfgpu_ipa_round_fn ipa_round, void* user,
+                                 void* a_hat_host) {
+  const vdfgpu_r1cs* s = nullptr;
+  PaddedLayout pad{};
+  SpartanBufs b;
+  bool holds = false;
+  int rc = guarded([&] {
+    if (!f || !g || !tau_host || !sc_round || !claims || !ipa_round || !a_hat_host)
+      throw ArgError("running_spartan_prove: null pointer");
+    s = f->shape;
+    check_gens_field(s, g, "running_spartan_prove: the IPA set: ");
+    pad = PaddedLayout::of(s->cons, s->vars, s->io);
+    if (!pad.fits()) throw ArgError("running_spartan_prove: 1 + num_io exceeds the padded size m");
+    if (g->n < pad.m + 1) throw ArgError("running_spartan_prove: the IPA set needs at least m + 1 points");
+    if (!f->have_running) throw StateError("running_spartan_prove: no running instance set");
+    require_ready();
+    cudaStream_t st = cur_stream();
+    CudaLaunch L = api_launch(st);
+    b.carve(s, pad, st);
+    s->refs++;
+    g->refs++;
+    f->refs++;
+    holds = true;
+    // the snapshot: from here on nothing reads the instance, so a later fold step cannot change the proof
+    running_after(f, st);
+    padded_copy(b.W, f->W, s->vars, pad.m, st);
+    padded_copy(b.E, f->E, s->cons, pad.m, st);
+    d2d(b.uX, f->uX, (1 + (size_t)s->io) * sizeof(fe), st);
+    running_done(f, st);
+    h2d(b.r, tau_host, pad.ell_x * sizeof(fe), st);
+    with_field(s->field, "running_spartan_prove", [&](auto F) {
+      using Fd = decltype(F);
+      eq_evals_enqueue<Fd>(L, b.r, pad.ell_x, b.eqt);
+      L.run<128>(pad.m, OuterTablesFn<Fd>{s->view(), ZView{b.W, b.uX, b.uX + 1}, b.E, b.Az, b.Bz, b.Cz, b.D});
+    });
+    // a pinned tau_host may still be in flight: the outer sum-check's first read-back waits for it
+  });
+  const int field = s ? s->field : 0;
+  SpartanRounds rounds{sc_round, user, field, {}, false};
+  fe fin[4], dots[2], r_abc[3];   // final evaluations, (claim_Cz, eval_E), (r_A, r_B, r_C)
+  std::vector<fe> r_x;
+  // outer sum-check -> r_x, claim_Az, claim_Bz; then claim_Cz and eval_E, and the OUTER stage
+  if (rc == VDFGPU_OK) {
+    fe* t[4] = {b.eqt, b.Az, b.Bz, b.D};
+    rc = spartan_sumcheck(rounds, t, 4, pad.ell_x, fin);
+    r_x = rounds.r;
+  }
+  if (rc == VDFGPU_OK)
+    rc = guarded([&] {
+      require_ready();
+      cudaStream_t st = cur_stream();
+      CudaLaunch L = api_launch(st);
+      h2d(b.r, r_x.data(), pad.ell_x * sizeof(fe), st);   // pageable: staged before cudaMemcpyAsync returns
+      with_field(field, "running_spartan_prove", [&](auto F) {
+        using Fd = decltype(F);
+        eq_evals_enqueue<Fd>(L, b.r, pad.ell_x, b.eqx);
+        spartan_dots<Fd, 2>(MultiDot<2>{{b.Cz, b.E}, {b.eqx, b.eqx}, {pad.m, pad.m}}, pad.m, b, dots, st);
+      });
+    });
+  if (rc == VDFGPU_OK) {
+    const fe in[4] = {fin[1], fin[2], dots[0], dots[1]};
+    rc = spartan_claims(field, claims, user, VDFGPU_SPARTAN_OUTER, in, 4, r_abc, 3);
+  }
+  // inner tables and inner sum-check -> r_y
+  if (rc == VDFGPU_OK)
+    rc = guarded([&] {
+      require_ready();
+      cudaStream_t st = cur_stream();
+      CudaLaunch L = api_launch(st);
+      h2d(b.coef, r_abc, sizeof(r_abc), st);
+      launch_bind_rows(L, s, b.eqx, b.coef, b.eq3, b.Mc);
+      with_field(field, "running_spartan_prove", [&](auto F) {
+        L.run<256>(2 * pad.m, PaddedScatterFn<decltype(F)>{pad, b.Mc, ZView{b.W, b.uX, b.uX + 1}, b.Az, b.Cz});
+      });
+    });
+  if (rc == VDFGPU_OK) {
+    fe* t[2] = {b.Az, b.Cz};
+    rc = spartan_sumcheck(rounds, t, 2, pad.ell_x + 1, fin);
+  }
+  // eval_W, the cross term T, and the EVAL stage
+  fe ev[3];   // eval_W, <E, eq(r_y')>, <W, eq(r_x)>
+  if (rc == VDFGPU_OK)
+    rc = guarded([&] {
+      require_ready();
+      cudaStream_t st = cur_stream();
+      CudaLaunch L = api_launch(st);
+      h2d(b.r, rounds.r.data() + 1, pad.ell_x * sizeof(fe), st);   // r_y' = r_y[1..]
+      with_field(field, "running_spartan_prove", [&](auto F) {
+        using Fd = decltype(F);
+        eq_evals_enqueue<Fd>(L, b.r, pad.ell_x, b.eqt);
+        spartan_dots<Fd, 3>(MultiDot<3>{{b.W, b.E, b.W}, {b.eqt, b.eqt, b.eqx}, {pad.m, pad.m, pad.m}}, pad.m, b, ev,
+                            st);
+      });
+    });
+  fe rho, c, u_scale;
+  if (rc == VDFGPU_OK) {
+    with_field(field, "running_spartan_prove", [&](auto F) {
+      using Fd = decltype(F);
+      ev[1] = Fd::add(ev[1], ev[2]);   // T
+    });
+    rc = spartan_claims(field, claims, user, VDFGPU_SPARTAN_EVAL, ev, 2, &rho, 1);
+  }
+  // the joint claim: a = E + rho W and b = eq(r_x) + rho eq(r_y') in place of E and eq(r_x), c on the host
+  if (rc == VDFGPU_OK)
+    rc = guarded([&] {
+      require_ready();
+      CudaLaunch L = api_launch(cur_stream());
+      with_field(field, "running_spartan_prove", [&](auto F) {
+        using Fd = decltype(F);
+        const fe eval_E = dots[1], T = ev[1], eval_W = ev[0];
+        c = Fd::add(eval_E, Fd::mul(rho, Fd::add(T, Fd::mul(rho, eval_W))));
+        L.run<256>(pad.m, IpaJoinFn<Fd>{b.E, b.W, b.eqx, b.eqt, rho, b.E, b.eqx});
+      });
+    });
+  if (rc == VDFGPU_OK) rc = spartan_claims(field, claims, user, VDFGPU_SPARTAN_IPA, &c, 1, &u_scale, 1);
+  // the opening; ipa_prove validates nothing the checks above have not (its set holds m + 1 points)
+  if (rc == VDFGPU_OK) {
+    rc = ipa_prove(g, b.E, b.eqx, false, pad.ell_x, &u_scale, ipa_round, user, a_hat_host);
+    if (rc != VDFGPU_OK) set_error(std::string("running_spartan_prove: ") + vdfgpu_last_error());
+  }
+  std::string keep = rc == VDFGPU_OK ? std::string() : std::string(vdfgpu_last_error());
+  guarded([&] {
+    if (holds) {
+      s->refs--;
+      g->refs--;
+      f->refs--;
+    }
+    if (b.block && ctx().ready) cudaFreeAsync(b.block, cur_stream());
+  });
+  if (rc != VDFGPU_OK) set_error(keep);
+  return rc;
+}
+
+// vdfgpu_r1cs_evaluate: (A, B, C)(r_x, r_y) = sum_x eq(r_x, x) sum_y M[x, y] eq(r_y, y) over the padded layout: the
+// rows' products with eq(r_y) read through the padded column map (MultiplyVecFn over PaddedLayout::view), then one
+// three-output pass against eq(r_x)
+template <class F>
+static void r1cs_evaluate_enqueue(const vdfgpu_r1cs* s, const PaddedLayout& pad, const void* rx_host,
+                                  const void* ry_host, void* out3_host) {
+  cudaStream_t st = cur_stream();
+  CudaLaunch L = api_launch(st);
+  const size_t nc = s->cons;
+  DevBuf<fe> r(2 * (size_t)pad.ell_x + 1, st), eqx(pad.m, st), eqy(2 * pad.m, st), rows(3 * nc, st),
+      partial((size_t)148 * 8 * 3, st), res(3, st);
+  h2d(r.p, rx_host, pad.ell_x * sizeof(fe), st);
+  h2d(r.p + pad.ell_x, ry_host, (pad.ell_x + 1) * sizeof(fe), st);
+  eq_evals_enqueue<F>(L, r.p, pad.ell_x, eqx.p);
+  eq_evals_enqueue<F>(L, r.p + pad.ell_x, pad.ell_x + 1, eqy.p);
+  launch_multiply_vec(L, s, pad.view(eqy.p), rows.p, rows.p + nc, rows.p + 2 * nc);
+  multi_dot_enqueue<F, 3>(st, MultiDot<3>{{rows.p, rows.p + nc, rows.p + 2 * nc}, {eqx.p, eqx.p, eqx.p}, {nc, nc, nc}},
+                          pad.m, partial.p, res.p);
+  fe* pin = pinned_evals();
+  d2h(pin, res.p, 3 * sizeof(fe), st);
+  sync_after_unlock(st);
+  copy_after_sync(out3_host, pin, 3 * sizeof(fe));
+}
+
+}  // namespace vdf
+
+extern "C" {
+#pragma GCC visibility push(default)
+
+int vdfgpu_running_spartan_prove(vdfgpu_running* f, vdfgpu_gens* ipa_gens, const void* tau_host,
+                                 vdfgpu_round_fn sc_round, vdfgpu_spartan_claims_fn claims,
+                                 vdfgpu_ipa_round_fn ipa_round, void* user, void* a_hat32_host) {
+  return running_spartan_prove(f, ipa_gens, tau_host, sc_round, claims, ipa_round, user, a_hat32_host);
+}
+
+int vdfgpu_r1cs_evaluate(const vdfgpu_r1cs* s, const void* rx_host, const void* ry_host, void* out3_host) {
+  return guarded([&] {
+    if (!s || !rx_host || !ry_host || !out3_host) throw ArgError("r1cs_evaluate: null pointer");
+    const PaddedLayout pad = PaddedLayout::of(s->cons, s->vars, s->io);
+    if (!pad.fits()) throw ArgError("r1cs_evaluate: 1 + num_io exceeds the padded size m");
+    with_field(s->field, "r1cs_evaluate", [&](auto F) {
+      require_ready();
+      r1cs_evaluate_enqueue<decltype(F)>(s, pad, rx_host, ry_host, out3_host);
+    });
   });
 }
 

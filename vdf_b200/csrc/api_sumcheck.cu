@@ -14,7 +14,7 @@ namespace vdf {
 void upload_constants_sumcheck() { VDF_CUDA_CHECK(upload_field_constants()); }
 
 template <class F>
-static void eq_evals_enqueue(CudaLaunch& L, const fe* r_dev, size_t ell, fe* out_dev) {
+void eq_evals_enqueue(CudaLaunch& L, const fe* r_dev, size_t ell, fe* out_dev) {
   const uint32_t lo_bits = (uint32_t)(ell / 2), hi_bits = (uint32_t)(ell - lo_bits);
   fe* hi = L.alloc<fe>((size_t)1 << hi_bits);
   fe* lo = L.alloc<fe>((size_t)1 << lo_bits);
@@ -34,7 +34,7 @@ struct ScScratch {   // per-call device scratch of the round loop (stream-ordere
 // so what a round costs is the round trip to the caller's transcript -- a pageable 96-byte copy is staged by the driver
 // (about 10 us), a pinned one is a plain DMA.  24 elements: the eight points a chunk of vdfgpu_ipa_verify_batch's
 // single-proof checks reads back.
-static fe* pinned_evals() {
+fe* pinned_evals() {
   static thread_local fe* p = nullptr;
   if (!p) VDF_CUDA_CHECK(cudaHostAlloc((void**)&p, 24 * sizeof(fe), cudaHostAllocDefault));
   return p;
@@ -67,11 +67,28 @@ static void dot_enqueue(cudaStream_t st, const fe* a, const fe* b, size_t n, con
   ctx().launches += 2;
 }
 
+template <class F, int K>
+void multi_dot_enqueue(cudaStream_t st, const MultiDot<K>& d, size_t n, fe* partial, fe* out) {
+  const uint32_t grid = sc_grid(n);
+  sc_multi_dot_kernel<F, K><<<grid, SC_BLOCK, 0, st>>>(d, n, partial);
+  sc_final_kernel<F, K><<<1, SC_BLOCK, 0, st>>>(partial, grid, out);
+  VDF_CUDA_CHECK(cudaGetLastError());
+  ctx().launches += 2;
+}
+
+// the instances other translation units use (ctx.cuh)
+template void eq_evals_enqueue<Fp>(CudaLaunch&, const fe*, size_t, fe*);
+template void eq_evals_enqueue<Fq>(CudaLaunch&, const fe*, size_t, fe*);
+template void multi_dot_enqueue<Fp, 2>(cudaStream_t, const MultiDot<2>&, size_t, fe*, fe*);
+template void multi_dot_enqueue<Fq, 2>(cudaStream_t, const MultiDot<2>&, size_t, fe*, fe*);
+template void multi_dot_enqueue<Fp, 3>(cudaStream_t, const MultiDot<3>&, size_t, fe*, fe*);
+template void multi_dot_enqueue<Fq, 3>(cudaStream_t, const MultiDot<3>&, size_t, fe*, fe*);
+
 // Both sum-checks, cubic (4 tables, 3 evaluations) and quadratic (2 tables, 2 evaluations), in both forms: tables on
 // the device, bound in place, or on the host (ell <= 30), uploaded first and freed at the end.  Every guarded() section
 // ends before the caller's round callback runs, so the tables and the scratch outlive several of them.
-static int sumcheck(int field, const void* const* tables, int n_polys, bool on_host, size_t ell, vdfgpu_round_fn fn,
-                    void* user, void* final_host) {
+int sumcheck(int field, const void* const* tables, int n_polys, bool on_host, size_t ell, vdfgpu_round_fn fn,
+             void* user, void* final_host) {
   const int n_evals = n_polys == 4 ? 3 : 2;
   PolySet P{{nullptr, nullptr, nullptr, nullptr}};
   ScScratch s;
@@ -211,8 +228,8 @@ static void ipa_coef_init(fe* coef, cudaStream_t st) {
 // pinned memory, normalised on the host after the wait (the transcript absorbs canonical points, whatever the set's
 // flags); the fold takes r and r^-1 by value.  The call holds a reference on g from its first guarded() section to its
 // last, so vdfgpu_gens_destroy from another thread between rounds is refused instead of freeing the points.
-static int ipa_prove(vdfgpu_gens* g, void* a_in, void* b_in, bool on_host, size_t ell, const void* u_scale_host,
-                     vdfgpu_ipa_round_fn fn, void* user, void* a_hat_host) {
+int ipa_prove(vdfgpu_gens* g, void* a_in, void* b_in, bool on_host, size_t ell, const void* u_scale_host,
+              vdfgpu_ipa_round_fn fn, void* user, void* a_hat_host) {
   IpaScratch s;
   fe u_scale;
   fe* a = reinterpret_cast<fe*>(a_in);

@@ -252,4 +252,23 @@ bool host_normalise_wanted(const vdfgpu_gens* g);
 // a^-1 in Montgomery form, computed on the host (a != 0): the per-round challenge inverse of the IPA
 fe host_inv(Fp, const fe& a);
 fe host_inv(Fq, const fe& a);
+
+// api_sumcheck.cu's building blocks, for the Spartan prover of the running instance (api_r1cs.cu).  Instances: Fp and
+// Fq, K = 2 and 3.
+template <int K>
+struct MultiDot;
+// eq(r) over 2^ell entries from ell challenges on the device
+template <class F>
+void eq_evals_enqueue(CudaLaunch& L, const fe* r_dev, size_t ell, fe* out_dev);
+// K inner products over n entries into out[0, K) (sumcheck.cuh MultiDot); partial: sc_grid(n) K elements
+template <class F, int K>
+void multi_dot_enqueue(cudaStream_t st, const MultiDot<K>& d, size_t n, fe* partial, fe* out);
+// per-thread pinned landing zone of small read-backs: 24 elements
+fe* pinned_evals();
+// the round loops of vdfgpu_sumcheck_{cubic,quad}[_dev] and vdfgpu_ipa_prove[_dev]: each is a whole call of its own
+// (several guarded() sections, the callback between them), so it is called outside any guarded() section
+int sumcheck(int field, const void* const* tables, int n_polys, bool on_host, size_t ell, vdfgpu_round_fn fn,
+             void* user, void* final_host);
+int ipa_prove(vdfgpu_gens* g, void* a_in, void* b_in, bool on_host, size_t ell, const void* u_scale_host,
+              vdfgpu_ipa_round_fn fn, void* user, void* a_hat_host);
 }

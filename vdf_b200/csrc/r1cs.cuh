@@ -268,6 +268,75 @@ struct BindHeavyFn {   // index = (position in the heavy list) * THREADS + threa
   }
 };
 
+// ---- Spartan's padded layout (vdfgpu_running_spartan_prove, vdfgpu_r1cs_evaluate) -----------------------------
+// nova's R1CSShape::pad [R]: m = the next power of two >= max(vars, cons); cons and vars are both padded to m, and the
+// columns from u on move up by m - vars, so W occupies [0, m), u is column m and X starts at m + 1.  z then has 2m
+// entries (ell_x = log2 m row variables, ell_y = ell_x + 1 column variables); 1 + io <= m is required.
+struct PaddedLayout {
+  uint32_t vars, io;
+  size_t m;
+  uint32_t ell_x;
+  static PaddedLayout of(uint32_t cons, uint32_t vars, uint32_t io) {
+    const uint32_t need = cons > vars ? cons : vars;
+    uint32_t ell = 0;
+    while (((size_t)1 << ell) < need) ell++;
+    return PaddedLayout{vars, io, (size_t)1 << ell, ell};
+  }
+  bool fits() const { return 1 + (size_t)io <= m; }
+  // padded column of the shape's column c
+  VDF_HD size_t col(uint32_t c) const { return c < vars ? c : c + (m - vars); }
+  // the shape's column at padded index j < 2m, or -1 for a padding slot (the inverse of col)
+  VDF_HD int64_t source(size_t j) const {
+    if (j < vars) return (int64_t)j;
+    if (j < m || j > m + io) return -1;
+    return (int64_t)(j - m + vars);
+  }
+  // a 2m-entry table over padded columns read through the shape's column numbers (z_at's mapping)
+  VDF_HD ZView view(const fe* t) const { return ZView{t, t + m, t + m + 1}; }
+};
+
+// the outer sum-check's tables, one thread per padded row r < m: Az, Bz, Cz (RelaxedSatFn's row loop) and
+// D = u Cz + E[r]; rows >= cons are zero.  E holds m entries (the zero-padded snapshot).
+template <class F>
+struct OuterTablesFn {
+  CsrView m;
+  ZView z;
+  const fe* E;
+  fe* Az; fe* Bz; fe* Cz; fe* D;
+  VDF_HD void operator()(size_t idx) const {
+    const uint32_t row = (uint32_t)idx;
+    fe acc[3] = {F::zero(), F::zero(), F::zero()};
+    if (row < m.cons) {
+      const fe one = F::one(), minus_one = F::neg(F::one());
+#pragma unroll
+      for (uint32_t mat = 0; mat < 3; mat++) {
+        const uint32_t lo = m.row_ptr[mat * m.cons + row], hi = m.row_ptr[mat * m.cons + row + 1];
+        for (uint32_t k = lo; k < hi; k++)
+          acc[mat] = mul_acc<F>(acc[mat], fe_load(m.val + k), z_at<F>(z, m.vars, m.col[k]), one, minus_one);
+      }
+    }
+    fe_store(Az + idx, acc[0]);
+    fe_store(Bz + idx, acc[1]);
+    fe_store(Cz + idx, acc[2]);
+    fe_store(D + idx, row < m.cons ? F::add(F::mul(fe_load(z.u), acc[2]), fe_load(E + idx)) : F::zero());
+  }
+};
+
+// the inner sum-check's tables over 2m padded columns j: Mp[j] = M[source(j)], zp[j] = z[source(j)], 0 in padding slots.
+// M: the bound rows (BindRowsFn's output over the shape's columns); z = [W | u | X] through z_at.
+template <class F>
+struct PaddedScatterFn {
+  PaddedLayout pad;
+  const fe* M;
+  ZView z;
+  fe* Mp; fe* zp;
+  VDF_HD void operator()(size_t j) const {
+    const int64_t c = pad.source(j);
+    fe_store(Mp + j, c < 0 ? F::zero() : fe_load(M + c));
+    fe_store(zp + j, c < 0 ? F::zero() : z_at<F>(z, pad.vars, (uint32_t)c));
+  }
+};
+
 // a[i] <- a[i] + r * b[i] over two vectors in one launch (W with W2, E with T)
 template <class F>
 struct FoldFn {

@@ -219,6 +219,46 @@ struct IpaBatchScalarsFn {
   }
 };
 
+// ---- Spartan over a resident running instance (vdfgpu_running_spartan_prove) ---------------------------------------
+// RelaxedR1CSSNARK::prove [R] on the padded layout (r1cs.cuh PaddedLayout; m rows, 2m columns, ell_x = log2 m):
+//   outer  sum_x eq(tau, x) (Az(x) Bz(x) - (u Cz(x) + E(x))) = 0, cubic sum-check over ell_x rounds -> r_x,
+//          claim_Az, claim_Bz from the bound tables, claim_Cz = <Cz, eq(r_x)>, eval_E = <E, eq(r_x)>
+//   inner  sum_y M(y) z(y) = r_A claim_Az + r_B claim_Bz + r_C claim_Cz with M(y) = sum_x eq(r_x, x) (r_A A + r_B B +
+//          r_C C)[x, y], quadratic sum-check over ell_x + 1 rounds -> r_y;  r_y' = r_y[1..]
+//   claims eval_W = <W, eq(r_y')>; the two evaluation claims E(r_x) = eval_E and W(r_y') = eval_W are folded into one
+//          inner-product claim with the challenge rho (nova's fold of two inner-product instances [R]):
+//          T = <E, eq(r_y')> + <W, eq(r_x)>,  a = E + rho W,  b = eq(r_x) + rho eq(r_y'),
+//          c = eval_E + rho T + rho^2 eval_W   (= <a, b>; its commitment is comm_E + rho comm_W)
+//   open   the inner-product argument of <a, b> = c (vdfgpu_ipa_prove above).
+
+// K inner products in one pass: out[q] = sum_{i < len[q]} v[q][i] eq[q][i].  Every vector may be shorter than the
+// launch's n entries: the entries past len[q] are zero (implicit padding, nothing is read there).
+template <int K>
+struct MultiDot {
+  const fe* v[K];
+  const fe* eq[K];
+  size_t len[K];
+  template <class F>
+  VDF_HD void add_terms(fe (&acc)[K], size_t i) const {
+#pragma unroll
+    for (int q = 0; q < K; q++)
+      if (i < len[q]) acc[q] = F::add(acc[q], F::mul(fe_load(v[q] + i), fe_load(eq[q] + i)));
+  }
+};
+
+// a[i] = E[i] + rho W[i], b[i] = eqx[i] + rho eqy[i]: the joint inner-product claim's vectors (a may be E, b may be eqx)
+template <class F>
+struct IpaJoinFn {
+  const fe* E; const fe* W; const fe* eqx; const fe* eqy;
+  fe rho;
+  fe* a; fe* b;
+  VDF_HD void operator()(size_t i) const {
+    const fe e = fe_load(E + i), w = fe_load(W + i), x = fe_load(eqx + i), y = fe_load(eqy + i);
+    fe_store(a + i, F::add(e, F::mul(rho, w)));
+    fe_store(b + i, F::add(x, F::mul(rho, y)));
+  }
+};
+
 constexpr int SC_BLOCK = 256;
 constexpr int SC_MAX_POLYS = 4;
 
@@ -367,6 +407,17 @@ __global__ void __launch_bounds__(SC_BLOCK) sc_cross_dot_kernel(const fe* A, con
     acc[1] = F::add(acc[1], F::mul(fe_load(A + half + i), fe_load(B + i)));
   }
   block_sum_store<F, 2>(acc, partial);
+}
+
+// K inner products over n entries (MultiDot above): per-block partials
+template <class F, int K>
+__global__ void __launch_bounds__(SC_BLOCK) sc_multi_dot_kernel(const MultiDot<K> d, size_t n, fe* partial) {
+  fe acc[K];
+#pragma unroll
+  for (int q = 0; q < K; q++) acc[q] = F::zero();
+  for (size_t i = (size_t)blockIdx.x * SC_BLOCK + threadIdx.x; i < n; i += (size_t)gridDim.x * SC_BLOCK)
+    d.template add_terms<F>(acc, i);
+  block_sum_store<F, K>(acc, partial);
 }
 
 // second stage: out[a] = sum over blocks of partial[block * NACC + a]; one block

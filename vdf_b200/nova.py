@@ -96,6 +96,19 @@ class R1CSShape:
                                                      _lib.as_ptr(fes_to_bytes(r_abc, self.m)), _lib.as_ptr(out)))
         return fes_from_bytes(bytes(out), self.m)
 
+    def evaluate(self, rx: Sequence[int], ry: Sequence[int]) -> Tuple[int, int, int]:
+        """(A, B, C)(r_x, r_y) over nova's padded layout (spartan.padded_layout): the sparse evaluation of
+        RelaxedR1CSSNARK::verify [R].  rx: log2 m coordinates, ry: log2 m + 1, most significant variable first."""
+        from .spartan import padded_layout
+        m, _ = padded_layout(self.num_cons, self.num_vars, self.num_io)
+        ell_x = m.bit_length() - 1
+        if len(rx) != ell_x or len(ry) != ell_x + 1:
+            raise ValueError("evaluate: rx needs log2 m coordinates and ry one more")
+        out = bytearray(96)
+        _lib.check(_lib.load().vdfgpu_r1cs_evaluate(self._h, _lib.as_ptr(fes_to_bytes(rx, self.m) or bytes(32)),
+                                                    _lib.as_ptr(fes_to_bytes(ry, self.m)), _lib.as_ptr(out)))
+        return tuple(fes_from_bytes(bytes(out), self.m))
+
     def commit_T(self, gens: Optional[Generators], W1: Sequence[int], u1: int, X1: Sequence[int],
                  W2: Sequence[int], X2: Sequence[int]) -> Tuple[List[int], Affine]:
         """Cross-term T and its commitment (u2 = 1 for the fresh instance)."""
@@ -222,6 +235,45 @@ class RelaxedR1CSInstance:  # nova RelaxedR1CSInstance
 
 
 @dataclass
+class SpartanProof:
+    """What vdfgpu_running_spartan_prove handed to the transcript, in order (RelaxedR1CSSNARK::prove [R]): the outer
+    sum-check's rounds ((e0, e2, e3), r), the OUTER claims (claim_Az, claim_Bz, claim_Cz, eval_E) and (r_A, r_B, r_C),
+    the inner rounds ((e0, e2), r), the EVAL claims (eval_W, T) and rho, the joint claim c and u_scale, the IPA's
+    (L, R, r) with L and R as 96-byte normalised points, and a_hat."""
+    outer: List[Tuple[Tuple[int, ...], int]]
+    outer_claims: Tuple[int, ...]
+    r_abc: Tuple[int, ...]
+    inner: List[Tuple[Tuple[int, ...], int]]
+    eval_claims: Tuple[int, ...]
+    rho: int
+    c: int
+    u_scale: int
+    ipa: List[Tuple[bytes, bytes, int]]
+    a_hat: int
+
+    @property
+    def r_x(self) -> List[int]:
+        return [r for _, r in self.outer]
+
+    @property
+    def r_y(self) -> List[int]:
+        return [r for _, r in self.inner]
+
+    @classmethod
+    def from_log(cls, log: list, a_hat: int) -> "SpartanProof":
+        rounds = [[], []]
+        claims = {}
+        for e in log:
+            if e[0] == "round":
+                rounds[1 if claims else 0].append((e[1], e[2]))
+            elif e[0] == "claims":
+                claims[e[1]] = (e[2], e[3])
+        (oc, rabc), (ev, rho), (c, us) = (claims[k] for k in range(3))
+        return cls(rounds[0], oc, rabc, rounds[1], ev, rho[0], c[0], us[0],
+                   [(e[1], e[2], e[3]) for e in log if e[0] == "ipa"], a_hat)
+
+
+@dataclass
 class RunningProver:
     """Device-resident running (W, E) for one curve + the instance on the host: NIFS::prove per step."""
     shape: R1CSShape
@@ -257,6 +309,25 @@ class RunningProver:
         rep = (ctypes.c_uint64 * 4)()
         _lib.check(_lib.load().vdfgpu_running_check(self._h, _lib.as_ptr(cW), _lib.as_ptr(cE), rep))
         return SatReport.from_words(rep, self.shape.num_cons)
+
+    def spartan_prove(self, ipa_gens: Generators, tau: Sequence[int], transcript) -> SpartanProof:
+        """RelaxedR1CSSNARK::prove [R] of the resident running instance in one call (vdfgpu_running_spartan_prove):
+        W, E, u and X are not read back.  ipa_gens: at least m + 1 points of this curve, the first m the commitment
+        generators.  tau: log2 m elements.  transcript: an object with sumcheck_round(rnd, evals), claims(stage, values)
+        and ipa_round(rnd, L, R), each returning an integer (or 32 raw bytes); see include/vdfgpu.h for what each stage
+        receives and returns."""
+        from .spartan import padded_layout, spartan_trampolines
+        s = self.shape
+        m_pad, _ = padded_layout(s.num_cons, s.num_vars, s.num_io)
+        if len(tau) != m_pad.bit_length() - 1:
+            raise ValueError("spartan_prove: tau needs log2 m elements")
+        log: list = []
+        cbs = spartan_trampolines(s.m, transcript, log)
+        a_hat = bytearray(32)
+        _lib.check(_lib.load().vdfgpu_running_spartan_prove(
+            self._h, ipa_gens._h, _lib.as_ptr(fes_to_bytes(tau, s.m) or bytes(32)),
+            *[ctypes.cast(cb, ctypes.c_void_p) for cb in cbs], None, _lib.as_ptr(a_hat)))
+        return SpartanProof.from_log(log, fes_from_bytes(bytes(a_hat), s.m)[0])
 
     def prove_step_bytes(self, W2: bytes, X2: bytes, r: Optional[int] = None):
         """One fold of a fresh satisfying (W2, X2): returns (comm_W2, comm_T, r) with points as 96-byte

@@ -219,3 +219,66 @@ def ipa_verify_batch(gens, proofs: Sequence[IpaProof], weights: Sequence[int] | 
                                                    _lib.as_ptr(rs), col(3), col(5), col(6), col(7),
                                                    _lib.as_ptr(fes_to_bytes(weights, order)), _lib.as_ptr(ok)))
     return [bool(v) for v in ok]
+
+
+# ---- Spartan of a resident running instance (RelaxedR1CSSNARK::prove [R], nova.RunningProver.spartan_prove) ----------
+SPARTAN_OUTER, SPARTAN_EVAL, SPARTAN_IPA = 0, 1, 2
+
+
+def padded_layout(num_cons: int, num_vars: int, num_io: int) -> Tuple[int, Callable[[int], int]]:
+    """nova's R1CSShape::pad [R]: m = the next power of two >= max(num_vars, num_cons), and the padded column of the
+    shape's column c (c if c < num_vars, else c + m - num_vars): W occupies [0, m), u is column m, X starts at m + 1, and
+    z has 2m entries.  The library requires 1 + num_io <= m."""
+    need = max(num_cons, num_vars, 1)
+    m = 1 << (need - 1).bit_length()
+    return m, lambda c: c if c < num_vars else c + m - num_vars
+
+
+def _value_bytes(v, m: int) -> bytes:
+    """a callback's answer as the library reads it: an integer (reduced, canonical), or 32 raw bytes passed as they are"""
+    if isinstance(v, (bytes, bytearray)):
+        if len(v) != 32:
+            raise ValueError("a raw value is 32 bytes")
+        return bytes(v)
+    return fe_to_bytes(v, m)
+
+
+def spartan_trampolines(m: int, transcript, log: list):
+    """The three C callbacks of vdfgpu_running_spartan_prove around a Python transcript object with sumcheck_round(rnd,
+    evals), claims(stage, values) and ipa_round(rnd, L, R); each answer is an integer or 32 raw bytes.  Every call is
+    appended to log as ("round", evals, r), ("claims", stage, values, answers) or ("ipa", L, R, r), answers as the
+    library decodes them.  m: the shape's field, which is the IPA set's scalar field.  An exception in the transcript
+    surfaces as VDFGPU_ERR_STATE."""
+    def sc(_user, rnd, evals_ptr, n_evals, r_out):
+        try:
+            evals = tuple(fes_from_bytes(ctypes.string_at(evals_ptr, 32 * n_evals), m))
+            raw = _value_bytes(transcript.sumcheck_round(int(rnd), evals), m)
+            log.append(("round", evals, fe_from_bytes(raw, m)))
+            ctypes.memmove(r_out, raw, 32)
+            return 0
+        except Exception:
+            return 1
+
+    def claims(_user, stage, in_ptr, n_in, out_ptr, n_out):
+        try:
+            vals = tuple(fes_from_bytes(ctypes.string_at(in_ptr, 32 * n_in), m))
+            ans = list(transcript.claims(int(stage), vals))
+            if len(ans) != n_out:
+                raise ValueError("claims: wrong number of answers")
+            raw = b"".join(_value_bytes(v, m) for v in ans)
+            log.append(("claims", int(stage), vals, tuple(fes_from_bytes(raw, m))))
+            ctypes.memmove(out_ptr, raw, 32 * n_out)
+            return 0
+        except Exception:
+            return 1
+
+    def ipa(_user, rnd, L_ptr, R_ptr, r_out):
+        try:
+            L, R = ctypes.string_at(L_ptr, 96), ctypes.string_at(R_ptr, 96)
+            raw = _value_bytes(transcript.ipa_round(int(rnd), L, R), m)
+            log.append(("ipa", L, R, fe_from_bytes(raw, m)))
+            ctypes.memmove(r_out, raw, 32)
+            return 0
+        except Exception:
+            return 1
+    return _lib.ROUND_FN(sc), _lib.CLAIMS_FN(claims), _lib.IPA_ROUND_FN(ipa)
