@@ -359,6 +359,56 @@ int vdfgpu_running_spartan_prove(vdfgpu_running* f, vdfgpu_gens* ipa_gens, const
  * above, A(r_x, r_y) = sum over entries (x, c, v) of v eq(r_x, x) eq(r_y, col(c)); r_x: ell_x elements, r_y: ell_x + 1
  * (most significant variable first).  1 + num_io > m: VDFGPU_ERR_ARG. */
 int vdfgpu_r1cs_evaluate(const vdfgpu_r1cs* s, const void* rx_host, const void* ry_host, void* out3_host);
+/* The same for k points in one pass: out[q] = (A, B, C)(r_x[q], r_y[q]), q < k; rx: [k][ell_x], ry: [k][ell_x + 1],
+ * out: [k][3], proof-major.  eq(r_x[q]) and eq(r_y[q]) are never written out: each is read from two half tables of
+ * about 2^(ell / 2) entries.  k = 0 or 1 + num_io > m: VDFGPU_ERR_ARG. */
+int vdfgpu_r1cs_evaluate_batch(const vdfgpu_r1cs* s, size_t k, const void* rx_host, const void* ry_host,
+                               void* out3_host);
+
+/* RelaxedR1CSSNARK::verify [R] of k proofs over one shape in one call, the transcript left to the caller: it replays
+ * each proof through its own transcript and hands the library the challenges it squeezed.  Notation and padded layout
+ * as for vdfgpu_running_spartan_prove (ell_x = log2 m, derived from the shape; ell_y = ell_x + 1; r_y' = r_y[1..]).
+ * Records are proof-major; scalars are 32-byte Montgomery elements of the shape's field, points 96-byte Jacobian
+ * (X, Y, Z) of ipa_gens' curve, normalised or not, the identity Z = 0.
+ *   inst:   [k][1 + num_io]  u, X
+ *   points: [k][POINTS]      comm_W, comm_E, L_0 .. L_{ell_x - 1}, R_0 .. R_{ell_x - 1}
+ *   proof:  [k][PROOF_FES]   outer rounds (e0, e2, e3) x ell_x, claim_Az, claim_Bz, claim_Cz, eval_E, inner rounds
+ *                            (e0, e2) x ell_y, eval_W, T, a_hat -- what vdfgpu_running_spartan_prove hands to its
+ *                            callbacks, in that order (c is not part of it: the library derives it)
+ *   chal:   [k][CHAL_FES]    tau x ell_x, r_x x ell_x, r_A, r_B, r_C, r_y x ell_y, rho, u_scale, the IPA's r_j x ell_x
+ *   w:      [k]              batch weights
+ * Proof q is valid iff
+ *   1. outer sum-check: starting from claim 0, each round's e1 = claim - e0 and the next claim is the degree-3
+ *      interpolant through e0, e1, e2, e3 at r_x[j]; the final claim = eq(tau, r_x) (claim_Az claim_Bz - u claim_Cz -
+ *      eval_E);
+ *   2. inner sum-check: the same (degree 2) from r_A claim_Az + r_B claim_Bz + r_C claim_Cz at r_y;
+ *   3. its final claim = (r_A A + r_B B + r_C C)(r_x, r_y) z(r_y), z(r_y) = (1 - r_y[0]) eval_W + r_y[0] eval_X,
+ *      eval_X = the zero-padded (u, X) at r_y' (A, B, C as vdfgpu_r1cs_evaluate, for all proofs in one pass);
+ *   4. the opening is valid (the equation of vdfgpu_ipa_verify_batch over ipa_gens, ell = ell_x) with comm_a = comm_E +
+ *      rho comm_W, c = eval_E + rho T + rho^2 eval_W, b_hat = prod_j ((1 - r_x,j) r_j^-1 + r_x,j r_j) + rho prod_j
+ *      ((1 - r_y',j) r_j^-1 + r_y',j r_j), and u_scale; c and b_hat are derived by the library, never taken from the
+ *      caller.
+ * Checks 1, 2 and the derivations run on the host, O(ell + num_io) field operations per proof; the evaluations of 3 run
+ * for all proofs in one device pass; the openings of 4 are ONE weighted sum over ipa_gens as in vdfgpu_ipa_verify_batch
+ * (comm_E and comm_W are two points of its small MSM, with the scalars -w and -w rho), with its single-proof fallback
+ * when the sum is not O.  A proof that fails a host check is left out of both; one that fails 3 is dropped after the
+ * opening.  ok_out[q] = 1 iff proof q is valid; the verdicts fail closed: ok_out is zeroed first and receives a 1 only
+ * when the whole call succeeded and every check of that proof passed.
+ * Verdicts and errors: anything the prover sent is a verdict.  A non-canonical value in the proof record, a
+ * non-canonical u or X, or a point with a coordinate >= p or off y^2 = x^3 + 5 gives ok_out[q] = 0 for that proof only
+ * and leaves it out of the weighted sum.  VDFGPU_ERR_ARG, before any device work: a null pointer, k = 0, ipa_gens of the
+ * wrong curve or with fewer than m + 1 points (U0 = G_m), 1 + num_io > m, a non-canonical value in a challenge record
+ * or a weight, an IPA challenge or a weight that is 0.  A sum-check challenge of 0 is legal.
+ * Soundness: the weights must be uniform and unpredictable to whoever produced the proofs (the OS CSPRNG, e.g. OsRng);
+ * a batch that contains an invalid opening then passes with probability at most 1 / order.  Weights the provers can
+ * predict let two invalid openings cancel.  The library never generates weights.  The shape and ipa_gens stay
+ * referenced for the whole call, which runs on the calling thread's stream and waits outside the library's lock. */
+#define VDFGPU_SPARTAN_PROOF_FES(ell_x) (5 * (ell_x) + 9)
+#define VDFGPU_SPARTAN_CHAL_FES(ell_x) (4 * (ell_x) + 6)
+#define VDFGPU_SPARTAN_POINTS(ell_x) (2 * (ell_x) + 2)
+int vdfgpu_spartan_verify_batch(const vdfgpu_r1cs* s, vdfgpu_gens* ipa_gens, size_t k, const void* inst32_host,
+                                const void* points96_host, const void* proof32_host, const void* chal32_host,
+                                const void* w32_host, uint8_t* ok_out_host);
 
 /* ---- a8: batched MinRoot verification.  Replaces a loop of MinRootVDF::check (src/minroot.rs:369-371)
  * / Evaluation::verify (:424-426) over independent chains.  ok_out[k] = 1 iff

@@ -229,6 +229,106 @@ fn sat_verdict(rep: &[u64; 4]) -> Result<(), NovaError> {
     }
 }
 
+/// What a verifier holds for one Spartan proof of `RelaxedR1CSSNARK::verify` [R]: the instance (u, X, comm_W, comm_E),
+/// tau, the proof's values as the prover's transcript saw them, and the challenges the verifier's own replay of the
+/// transcript squeezed (`GpuShape::spartan_verify_batch`).
+pub struct SpartanVerifyItem<'a, G: GpuCurve> {
+    pub u: G::Scalar,
+    pub x: &'a [G::Scalar],
+    pub comm_w: G::Point,
+    pub comm_e: G::Point,
+    pub tau: &'a [G::Scalar],
+    pub outer: &'a [[G::Scalar; 3]],      // (e0, e2, e3) x ell_x
+    pub outer_claims: [G::Scalar; 4],     // claim_Az, claim_Bz, claim_Cz, eval_E
+    pub inner: &'a [[G::Scalar; 2]],      // (e0, e2) x (ell_x + 1)
+    pub eval_w: G::Scalar,
+    pub t: G::Scalar,
+    pub l: &'a [G::Point],
+    pub r: &'a [G::Point],
+    pub a_hat: G::Scalar,
+    pub r_x: &'a [G::Scalar],
+    pub r_abc: [G::Scalar; 3],
+    pub r_y: &'a [G::Scalar],
+    pub rho: G::Scalar,
+    pub u_scale: G::Scalar,
+    pub ipa_r: &'a [G::Scalar],
+}
+
+/// The sizes of one record of `vdfgpu_spartan_verify_batch` at ell_x = log2 m (the header's VDFGPU_SPARTAN_* macros)
+pub fn spartan_proof_fes(ell_x: usize) -> usize {
+    5 * ell_x + 9
+}
+pub fn spartan_chal_fes(ell_x: usize) -> usize {
+    4 * ell_x + 6
+}
+pub fn spartan_points(ell_x: usize) -> usize {
+    2 * ell_x + 2
+}
+
+/// The four records of `vdfgpu_spartan_verify_batch` in the header's layout, proof-major: (u, X), (comm_W, comm_E,
+/// L_j, R_j), the prover's scalars, the transcript's challenges.  `None` if an item's lengths do not fit ell_x.
+#[allow(clippy::type_complexity)]
+pub fn spartan_records<G: GpuCurve>(ell_x: usize, num_io: usize, items: &[SpartanVerifyItem<'_, G>])
+                                    -> Option<(Vec<G::Scalar>, Vec<G::Point>, Vec<G::Scalar>, Vec<G::Scalar>)> {
+    let (mut inst, mut pts, mut proof, mut chal) = (Vec::new(), Vec::new(), Vec::new(), Vec::new());
+    for it in items {
+        if it.x.len() != num_io || it.tau.len() != ell_x || it.outer.len() != ell_x || it.inner.len() != ell_x + 1
+            || it.l.len() != ell_x || it.r.len() != ell_x || it.r_x.len() != ell_x || it.r_y.len() != ell_x + 1
+            || it.ipa_r.len() != ell_x {
+            return None;
+        }
+        inst.push(it.u);
+        inst.extend_from_slice(it.x);
+        pts.push(it.comm_w);
+        pts.push(it.comm_e);
+        pts.extend_from_slice(it.l);
+        pts.extend_from_slice(it.r);
+        it.outer.iter().for_each(|e| proof.extend_from_slice(e));
+        proof.extend_from_slice(&it.outer_claims);
+        it.inner.iter().for_each(|e| proof.extend_from_slice(e));
+        proof.extend_from_slice(&[it.eval_w, it.t, it.a_hat]);
+        chal.extend_from_slice(it.tau);
+        chal.extend_from_slice(it.r_x);
+        chal.extend_from_slice(&it.r_abc);
+        chal.extend_from_slice(it.r_y);
+        chal.extend_from_slice(&[it.rho, it.u_scale]);
+        chal.extend_from_slice(it.ipa_r);
+    }
+    Some((inst, pts, proof, chal))
+}
+
+impl<G: GpuCurve> GpuShape<G> {
+    /// ell_x = log2 m of nova's padded shape (`R1CSShape::pad` [R])
+    pub fn padded_ell(&self) -> usize {
+        let need = self.num_cons.max(self.num_vars).max(1);
+        need.next_power_of_two().trailing_zeros() as usize
+    }
+    /// `RelaxedR1CSSNARK::verify` [R] of k proofs over this shape in one call, one verdict per proof.  The caller has
+    /// replayed each proof through nova's transcript in the order `GpuRunning::spartan_prove` recalls and filled the
+    /// items' challenges from it; the library runs both sum-checks' checks and derives c and b_hat on the host, the
+    /// sparse evaluations of all proofs in one device pass, and the openings as one weighted sum over `ipa_gens`
+    /// (m + 1 points, gens_c last).  `weights`: one per proof, uniform and unpredictable to the provers (OsRng).
+    pub fn spartan_verify_batch(&self, ipa_gens: &GpuGens<G>, items: &[SpartanVerifyItem<'_, G>],
+                                weights: &[G::Scalar]) -> Result<Vec<bool>, GpuError> {
+        let ell_x = self.padded_ell();
+        if items.is_empty() || weights.len() != items.len() {
+            return Err(GpuError::Argument("spartan_verify_batch: one weight per proof, at least one proof".into()));
+        }
+        let (inst, pts, proof, chal) = spartan_records::<G>(ell_x, self.num_io, items)
+            .ok_or_else(|| GpuError::Argument("spartan_verify_batch: an item does not fit the padded shape".into()))?;
+        debug_assert_eq!(proof.len(), items.len() * spartan_proof_fes(ell_x));
+        debug_assert_eq!(chal.len(), items.len() * spartan_chal_fes(ell_x));
+        debug_assert_eq!(pts.len(), items.len() * spartan_points(ell_x));
+        let mut ok = vec![0u8; items.len()];
+        check(unsafe {
+            sys::vdfgpu_spartan_verify_batch(self.h, ipa_gens.h, items.len(), inst.as_ptr().cast(), pts.as_ptr().cast(),
+                                             proof.as_ptr().cast(), chal.as_ptr().cast(), weights.as_ptr().cast(),
+                                             ok.as_mut_ptr())
+        })?;
+        Ok(ok.into_iter().map(|b| b != 0).collect())
+    }
+}
+
 impl<G: GpuCurve> Drop for GpuShape<G> {
     fn drop(&mut self) {
         unsafe { sys::vdfgpu_r1cs_destroy(self.h) };

@@ -206,6 +206,12 @@ extern "C" {
                                         a_hat32_host: *mut c_void) -> c_int;
     pub fn vdfgpu_r1cs_evaluate(s: *const vdfgpu_r1cs, rx_host: *const c_void, ry_host: *const c_void,
                                 out3_host: *mut c_void) -> c_int;
+    pub fn vdfgpu_r1cs_evaluate_batch(s: *const vdfgpu_r1cs, k: size_t, rx_host: *const c_void, ry_host: *const c_void,
+                                      out3_host: *mut c_void) -> c_int;
+    pub fn vdfgpu_spartan_verify_batch(s: *const vdfgpu_r1cs, ipa_gens: *mut vdfgpu_gens, k: size_t,
+                                       inst32_host: *const c_void, points96_host: *const c_void,
+                                       proof32_host: *const c_void, chal32_host: *const c_void,
+                                       w32_host: *const c_void, ok_out_host: *mut u8) -> c_int;
 
     // ---- a8: batched MinRoot verification
     pub fn vdfgpu_minroot_check_batch(field: c_int, results_state96_host: *const c_void,

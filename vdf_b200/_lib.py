@@ -79,6 +79,8 @@ PROTOTYPES = {
     "vdfgpu_running_check": (c_int, [c_void_p, c_void_p, c_void_p, POINTER(c_uint64)]),
     "vdfgpu_running_spartan_prove": (c_int, [c_void_p] * 8),
     "vdfgpu_r1cs_evaluate": (c_int, [c_void_p] * 4),
+    "vdfgpu_r1cs_evaluate_batch": (c_int, [c_void_p, c_size_t, c_void_p, c_void_p, c_void_p]),
+    "vdfgpu_spartan_verify_batch": (c_int, [c_void_p, c_void_p, c_size_t] + [c_void_p] * 6),
     "vdfgpu_eq_evals": (c_int, [c_int, c_void_p, c_size_t, c_void_p]),
     "vdfgpu_eq_evals_dev": (c_int, [c_int, c_void_p, c_size_t, c_void_p]),
     "vdfgpu_sumcheck_cubic": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p]),

@@ -1,5 +1,6 @@
 // C ABI, part 2: R1CS shape upload (COO -> CSR), multiply_vec, commit_T, fold, and the device-resident
 // running instance used for a chain of fold steps.  Contract and reference pointers: include/vdfgpu.h.
+#include <algorithm>
 #include <cstring>
 #include <memory>
 #include <type_traits>
@@ -961,10 +962,292 @@ static void r1cs_evaluate_enqueue(const vdfgpu_r1cs* s, const PaddedLayout& pad,
   copy_after_sync(out3_host, pin, 3 * sizeof(fe));
 }
 
+// ---- the sparse evaluation of k proofs in one pass, and RelaxedR1CSSNARK::verify of k proofs in one call -------------
+// pinned landing zone of the batched evaluation's 3k values, one per calling thread (its previous call has been waited
+// for), grown on demand
+static fe* pinned_abc(size_t count) {
+  static thread_local fe* p = nullptr;
+  static thread_local size_t cap = 0;
+  if (count > cap) {
+    if (p) cudaFreeHost(p);
+    p = nullptr;
+    cap = 0;
+    VDF_CUDA_CHECK(cudaHostAlloc((void**)&p, count * sizeof(fe), cudaHostAllocDefault));
+    cap = count;
+  }
+  return p;
+}
+
+// (A, B, C)(r_x,q, r_y,q) for q < k (r1cs.cuh): the 4k half tables in one launch, SparseEvalBatchFn over every
+// (row, proof), the per-block partials summed per output.  rx: [k][ell_x], ry: [k][ell_x + 1] on the host (pageable:
+// staged before the copies return); out_host (pinned) receives [k][3] behind the caller's wait.
+template <class F>
+static void r1cs_evaluate_batch_enqueue(const vdfgpu_r1cs* s, const PaddedLayout& pad, size_t k, const fe* rx,
+                                        const fe* ry, fe* out_host, cudaStream_t st) {
+  CudaLaunch L = api_launch(st);
+  const EqHalves h = EqHalves::of(pad.ell_x);
+  uint32_t kq_log = 0;
+  while (kq_log < 5 && ((size_t)1 << kq_log) < k) kq_log++;
+  const uint32_t gy = (uint32_t)((k + (1u << kq_log) - 1) >> kq_log);
+  const size_t rows_per_block = (size_t)SE_BLOCK >> kq_log, need = (s->cons + rows_per_block - 1) / rows_per_block;
+  const uint32_t gx = (uint32_t)std::max<size_t>(1, std::min<size_t>(need, std::max<size_t>(1, 148 * 8 / gy)));
+  const size_t nx = k * pad.ell_x, ny = k * (pad.ell_x + 1);
+  DevBuf<fe> r(nx + ny, st), tables(k * h.per, st), partial((size_t)gx * k * 3, st), res(3 * k, st);
+  h2d(r.p, rx, nx * sizeof(fe), st);
+  h2d(r.p + nx, ry, ny * sizeof(fe), st);
+  L.run<256>(k * h.per, EqHalfTablesBatchFn<F>{r.p, r.p + nx, pad.ell_x, h, tables.p});
+  sparse_eval_batch_kernel<F><<<dim3(gx, gy), SE_BLOCK, 0, st>>>(SparseEvalBatchFn<F>{s->view(), pad, h, tables.p, k},
+                                                                 kq_log, partial.p);
+  sc_column_sum_kernel<F><<<(unsigned)(3 * k), SC_BLOCK, 0, st>>>(partial.p, gx, 3 * k, res.p);
+  VDF_CUDA_CHECK(cudaGetLastError());
+  ctx().launches += 2;
+  d2h(out_host, res.p, 3 * k * sizeof(fe), st);
+}
+
+// Offsets in the records of vdfgpu_spartan_verify_batch (include/vdfgpu.h), ell = ell_x
+struct SpartanRecords {
+  size_t ell;
+  size_t proof_fes() const { return 5 * ell + 9; }
+  size_t chal_fes() const { return 4 * ell + 6; }
+  size_t points() const { return 2 * ell + 2; }
+  // proof: outer rounds (e0, e2, e3) x ell, claim_Az, claim_Bz, claim_Cz, eval_E, inner rounds (e0, e2) x (ell + 1),
+  // eval_W, T, a_hat
+  size_t claims() const { return 3 * ell; }
+  size_t inner() const { return 3 * ell + 4; }
+  size_t eval_W() const { return 5 * ell + 6; }
+  size_t a_hat() const { return 5 * ell + 8; }
+  // challenges: tau x ell, r_x x ell, r_A, r_B, r_C, r_y x (ell + 1), rho, u_scale, the IPA's r_j x ell
+  size_t r_x() const { return ell; }
+  size_t r_abc() const { return 2 * ell; }
+  size_t r_y() const { return 2 * ell + 3; }
+  size_t rho() const { return 3 * ell + 4; }
+  size_t ipa() const { return 3 * ell + 6; }
+};
+
+// What the host derives from k proofs: admit[q] = well-formed and every host check passed; the opening's arrays for
+// ipa_verify_batch (zero for a proof not admitted); the inner final claim and z(r_y) the device's (A, B, C) completes
+struct SpartanVerifyPlan {
+  std::vector<uint8_t> admit;
+  std::vector<fe> r, a_hat, c, b_hat, u_scale, coef;   // [k][ell], [k] x 4, [k][2] = (rho, 1): comm_W, comm_E
+  std::vector<fe> inner_final, z_ry;                   // [k]
+};
+
+// The host checks of proof q, O(ell + io) field operations: canonical values, both sum-checks round by round
+// (interpolation on 0..3 and 0..2 with the denominators inverted once per call), eq(tau, r_x), the outer final claim,
+// eval_X and z(r_y), c and b_hat (r_inv: the IPA challenges' inverses).  The inner final claim waits for (A, B, C).
+template <class F>
+static void spartan_host_check(const SpartanRecords& R, uint32_t io, const fe* inst, const fe* pf, const fe* ch,
+                               const fe* r_inv, const fe (&inv)[2], SpartanVerifyPlan& v, size_t q) {
+  const size_t ell = R.ell;
+  if (!canonical_all<F>(pf, R.proof_fes()) || !canonical_all<F>(inst, 1 + (size_t)io)) return;
+  const fe one = F::one(), two = F::add(one, one), three = F::add(two, one);
+  const fe inv2 = inv[0], inv6 = inv[1];
+  // claim' = the degree-3 (or 2) interpolant through (0, e0), (1, claim - e0), (2, e2) [, (3, e3)] at r
+  auto next = [&](const fe* e, int deg, const fe& claim, const fe& r) {
+    const fe y1 = F::sub(claim, e[0]);
+    const fe a0 = r, a1 = F::sub(r, one), a2 = F::sub(r, two);
+    if (deg == 2)   // y0 a1 a2 / 2 - y1 a0 a2 + y2 a0 a1 / 2
+      return F::add(F::sub(F::mul(F::mul(e[0], F::mul(a1, a2)), inv2), F::mul(y1, F::mul(a0, a2))),
+                    F::mul(F::mul(e[1], F::mul(a0, a1)), inv2));
+    const fe a3 = F::sub(r, three);   // -y0 a1 a2 a3 / 6 + y1 a0 a2 a3 / 2 - y2 a0 a1 a3 / 2 + y3 a0 a1 a2 / 6
+    const fe t0 = F::mul(F::mul(e[0], F::mul(a1, F::mul(a2, a3))), inv6);
+    const fe t1 = F::mul(F::mul(y1, F::mul(a0, F::mul(a2, a3))), inv2);
+    const fe t2 = F::mul(F::mul(e[1], F::mul(a0, F::mul(a1, a3))), inv2);
+    const fe t3 = F::mul(F::mul(e[2], F::mul(a0, F::mul(a1, a2))), inv6);
+    return F::add(F::sub(F::sub(t1, t0), t2), t3);
+  };
+  const fe* tau = ch;
+  const fe* rx = ch + R.r_x();
+  const fe* ry = ch + R.r_y();
+  const fe u = inst[0];
+  fe claim = F::zero(), eq_tau = one;
+  for (size_t j = 0; j < ell; j++) {
+    claim = next(pf + 3 * j, 3, claim, rx[j]);
+    eq_tau = F::mul(eq_tau, F::add(F::mul(tau[j], rx[j]), F::mul(F::sub(one, tau[j]), F::sub(one, rx[j]))));
+  }
+  const fe* cl = pf + R.claims();   // claim_Az, claim_Bz, claim_Cz, eval_E
+  if (!F::eq(claim, F::mul(eq_tau, F::sub(F::sub(F::mul(cl[0], cl[1]), F::mul(u, cl[2])), cl[3])))) return;
+  const fe* rabc = ch + R.r_abc();
+  claim = F::add(F::add(F::mul(rabc[0], cl[0]), F::mul(rabc[1], cl[1])), F::mul(rabc[2], cl[2]));
+  for (size_t j = 0; j <= ell; j++) claim = next(pf + R.inner() + 2 * j, 2, claim, ry[j]);
+  // eval_X = sum_{i <= io} (u, X)[i] eq(r_y', i): eq over the b low variables (2^b > io) times prod (1 - r_y'_j) above
+  uint32_t b = 0;
+  while (((size_t)1 << b) <= io) b++;
+  const fe* ryp = ry + 1;
+  fe high = one;
+  for (size_t j = 0; j + b < ell; j++) high = F::mul(high, F::sub(one, ryp[j]));
+  std::vector<fe> eq_lo(1, high);
+  for (size_t j = ell - b; j < ell; j++) {
+    std::vector<fe> nxt(2 * eq_lo.size());
+    for (size_t i = 0; i < eq_lo.size(); i++) {
+      nxt[2 * i + 1] = F::mul(eq_lo[i], ryp[j]);
+      nxt[2 * i] = F::sub(eq_lo[i], nxt[2 * i + 1]);
+    }
+    eq_lo.swap(nxt);
+  }
+  fe eval_X = F::zero();
+  for (size_t i = 0; i <= io; i++) eval_X = F::add(eval_X, F::mul(inst[i], eq_lo[i]));
+  const fe eval_W = pf[R.eval_W()], T = pf[R.eval_W() + 1], eval_E = cl[3], rho = ch[R.rho()];
+  v.inner_final[q] = claim;
+  v.z_ry[q] = F::add(F::mul(F::sub(one, ry[0]), eval_W), F::mul(ry[0], eval_X));
+  // the opening: c = eval_E + rho T + rho^2 eval_W, b_hat over the terms (1, r_x) and (rho, r_y')
+  v.c[q] = F::add(eval_E, F::mul(rho, F::add(T, F::mul(rho, eval_W))));
+  const fe* r = ch + R.ipa();
+  fe bx = one, by = one;
+  for (size_t j = 0; j < ell; j++) {
+    bx = F::mul(bx, F::add(F::mul(F::sub(one, rx[j]), r_inv[j]), F::mul(rx[j], r[j])));
+    by = F::mul(by, F::add(F::mul(F::sub(one, ryp[j]), r_inv[j]), F::mul(ryp[j], r[j])));
+  }
+  v.b_hat[q] = F::add(bx, F::mul(rho, by));
+  v.a_hat[q] = pf[R.a_hat()];
+  v.u_scale[q] = ch[R.rho() + 1];
+  v.coef[2 * q] = rho;
+  v.coef[2 * q + 1] = one;
+  std::copy(r, r + ell, v.r.begin() + q * ell);
+  v.admit[q] = 1;
+}
+
+// the batched evaluation for the proofs the opening's batch keeps (ipa_verify_batch's hook)
+struct SpartanEvalHook {
+  const vdfgpu_r1cs* s;
+  PaddedLayout pad;
+  const fe* chal;
+  SpartanRecords R;
+  std::vector<size_t> active;
+  std::vector<fe> abc;   // [active][3]
+};
+
+static void spartan_eval_hook(void* user, const std::vector<size_t>& active, cudaStream_t st) {
+  SpartanEvalHook& h = *static_cast<SpartanEvalHook*>(user);
+  const size_t ka = active.size(), lx = h.R.ell, ly = lx + 1;
+  h.active = active;
+  std::vector<fe> rx(ka * lx + 1), ry(ka * ly);
+  for (size_t x = 0; x < ka; x++) {
+    const fe* ch = h.chal + active[x] * h.R.chal_fes();
+    std::copy(ch + h.R.r_x(), ch + h.R.r_x() + lx, rx.begin() + x * lx);
+    std::copy(ch + h.R.r_y(), ch + h.R.r_y() + ly, ry.begin() + x * ly);
+  }
+  fe* pin = pinned_abc(3 * ka);
+  with_field(h.s->field, "spartan_verify_batch", [&](auto F) {
+    r1cs_evaluate_batch_enqueue<decltype(F)>(h.s, h.pad, ka, rx.data(), ry.data(), pin, st);
+  });
+  h.abc.resize(3 * ka);
+  copy_after_sync(h.abc.data(), pin, 3 * ka * sizeof(fe));
+}
+
+// vdfgpu_spartan_verify_batch: the argument checks and the host checks in one guarded() section, then the opening of
+// every admitted proof through ipa_verify_batch, whose first section also enqueues the batched evaluation (one wait
+// for both), then the inner final claims on the host.  Shape and set stay referenced from the host checks to the end.
+static int spartan_verify_batch(const vdfgpu_r1cs* s, vdfgpu_gens* g, size_t k, const fe* inst, const uint8_t* pts,
+                                const fe* proof, const fe* chal, const fe* w, uint8_t* ok) {
+  PaddedLayout pad{};
+  SpartanRecords R{0};
+  SpartanVerifyPlan v;
+  bool holds = false;
+  int rc = guarded([&] {
+    if (!s || !g || !inst || !pts || !proof || !chal || !w || !ok) throw ArgError("spartan_verify_batch: null pointer");
+    if (k == 0) throw ArgError("spartan_verify_batch: no proofs");
+    std::memset(ok, 0, k);
+    check_gens_field(s, g, "spartan_verify_batch: the IPA set: ");
+    pad = PaddedLayout::of(s->cons, s->vars, s->io);
+    if (!pad.fits()) throw ArgError("spartan_verify_batch: 1 + num_io exceeds the padded size m");
+    if (g->n < pad.m + 1) throw ArgError("spartan_verify_batch: the IPA set needs at least m + 1 points");
+    R.ell = pad.ell_x;
+    with_field(s->field, "spartan_verify_batch", [&](auto F) {
+      using Fd = decltype(F);
+      for (size_t q = 0; q < k; q++) {
+        const fe* ch = chal + q * R.chal_fes();
+        if (!canonical_all<Fd>(ch, R.chal_fes()))
+          throw ArgError("spartan_verify_batch: a challenge of the caller's transcript is non-canonical");
+        for (size_t j = 0; j < R.ell; j++)
+          if (!usable_challenge<Fd>(ch[R.ipa() + j])) throw ArgError("spartan_verify_batch: an IPA challenge is 0");
+        if (!usable_challenge<Fd>(w[q])) throw ArgError("spartan_verify_batch: a weight is 0 or non-canonical");
+      }
+      std::vector<fe> r_inv(k * R.ell);
+      for (size_t q = 0; q < k; q++)
+        std::copy(chal + q * R.chal_fes() + R.ipa(), chal + q * R.chal_fes() + R.ipa() + R.ell, r_inv.begin() + q * R.ell);
+      std::vector<fe> inv{Fd::add(Fd::one(), Fd::one()), Fd::zero()};   // 1/2, 1/6
+      inv[1] = Fd::add(Fd::add(inv[0], inv[0]), inv[0]);
+      inv.insert(inv.end(), r_inv.begin(), r_inv.end());
+      batch_invert<Fd>(inv);
+      const fe inv26[2] = {inv[0], inv[1]};
+      const size_t io1 = 1 + (size_t)s->io;
+      v.admit.assign(k, 0);
+      for (auto* x : {&v.a_hat, &v.c, &v.b_hat, &v.u_scale, &v.inner_final, &v.z_ry}) x->assign(k, Fd::zero());
+      v.r.assign(k * R.ell, Fd::one());
+      v.coef.assign(2 * k, Fd::zero());
+      for (size_t q = 0; q < k; q++)
+        spartan_host_check<Fd>(R, s->io, inst + q * io1, proof + q * R.proof_fes(), chal + q * R.chal_fes(),
+                               inv.data() + 2 + q * R.ell, inv26, v, q);
+    });
+    if (std::find(v.admit.begin(), v.admit.end(), 1) == v.admit.end()) return;
+    s->refs++;
+    g->refs++;
+    holds = true;
+  });
+  SpartanEvalHook hook{s, pad, chal, R, {}, {}};
+  std::vector<uint8_t> opened(k, 0), verdict(k, 0);
+  if (rc == VDFGPU_OK && holds) {
+    IpaVerifyArgs a{pts, pts + 2 * 96, pts + (2 + R.ell) * 96, v.r.data(), v.a_hat.data(), v.c.data(),
+                    v.b_hat.data(), v.u_scale.data(), w, 2, R.points(), R.points(), v.coef.data(), v.admit.data()};
+    rc = ipa_verify_batch(g, R.ell, k, a, opened.data(), "spartan_verify_batch", spartan_eval_hook, &hook);
+  }
+  // the inner final claim: (r_A A + r_B B + r_C C)(r_x, r_y) z(r_y); a proof failing it is dropped after the opening,
+  // which is sound: the weighted sum passing says nothing in its favour
+  if (rc == VDFGPU_OK && holds)
+    with_field(s->field, "spartan_verify_batch", [&](auto F) {
+      using Fd = decltype(F);
+      for (size_t x = 0; x < hook.active.size(); x++) {
+        const size_t q = hook.active[x];
+        const fe* rabc = chal + q * R.chal_fes() + R.r_abc();
+        const fe* abc = hook.abc.data() + 3 * x;
+        const fe m = Fd::add(Fd::add(Fd::mul(rabc[0], abc[0]), Fd::mul(rabc[1], abc[1])), Fd::mul(rabc[2], abc[2]));
+        verdict[q] = opened[q] && Fd::eq(v.inner_final[q], Fd::mul(m, v.z_ry[q]));
+      }
+    });
+  if (rc == VDFGPU_OK) std::memcpy(ok, verdict.data(), k);
+  if (holds) {
+    std::string keep = rc == VDFGPU_OK ? std::string() : std::string(vdfgpu_last_error());
+    guarded([&] {
+      s->refs--;
+      g->refs--;
+    });
+    if (rc != VDFGPU_OK) set_error(keep);
+  }
+  return rc;
+}
+
 }  // namespace vdf
 
 extern "C" {
 #pragma GCC visibility push(default)
+
+int vdfgpu_r1cs_evaluate_batch(const vdfgpu_r1cs* s, size_t k, const void* rx_host, const void* ry_host,
+                               void* out3_host) {
+  return guarded([&] {
+    if (!s || !rx_host || !ry_host || !out3_host) throw ArgError("r1cs_evaluate_batch: null pointer");
+    if (k == 0) throw ArgError("r1cs_evaluate_batch: no points");
+    const PaddedLayout pad = PaddedLayout::of(s->cons, s->vars, s->io);
+    if (!pad.fits()) throw ArgError("r1cs_evaluate_batch: 1 + num_io exceeds the padded size m");
+    with_field(s->field, "r1cs_evaluate_batch", [&](auto F) {
+      require_ready();
+      cudaStream_t st = cur_stream();
+      fe* pin = pinned_abc(3 * k);
+      r1cs_evaluate_batch_enqueue<decltype(F)>(s, pad, k, reinterpret_cast<const fe*>(rx_host),
+                                               reinterpret_cast<const fe*>(ry_host), pin, st);
+      sync_after_unlock(st);
+      copy_after_sync(out3_host, pin, 3 * k * sizeof(fe));
+    });
+  });
+}
+
+int vdfgpu_spartan_verify_batch(const vdfgpu_r1cs* s, vdfgpu_gens* ipa_gens, size_t k, const void* inst32_host,
+                                const void* points96_host, const void* proof32_host, const void* chal32_host,
+                                const void* w32_host, uint8_t* ok_out_host) {
+  auto fes = [](const void* p) { return reinterpret_cast<const fe*>(p); };
+  return spartan_verify_batch(s, ipa_gens, k, fes(inst32_host), reinterpret_cast<const uint8_t*>(points96_host),
+                              fes(proof32_host), fes(chal32_host), fes(w32_host), ok_out_host);
+}
 
 int vdfgpu_running_spartan_prove(vdfgpu_running* f, vdfgpu_gens* ipa_gens, const void* tau_host,
                                  vdfgpu_round_fn sc_round, vdfgpu_spartan_claims_fn claims,

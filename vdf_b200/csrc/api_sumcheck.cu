@@ -192,12 +192,6 @@ static void poly_evaluate_enqueue(const fe* poly_dev, const void* r_host, size_t
 }
 
 // ---- the inner-product argument (notation: sumcheck.cuh) -------------------------------------------------------
-// a challenge the round loop can use: canonical (< m, so r = m is not a disguised 0) and not 0, which has no inverse
-template <class F>
-static bool usable_challenge(const fe& r) {
-  return F::is_canonical(r) && !F::is_zero(r);
-}
-
 struct IpaScratch {   // per-call device scratch of the IPA round loop (stream-ordered pool allocations)
   fe* a = nullptr;         // host form only: the uploaded a and b
   fe* b = nullptr;
@@ -351,18 +345,15 @@ static void ipa_gens_hat_enqueue(vdfgpu_gens* g, const fe* r, const fe* r_inv, s
 }
 
 // ---- batch verification of inner-product arguments (notation: sumcheck.cuh) ---------------------------------------
-struct IpaVerifyArgs {   // the caller's arrays, as vdfgpu_ipa_verify_batch takes them
-  const uint8_t* comm; const uint8_t* L; const uint8_t* R;   // 96-byte Jacobian points
-  const fe* r; const fe* a_hat; const fe* c; const fe* b_hat; const fe* u_scale; const fe* w;
-};
-
-// What the host derives from the well-formed proofs ("active", in order, ka of them; per = 2 ell + 1 points each)
+// What the host derives from the well-formed proofs ("active", in order, ka of them; per = terms + 2 ell points each)
 struct IpaVerifyPlan {
+  size_t per = 0;
   std::vector<size_t> active;
   std::vector<fe> rr;             // r [ka][ell], then r^-1 [ka][ell], then w a_hat [ka]: the IpaHalfTablesFn inputs
   std::vector<fe> last;           // [ka] w u_scale (a_hat b_hat - c): S[n] of proof q alone; the batch's is their sum
-  std::vector<uint8_t> pts72;     // [ka][per] comm_a, L_0 .. L_{ell-1}, R_0 .. R_{ell-1} as 72-byte affine records
-  std::vector<fe> small;          // [ka][per] their scalars -w, -w r_j^2, -w r_j^-2
+  std::vector<uint8_t> pts72;     // [ka][per] the commitment's terms, L_0 .. L_{ell-1}, R_0 .. R_{ell-1} as 72-byte
+                                  // affine records
+  std::vector<fe> small;          // [ka][per] their scalars -w coef_t, -w r_j^2, -w r_j^-2
 };
 
 struct IpaVerifyScratch {   // device buffers of one call, kept for the single-proof checks of a failing batch
@@ -378,41 +369,24 @@ struct IpaVerifyScratch {   // device buffers of one call, kept for the single-p
   std::vector<void*> all() const { return {rr, tables, S, small, raw, pts, out, S4, small4}; }
 };
 
-// v[i] <- v[i]^-1 for non-zero v with ONE inversion (Montgomery's trick)
-template <class F>
-static void batch_invert(std::vector<fe>& v) {
-  if (v.empty()) return;
-  std::vector<fe> pre(v.size());
-  fe acc = F::one();
-  for (size_t i = 0; i < v.size(); i++) {
-    pre[i] = acc;
-    acc = F::mul(acc, v[i]);
-  }
-  fe inv = host_inv(F{}, acc);
-  for (size_t i = v.size(); i-- > 0;) {
-    const fe vi = v[i];
-    v[i] = F::mul(inv, pre[i]);
-    inv = F::mul(inv, vi);
-  }
-}
-
-// The host half of the call: the well-formed proofs (the others keep verdict 0), their points checked on the curve and
-// written as affine records (one batched inversion for every Z other than 0 and 1; L and R from vdfgpu_ipa_prove have
-// Z = 1), r^-1 by one batched inversion, and the scalars of both MSMs.  Challenges and weights were checked by the
-// caller.
+// The host half of the call: the well-formed admitted proofs (the others keep verdict 0), their points checked on the
+// curve and written as affine records (one batched inversion for every Z other than 0 and 1; L and R from
+// vdfgpu_ipa_prove have Z = 1), r^-1 by one batched inversion, and the scalars of both MSMs.  Challenges and weights
+// were checked by the caller.
 template <class BF, class SF>
 static IpaVerifyPlan ipa_verify_prepare(size_t ell, size_t k, const IpaVerifyArgs& a) {
   std::vector<uint8_t> good(k);   // well-formed so far
-  const size_t per = 2 * ell + 1;
+  const size_t nt = a.terms, per = nt + 2 * ell;
   const fe one = BF::one(), b = BF::add(BF::add(BF::add(one, one), BF::add(one, one)), one);   // y^2 = x^3 + 5
   auto point = [&](size_t q, size_t i) -> const uint8_t* {
-    return i == 0 ? a.comm + 96 * q : i <= ell ? a.L + 96 * (q * ell + i - 1) : a.R + 96 * (q * ell + i - 1 - ell);
+    return i < nt ? a.comm + 96 * (q * a.comm_stride + i)
+                  : i < nt + ell ? a.L + 96 * (q * a.lr_stride + i - nt) : a.R + 96 * (q * a.lr_stride + i - nt - ell);
   };
   std::vector<fe> X(k * per), Y(k * per), Z(k * per), zi;
   std::vector<size_t> zi_at;
   for (size_t q = 0; q < k; q++) {
-    good[q] = SF::is_canonical(a.a_hat[q]) && SF::is_canonical(a.c[q]) && SF::is_canonical(a.b_hat[q]) &&
-            SF::is_canonical(a.u_scale[q]);
+    good[q] = (!a.admit || a.admit[q]) && SF::is_canonical(a.a_hat[q]) && SF::is_canonical(a.c[q]) &&
+              SF::is_canonical(a.b_hat[q]) && SF::is_canonical(a.u_scale[q]);
     for (size_t i = 0; good[q] && i < per; i++) {
       const size_t at = q * per + i;
       std::memcpy(&X[at], point(q, i), 32);
@@ -433,6 +407,7 @@ static IpaVerifyPlan ipa_verify_prepare(size_t ell, size_t k, const IpaVerifyArg
     Y[at] = BF::mul(Y[at], BF::mul(z2, zi[m]));
   }
   IpaVerifyPlan p;
+  p.per = per;
   for (size_t q = 0; q < k; q++) {
     for (size_t i = 0; good[q] && i < per; i++) {
       const size_t at = q * per + i;
@@ -459,10 +434,10 @@ static IpaVerifyPlan ipa_verify_prepare(size_t ell, size_t k, const IpaVerifyArg
     scale[x] = SF::mul(w, a.a_hat[q]);
     p.last[x] = SF::mul(SF::mul(w, a.u_scale[q]), SF::sub(SF::mul(a.a_hat[q], a.b_hat[q]), a.c[q]));
     fe* sm = p.small.data() + x * per;
-    sm[0] = nw;
+    for (size_t t = 0; t < nt; t++) sm[t] = a.coef ? SF::mul(nw, a.coef[q * nt + t]) : nw;
     for (size_t j = 0; j < ell; j++) {
-      sm[1 + j] = SF::mul(nw, SF::mul(r[x * ell + j], r[x * ell + j]));
-      sm[1 + ell + j] = SF::mul(nw, SF::mul(r_inv[x * ell + j], r_inv[x * ell + j]));
+      sm[nt + j] = SF::mul(nw, SF::mul(r[x * ell + j], r[x * ell + j]));
+      sm[nt + ell + j] = SF::mul(nw, SF::mul(r_inv[x * ell + j], r_inv[x * ell + j]));
     }
     for (size_t i = 0; i < per; i++) {
       const size_t at = q * per + i;
@@ -533,7 +508,7 @@ static void ipa_verify_chunk_enqueue(vdfgpu_gens* g, size_t ell, const IpaVerify
                                      size_t first, uint32_t kc, void* out_host) {
   cudaStream_t st = cur_stream();
   CudaLaunch L = api_launch(st);
-  const size_t ka = p.active.size(), n = (size_t)1 << ell, ns = p.small.size(), per = 2 * ell + 1;
+  const size_t ka = p.active.size(), n = (size_t)1 << ell, ns = p.small.size(), per = p.per;
   const uint32_t lo_bits = (uint32_t)(ell / 2), hi_bits = (uint32_t)ell - lo_bits;
   if (!s.S4) {
     s.S4 = pool_alloc<fe>(MSM_MAX_BATCH * (n + 1), st);
@@ -567,33 +542,36 @@ static void ipa_verify_chunk_enqueue(vdfgpu_gens* g, size_t ell, const IpaVerify
   normalise_after_sync(reinterpret_cast<uint8_t*>(out_host) + MSM_MAX_BATCH * sizeof(jac_t), kc, g->curve);
 }
 
-// vdfgpu_ipa_verify_batch.  Like ipa_prove, the call holds a reference on g from its first guarded() section to its
-// last; the batch is one section, each chunk of single-proof checks of a failing batch one more.  The verdicts fail
-// closed: ok is zeroed first, and a 1 reaches it only when the whole call succeeded and that proof's check passed.
-static int ipa_verify_batch(vdfgpu_gens* g, size_t ell, size_t k, const IpaVerifyArgs& a, uint8_t* ok) {
+// vdfgpu_ipa_verify_batch (ctx.cuh).  Like ipa_prove, the call holds a reference on g from its first guarded() section
+// to its last; the batch is one section, each chunk of single-proof checks of a failing batch one more.  The verdicts
+// fail closed: ok is zeroed first, and a 1 reaches it only when the whole call succeeded and that proof's check passed.
+int ipa_verify_batch(vdfgpu_gens* g, size_t ell, size_t k, const IpaVerifyArgs& a, uint8_t* ok, const char* who,
+                     IpaVerifyHook hook, void* hook_user) {
   IpaVerifyPlan p;
   IpaVerifyScratch s;
   bool holds_g = false;
   uint8_t sum[96];
   std::vector<uint8_t> verdict(k, 0);
+  const std::string name(who);
   int rc = guarded([&] {
     if (!g || !a.comm || !a.a_hat || !a.c || !a.b_hat || !a.u_scale || !a.w || !ok || (ell && (!a.L || !a.R || !a.r)))
-      throw ArgError("ipa_verify_batch: null pointer");   // L, R and r may be NULL at ell = 0
-    if (k == 0) throw ArgError("ipa_verify_batch: no proofs");
+      throw ArgError(name + ": null pointer");   // L, R and r may be NULL at ell = 0
+    if (k == 0) throw ArgError(name + ": no proofs");
     std::memset(ok, 0, k);
     if (ell > 40 || g->n < ((size_t)1 << ell) + 1)
-      throw ArgError("ipa_verify_batch: the generator set needs at least 2^ell + 1 points");
-    with_curve(g->curve, "ipa_verify_batch", [&](auto C, auto BF, auto SF) {
+      throw ArgError(name + ": the generator set needs at least 2^ell + 1 points");
+    with_curve(g->curve, who, [&](auto C, auto BF, auto SF) {
       using F = decltype(SF);
       for (size_t i = 0; i < k * ell; i++)
-        if (!usable_challenge<F>(a.r[i])) throw ArgError("ipa_verify_batch: a challenge is 0 or non-canonical");
+        if (!usable_challenge<F>(a.r[i])) throw ArgError(name + ": a challenge is 0 or non-canonical");
       for (size_t q = 0; q < k; q++)
-        if (!usable_challenge<F>(a.w[q])) throw ArgError("ipa_verify_batch: a weight is 0 or non-canonical");
+        if (!usable_challenge<F>(a.w[q])) throw ArgError(name + ": a weight is 0 or non-canonical");
       p = ipa_verify_prepare<decltype(BF), F>(ell, k, a);
       if (p.active.empty()) return;
       require_ready();
       g->refs++;
       holds_g = true;
+      if (hook) hook(hook_user, p.active, cur_stream());
       ipa_verify_batch_enqueue<decltype(C), F>(g, ell, p, s, sum);
     });
   });
@@ -604,13 +582,13 @@ static int ipa_verify_batch(vdfgpu_gens* g, size_t ell, size_t k, const IpaVerif
       uint8_t res[2 * MSM_MAX_BATCH][96];
       rc = guarded([&] {
         require_ready();
-        with_curve(g->curve, "ipa_verify_batch", [&](auto, auto, auto SF) {
+        with_curve(g->curve, who, [&](auto, auto, auto SF) {
           ipa_verify_chunk_enqueue<decltype(SF)>(g, ell, p, s, first, kc, res);
         });
       });
       if (rc != VDFGPU_OK) break;
       // proof valid iff (its share over g) = -(its share over its own points): both normalised, identity all zero
-      with_curve(g->curve, "ipa_verify_batch", [&](auto, auto BF, auto) {
+      with_curve(g->curve, who, [&](auto, auto BF, auto) {
         using F = decltype(BF);
         for (uint32_t j = 0; j < kc; j++) {
           fe P[3], Q[3];
@@ -815,8 +793,8 @@ int vdfgpu_ipa_verify_batch(vdfgpu_gens* g, size_t ell, size_t k, const void* co
   auto fes = [](const void* p) { return reinterpret_cast<const fe*>(p); };
   const IpaVerifyArgs a{reinterpret_cast<const uint8_t*>(comm_a96_host), reinterpret_cast<const uint8_t*>(L96_host),
                         reinterpret_cast<const uint8_t*>(R96_host), fes(r32_host), fes(a_hat32_host), fes(c32_host),
-                        fes(b_hat32_host), fes(u_scale32_host), fes(w32_host)};
-  return ipa_verify_batch(g, ell, k, a, ok_out_host);
+                        fes(b_hat32_host), fes(u_scale32_host), fes(w32_host), 1, 1, ell};
+  return ipa_verify_batch(g, ell, k, a, ok_out_host, "ipa_verify_batch");
 }
 
 #pragma GCC visibility pop

@@ -271,4 +271,46 @@ int sumcheck(int field, const void* const* tables, int n_polys, bool on_host, si
              void* user, void* final_host);
 int ipa_prove(vdfgpu_gens* g, void* a_in, void* b_in, bool on_host, size_t ell, const void* u_scale_host,
               vdfgpu_ipa_round_fn fn, void* user, void* a_hat_host);
+
+// a challenge the round loop can use: canonical (< m, so r = m is not a disguised 0) and not 0, which has no inverse
+template <class F>
+bool usable_challenge(const fe& r) {
+  return F::is_canonical(r) && !F::is_zero(r);
+}
+
+// v[i] <- v[i]^-1 for non-zero v with ONE inversion (Montgomery's trick)
+template <class F>
+void batch_invert(std::vector<fe>& v) {
+  if (v.empty()) return;
+  std::vector<fe> pre(v.size());
+  fe acc = F::one();
+  for (size_t i = 0; i < v.size(); i++) {
+    pre[i] = acc;
+    acc = F::mul(acc, v[i]);
+  }
+  fe inv = host_inv(F{}, acc);
+  for (size_t i = v.size(); i-- > 0;) {
+    const fe vi = v[i];
+    v[i] = F::mul(inv, pre[i]);
+    inv = F::mul(inv, vi);
+  }
+}
+
+// Batch verification of inner-product arguments (vdfgpu_ipa_verify_batch; notation in sumcheck.cuh), shared with the
+// Spartan verifier (api_r1cs.cu).  Proof q's commitment is a short sum of terms, comm_a = sum_t coef[q][t] P[q][t]:
+// vdfgpu_ipa_verify_batch has one term with coefficient 1, the Spartan opening comm_E + rho comm_W two.  Point j of
+// proof q's commitment is at comm + 96 (q comm_stride + j), L_j at L + 96 (q lr_stride + j), R_j likewise.
+struct IpaVerifyArgs {
+  const uint8_t* comm; const uint8_t* L; const uint8_t* R;   // 96-byte Jacobian points
+  const fe* r; const fe* a_hat; const fe* c; const fe* b_hat; const fe* u_scale; const fe* w;
+  size_t terms = 1, comm_stride = 1, lr_stride = 0;
+  const fe* coef = nullptr;          // [k][terms]; nullptr: every coefficient is 1
+  const uint8_t* admit = nullptr;    // [k]: 0 for a proof the caller has already rejected; nullptr: all admitted
+};
+// Runs after the host checks inside the call's first guarded() section, on its stream, before the batch is enqueued:
+// it may enqueue work and read-backs for the active proofs (ascending), which land behind the batch's one wait.
+using IpaVerifyHook = void (*)(void* user, const std::vector<size_t>& active, cudaStream_t st);
+// ok: k verdicts (zeroed first; fail closed).  `who` names the entry point in argument errors.
+int ipa_verify_batch(vdfgpu_gens* g, size_t ell, size_t k, const IpaVerifyArgs& a, uint8_t* ok, const char* who,
+                     IpaVerifyHook hook = nullptr, void* hook_user = nullptr);
 }

@@ -337,6 +337,128 @@ struct PaddedScatterFn {
   }
 };
 
+// ---- the sparse evaluation of k proofs in one pass (vdfgpu_r1cs_evaluate_batch, vdfgpu_spartan_verify_batch) ----------
+// (A, B, C)(r_x,q, r_y,q) for q < k over the padded layout, sum over entries (x, c, v) of v eq(r_x,q)[x] eq(r_y,q)[col(c)].
+// Per proof q, eq(r_x) and eq(r_y) are never written out: eq(r)[i] = Hi(r)[i >> lo_bits] Lo(r)[i & (2^lo_bits - 1)]
+// (EqCombineFn's factorisation), lo_bits = floor(ell / 2).  Four half tables per proof, back to back at q * per:
+// Hi(r_x), Lo(r_x), Hi(r_y), Lo(r_y) -- 2^9 entries each at ell_y = 18, about 4 MB at k = 64, resident in L2.
+struct EqHalves {
+  uint32_t bits[4];   // table t has 2^bits[t] entries: Hi(r_x), Lo(r_x), Hi(r_y), Lo(r_y)
+  size_t off[4];      // its offset in a proof's record
+  size_t per;         // entries per proof
+  static EqHalves of(uint32_t ell_x) {
+    const uint32_t ell_y = ell_x + 1;
+    EqHalves h{{ell_x - ell_x / 2, ell_x / 2, ell_y - ell_y / 2, ell_y / 2}, {0, 0, 0, 0}, 0};
+    for (int t = 0; t < 4; t++) {
+      h.off[t] = h.per;
+      h.per += (size_t)1 << h.bits[t];
+    }
+    return h;
+  }
+  // eq(r_x) (t = 0) or eq(r_y) (t = 2) of the proof whose record starts at `rec`, at index i: one multiplication
+  template <class F>
+  VDF_HD fe at(const fe* rec, int t, size_t i) const {
+    return F::mul(fe_load(rec + off[t] + (i >> bits[t + 1])), fe_load(rec + off[t + 1] + (i & (((size_t)1 << bits[t + 1]) - 1))));
+  }
+};
+
+// All k proofs' half tables in one launch, index space k per: entry e of table t of proof q is EqPartFn over the bit
+// range of r that table covers (Hi: the first bits[0] / bits[2] coordinates, Lo: the rest).  rx: [k][ell_x],
+// ry: [k][ell_x + 1], most significant variable first.
+template <class F>
+struct EqHalfTablesBatchFn {
+  const fe* rx; const fe* ry;
+  uint32_t ell_x;
+  EqHalves h;
+  fe* out;   // [k][h.per]
+  VDF_HD void operator()(size_t idx) const {
+    const size_t q = idx / h.per, e = idx - q * h.per;
+    // which table: selects rather than a run-time index into h, which would put h in local memory
+    const bool y = e >= h.off[2], lo = y ? e >= h.off[3] : e >= h.off[1];
+    const size_t i = e - (y ? (lo ? h.off[3] : h.off[2]) : (lo ? h.off[1] : 0));
+    const fe* r = y ? ry + q * (ell_x + 1) : rx + q * ell_x;
+    const uint32_t hb = y ? h.bits[2] : h.bits[0], first = lo ? hb : 0u, nbits = lo ? (y ? h.bits[3] : h.bits[1]) : hb;
+    const fe one = F::one();
+    fe acc = one;
+#pragma unroll 1
+    for (uint32_t j = 0; j < nbits; j++) {
+      const fe rj = fe_load(r + first + j);
+      acc = F::mul(acc, ((i >> (nbits - 1 - j)) & 1u) ? rj : F::sub(one, rj));
+    }
+    fe_store(out + idx, acc);
+  }
+};
+
+// One (row, proof) term of the batch: for row x < cons and proof q, acc[mat] += eq_x,q[x] sum_{entries (c, v) of row x
+// of mat} v eq_y,q[col(c)].  One multiplication per entry for its eq_y value (from the halves), mul_acc's for v (an
+// addition when v = +-1), four per row: nnz (1 + f) + 4 cons per proof, f the share of non-unit coefficients.
+template <class F>
+struct SparseEvalBatchFn {
+  CsrView m;
+  PaddedLayout pad;
+  EqHalves h;
+  const fe* tables;   // EqHalfTablesBatchFn's output, [k][h.per]
+  size_t k;
+  VDF_HD void add_row(fe (&acc)[3], size_t q, uint32_t row) const {
+    const fe* rec = tables + q * h.per;
+    const fe one = F::one(), minus_one = F::neg(F::one());
+    const fe ex = h.at<F>(rec, 0, row);
+#pragma unroll
+    for (uint32_t mat = 0; mat < 3; mat++) {
+      const uint32_t lo = m.row_ptr[mat * m.cons + row], hi = m.row_ptr[mat * m.cons + row + 1];
+      fe s = F::zero();
+      for (uint32_t e = lo; e < hi; e++)
+        s = mul_acc<F>(s, fe_load(m.val + e), h.at<F>(rec, 2, pad.col(m.col[e])), one, minus_one);
+      acc[mat] = F::add(acc[mat], F::mul(ex, s));
+    }
+  }
+};
+
+#if defined(__CUDACC__)
+constexpr int SE_BLOCK = 256;
+
+// SparseEvalBatchFn over all rows and proofs.  Proofs fastest: the kq = 2^kq_log lanes of a group (kq = k rounded up
+// to a power of two, at most 32) take the proofs blockIdx.y kq + lane, the 32 / kq groups of a warp take different
+// rows, so at k >= 32 a warp's row_ptr, col and val loads are broadcasts.  Each thread runs a strided loop over rows
+// with its proof fixed and three accumulators; a block's sums go to partial[(blockIdx.x k + q) 3 + mat]
+// (sc_column_sum_kernel adds them up over gridDim.x blocks).
+template <class F>
+__global__ void __launch_bounds__(SE_BLOCK) sparse_eval_batch_kernel(const SparseEvalBatchFn<F> f, uint32_t kq_log,
+                                                                     fe* partial) {
+  const uint32_t kq = 1u << kq_log, lane_q = threadIdx.x & (kq - 1u), rows_per_block = SE_BLOCK >> kq_log;
+  const size_t q = (size_t)blockIdx.y * kq + lane_q;
+  fe acc[3] = {F::zero(), F::zero(), F::zero()};
+  if (q < f.k)
+    for (size_t row = (size_t)blockIdx.x * rows_per_block + (threadIdx.x >> kq_log); row < f.m.cons;
+         row += (size_t)gridDim.x * rows_per_block)
+      f.add_row(acc, q, (uint32_t)row);
+  // the lanes of one proof in a warp differ in the bits above kq_log: a butterfly over those bits
+#pragma unroll 1
+  for (uint32_t d = 16; d >= kq; d >>= 1)
+#pragma unroll
+    for (int mat = 0; mat < 3; mat++) {
+      fe o;
+#pragma unroll
+      for (int w = 0; w < 8; w++) o.v[w] = __shfl_xor_sync(0xffffffffu, acc[mat].v[w], d);
+      acc[mat] = F::add(acc[mat], o);
+    }
+  __shared__ fe sm[3][SE_BLOCK / 32][32];
+  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+  if (lane < kq)
+#pragma unroll
+    for (int mat = 0; mat < 3; mat++) sm[mat][warp][lane] = acc[mat];
+  __syncthreads();
+  if (threadIdx.x < 3 * kq) {
+    const uint32_t mat = threadIdx.x >> kq_log, ql = threadIdx.x & (kq - 1u);
+    fe s = sm[mat][0][ql];
+#pragma unroll 1
+    for (int w = 1; w < SE_BLOCK / 32; w++) s = F::add(s, sm[mat][w][ql]);
+    const size_t qq = (size_t)blockIdx.y * kq + ql;
+    if (qq < f.k) fe_store(partial + ((size_t)blockIdx.x * f.k + qq) * 3 + mat, s);
+  }
+}
+#endif  // __CUDACC__
+
 // a[i] <- a[i] + r * b[i] over two vectors in one launch (W with W2, E with T)
 template <class F>
 struct FoldFn {

@@ -432,6 +432,17 @@ __global__ void __launch_bounds__(SC_BLOCK) sc_final_kernel(const fe* partial, u
   block_sum_store<F, NACC>(acc, out);   // gridDim.x == 1: writes out[0 .. NACC)
 }
 
+// second stage of a reduction with many outputs: out[o] = sum over blocks b of partial[b * n_out + o]; one block per
+// output (gridDim.x == n_out)
+template <class F>
+__global__ void __launch_bounds__(SC_BLOCK) sc_column_sum_kernel(const fe* partial, uint32_t nblocks, size_t n_out,
+                                                                 fe* out) {
+  fe acc[1] = {F::zero()};
+  for (uint32_t b = threadIdx.x; b < nblocks; b += SC_BLOCK)
+    acc[0] = F::add(acc[0], fe_load(partial + (size_t)b * n_out + blockIdx.x));
+  block_sum_store<F, 1>(acc, out);   // writes out[blockIdx.x]
+}
+
 // grid for a reduction over `items`: enough blocks to fill the GPU, never more partials than the final block likes
 static inline uint32_t sc_grid(size_t items) {
   size_t blocks = (items + SC_BLOCK - 1) / SC_BLOCK;

@@ -109,6 +109,21 @@ class R1CSShape:
                                                     _lib.as_ptr(fes_to_bytes(ry, self.m)), _lib.as_ptr(out)))
         return tuple(fes_from_bytes(bytes(out), self.m))
 
+    def evaluate_batch(self, rxs: Sequence[Sequence[int]], rys: Sequence[Sequence[int]]) -> List[Tuple[int, int, int]]:
+        """evaluate at k points in one pass (vdfgpu_r1cs_evaluate_batch): one (A, B, C) per (rx, ry) pair."""
+        from .spartan import padded_layout
+        m, _ = padded_layout(self.num_cons, self.num_vars, self.num_io)
+        ell_x = m.bit_length() - 1
+        k = len(rxs)
+        if k == 0 or len(rys) != k or any(len(rx) != ell_x for rx in rxs) or any(len(ry) != ell_x + 1 for ry in rys):
+            raise ValueError("evaluate_batch: k >= 1 points, each rx with log2 m coordinates and ry with one more")
+        out = bytearray(96 * k)
+        _lib.check(_lib.load().vdfgpu_r1cs_evaluate_batch(
+            self._h, k, _lib.as_ptr(fes_to_bytes([v for rx in rxs for v in rx], self.m) or bytes(32)),
+            _lib.as_ptr(fes_to_bytes([v for ry in rys for v in ry], self.m)), _lib.as_ptr(out)))
+        vals = fes_from_bytes(bytes(out), self.m)
+        return [tuple(vals[3 * q:3 * q + 3]) for q in range(k)]
+
     def commit_T(self, gens: Optional[Generators], W1: Sequence[int], u1: int, X1: Sequence[int],
                  W2: Sequence[int], X2: Sequence[int]) -> Tuple[List[int], Affine]:
         """Cross-term T and its commitment (u2 = 1 for the fresh instance)."""

@@ -282,3 +282,60 @@ def spartan_trampolines(m: int, transcript, log: list):
         except Exception:
             return 1
     return _lib.ROUND_FN(sc), _lib.CLAIMS_FN(claims), _lib.IPA_ROUND_FN(ipa)
+
+
+# ---- verification of Spartan proofs in batches (RelaxedR1CSSNARK::verify [R], vdfgpu_spartan_verify_batch) -----------
+# An item as the verifier holds it: the instance (u, X, comm_W, comm_E; commitments as affine tuples or 96-byte
+# Jacobian points), tau, and the SpartanProof the prover's transcript saw.  pf.c is not used: the library derives c.
+SpartanItem = Tuple[int, Sequence[int], object, object, Sequence[int], object]
+
+
+def spartan_records(shape, curve: int, items: Sequence[SpartanItem]) -> Tuple[bytes, bytes, bytes, bytes]:
+    """The four proof-major records vdfgpu_spartan_verify_batch reads (include/vdfgpu.h): (u, X), (comm_W, comm_E,
+    L_j, R_j), the prover's scalars and the transcript's challenges, as bytes.  A commitment None is the identity."""
+    from .encoding import CURVE_BASE
+    from .nova import _point_arg
+    m = shape.m
+    base = CURVE_BASE[curve]
+    inst, pts, proof, chal = [], [], [], []
+    point = lambda c: bytes(96) if c is None else _point_arg(c, base)   # noqa: E731  (None: the identity)
+    for u, X, comm_W, comm_E, tau, pf in items:
+        if len(X) != shape.num_io:
+            raise ValueError("spartan_verify_batch: X needs num_io entries")
+        inst.append(fes_to_bytes([u] + list(X), m))
+        pts.append(point(comm_W) + point(comm_E) + b"".join(L for L, _, _ in pf.ipa) +
+                   b"".join(R for _, R, _ in pf.ipa))
+        proof.append(fes_to_bytes([v for e, _ in pf.outer for v in e] + list(pf.outer_claims) +
+                                  [v for e, _ in pf.inner for v in e] + list(pf.eval_claims) + [pf.a_hat], m))
+        chal.append(fes_to_bytes(list(tau) + pf.r_x + list(pf.r_abc) + pf.r_y + [pf.rho, pf.u_scale] +
+                                 [r for _, _, r in pf.ipa], m))
+    return b"".join(inst), b"".join(pts), b"".join(proof), b"".join(chal)
+
+
+def spartan_verify_records(shape, ipa_gens, k: int, inst: bytes, pts: bytes, proof: bytes, chal: bytes,
+                           weights: Sequence[int] | None = None) -> List[bool]:
+    """vdfgpu_spartan_verify_batch on records already encoded (spartan_records); weights as in spartan_verify_batch."""
+    import secrets
+    m = shape.m
+    if weights is None:
+        weights = [1 + secrets.randbelow(m - 1) for _ in range(k)]
+    if len(weights) != k:
+        raise ValueError("spartan_verify_batch: one weight per proof")
+    ok = bytearray(max(k, 1))
+    _lib.check(_lib.load().vdfgpu_spartan_verify_batch(shape._h, ipa_gens._h, k, _lib.as_ptr(inst), _lib.as_ptr(pts),
+                                                       _lib.as_ptr(proof), _lib.as_ptr(chal),
+                                                       _lib.as_ptr(fes_to_bytes(weights, m) or bytes(32)),
+                                                       _lib.as_ptr(ok)))
+    return [bool(v) for v in ok[:k]]
+
+
+def spartan_verify_batch(shape, ipa_gens, items: Sequence[SpartanItem], weights: Sequence[int] | None = None) -> List[bool]:
+    """RelaxedR1CSSNARK::verify [R] of k proofs over one shape (nova.R1CSShape) in one call, one verdict per proof.
+    ipa_gens: at least m + 1 points of the curve whose scalar field is the shape's (U0 = G_m).  Every proof's
+    challenges must be what the caller's transcript derived from it.  weights: one non-zero weight per proof for the
+    random linear combination of the openings; None draws them with `secrets`.  A caller that passes its own must draw
+    them uniformly and out of the provers' sight: predictable weights let two invalid openings cancel."""
+    if not items:
+        return []
+    inst, pts, proof, chal = spartan_records(shape, ipa_gens.curve, items)
+    return spartan_verify_records(shape, ipa_gens, len(items), inst, pts, proof, chal, weights)
