@@ -60,14 +60,19 @@ def test_point_normalise_host_matches_oracle():
     rng = O.XorShiftRng()
     for cv in (O.PALLAS, O.VESTA):
         m = cv.base
-        buf, want = bytearray(), bytearray()
-        for k in range(20):
-            pt = cv.mul(O.field_random(rng, cv.order), cv.gen)
-            z = O.field_random(rng, m) if k else 1
-            buf += O.fe_to_bytes(pt[0] * z * z, m) + O.fe_to_bytes(pt[1] * z * z * z, m) + O.fe_to_bytes(z, m)
-            want += O.jac_to_bytes(cv, pt)
-        buf += O.fe_to_bytes(5, m) + O.fe_to_bytes(7, m) + bytes(32)      # Z = 0: the identity
-        want += bytes(96)
-        assert lib.vdfgpu_point_normalise_host(cv.cid, _lib.as_ptr(buf), 21) == 0
-        assert bytes(buf) == bytes(want)
+        # Z per point, None = random: 20 points led by a normalised one, then the identity; then 25 points with
+        # Z = 1 and Z = 0 interleaved among un-normalised ones
+        for zs in ([1] + [None] * 19 + [0], [(None, 1, None, 0, None)[k % 5] for k in range(25)]):
+            buf, want = bytearray(), bytearray()
+            for z in zs:
+                if z == 0:      # the identity, whatever X and Y hold
+                    buf += O.fe_to_bytes(5, m) + O.fe_to_bytes(7, m) + bytes(32)
+                    want += bytes(96)
+                    continue
+                pt = cv.mul(O.field_random(rng, cv.order), cv.gen)
+                z = O.field_random(rng, m) if z is None else z
+                buf += O.fe_to_bytes(pt[0] * z * z, m) + O.fe_to_bytes(pt[1] * z * z * z, m) + O.fe_to_bytes(z, m)
+                want += O.jac_to_bytes(cv, pt)
+            assert lib.vdfgpu_point_normalise_host(cv.cid, _lib.as_ptr(buf), len(zs)) == 0
+            assert bytes(buf) == bytes(want)
     assert lib.vdfgpu_point_normalise_host(7, None, 0) == -1

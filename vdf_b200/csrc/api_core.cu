@@ -37,112 +37,6 @@ static long env_long(const char* name, long dflt, long lo, long hi) {
   return v < lo ? lo : (v > hi ? hi : v);
 }
 
-// ---- host-side normalisation of returned points (see ctx.cuh) ----------------------------------------------------
-namespace hostfield {
-typedef unsigned __int128 u128;
-struct Mod { uint64_t m[4], one[4], inv; };   // modulus, R mod m, -m^-1 mod 2^64
-static const Mod FP_MOD = {{0x992d30ed00000001ull, 0x224698fc094cf91bull, 0x0000000000000000ull, 0x4000000000000000ull},
-                           {0x34786d38fffffffdull, 0x992c350be41914adull, 0xffffffffffffffffull, 0x3fffffffffffffffull},
-                           0x992d30ecffffffffull};
-static const Mod FQ_MOD = {{0x8c46eb2100000001ull, 0x224698fc0994a8ddull, 0x0000000000000000ull, 0x4000000000000000ull},
-                           {0x5b2b3e9cfffffffdull, 0x992c350be3420567ull, 0xffffffffffffffffull, 0x3fffffffffffffffull},
-                           0x8c46eb20ffffffffull};
-
-static const Mod& mod_of(Fp) { return FP_MOD; }
-static const Mod& mod_of(Fq) { return FQ_MOD; }
-// the coordinate field of `curve`
-static const Mod& coord_mod(int curve) {
-  return with_curve(curve, "point_normalise_host", [](auto, auto f, auto) -> const Mod& { return mod_of(f); });
-}
-
-static void mul(uint64_t* r, const uint64_t* a, const uint64_t* b, const Mod& f) {   // Montgomery CIOS, 4 x 64
-  uint64_t t[6] = {0, 0, 0, 0, 0, 0};
-  for (int i = 0; i < 4; i++) {
-    u128 c = 0;
-    for (int j = 0; j < 4; j++) { c += (u128)a[j] * b[i] + t[j]; t[j] = (uint64_t)c; c >>= 64; }
-    c += t[4]; t[4] = (uint64_t)c; t[5] = (uint64_t)(c >> 64);
-    const uint64_t q = t[0] * f.inv;
-    c = ((u128)q * f.m[0] + t[0]) >> 64;
-    for (int j = 1; j < 4; j++) { c += (u128)q * f.m[j] + t[j]; t[j - 1] = (uint64_t)c; c >>= 64; }
-    c += t[4]; t[3] = (uint64_t)c; t[4] = t[5] + (uint64_t)(c >> 64);
-  }
-  uint64_t s[4];
-  u128 bw = 0;
-  for (int j = 0; j < 4; j++) { u128 d = (u128)t[j] - f.m[j] - (uint64_t)bw; s[j] = (uint64_t)d; bw = (d >> 64) & 1; }
-  const bool ge = t[4] != 0 || bw == 0;
-  for (int j = 0; j < 4; j++) r[j] = ge ? s[j] : t[j];
-}
-
-static void inv(uint64_t* r, const uint64_t* a, const Mod& f) {   // a^(m-2)
-  uint64_t e[4] = {f.m[0] - 2, f.m[1], f.m[2], f.m[3]};
-  uint64_t acc[4];
-  std::memcpy(acc, f.one, 32);
-  for (int i = 255; i >= 0; i--) {
-    mul(acc, acc, acc, f);
-    if ((e[i >> 6] >> (i & 63)) & 1) mul(acc, acc, a, f);
-  }
-  std::memcpy(r, acc, 32);
-}
-
-// (X, Y, Z) Jacobian, Montgomery limbs -> (X / Z^2, Y / Z^3, 1), or all zero for the identity
-static void normalise(uint8_t* p96, int curve) {
-  const Mod& f = coord_mod(curve);
-  uint64_t X[4], Y[4], Z[4];
-  std::memcpy(X, p96, 32); std::memcpy(Y, p96 + 32, 32); std::memcpy(Z, p96 + 64, 32);
-  if ((Z[0] | Z[1] | Z[2] | Z[3]) == 0) {
-    std::memset(p96, 0, 96);
-    return;
-  }
-  uint64_t zi[4], zi2[4], zi3[4];
-  inv(zi, Z, f);
-  mul(zi2, zi, zi, f);
-  mul(zi3, zi2, zi, f);
-  mul(X, X, zi2, f);
-  mul(Y, Y, zi3, f);
-  std::memcpy(p96, X, 32); std::memcpy(p96 + 32, Y, 32); std::memcpy(p96 + 64, f.one, 32);
-}
-
-// the same for m <= 16 points with one inversion: 1 / (Z_0 ... Z_{m-1}), then the individual inverses by back-substitution
-static void normalise_batch(uint8_t* const* pts, size_t m, int curve) {
-  const Mod& f = coord_mod(curve);
-  uint64_t Z[16][4], pre[16][4], run[4];
-  std::memcpy(run, f.one, 32);
-  for (size_t k = 0; k < m; k++) {
-    std::memcpy(Z[k], pts[k] + 64, 32);
-    std::memcpy(pre[k], run, 32);
-    if (Z[k][0] | Z[k][1] | Z[k][2] | Z[k][3]) mul(run, run, Z[k], f);
-  }
-  uint64_t inv_all[4];
-  inv(inv_all, run, f);
-  for (size_t k = m; k-- > 0;) {
-    if ((Z[k][0] | Z[k][1] | Z[k][2] | Z[k][3]) == 0) {
-      std::memset(pts[k], 0, 96);
-      continue;
-    }
-    uint64_t zi[4], zi2[4], zi3[4], X[4], Y[4];
-    mul(zi, inv_all, pre[k], f);
-    mul(inv_all, inv_all, Z[k], f);
-    std::memcpy(X, pts[k], 32); std::memcpy(Y, pts[k] + 32, 32);
-    mul(zi2, zi, zi, f);
-    mul(zi3, zi2, zi, f);
-    mul(X, X, zi2, f);
-    mul(Y, Y, zi3, f);
-    std::memcpy(pts[k], X, 32); std::memcpy(pts[k] + 32, Y, 32); std::memcpy(pts[k] + 64, f.one, 32);
-  }
-}
-}  // namespace hostfield
-
-static fe host_inv_mod(const fe& a, const hostfield::Mod& f) {
-  uint64_t x[4], r[4];
-  std::memcpy(x, &a, 32);
-  hostfield::inv(r, x, f);
-  fe out;
-  std::memcpy(&out, r, 32);
-  return out;
-}
-fe host_inv(Fp, const fe& a) { return host_inv_mod(a, hostfield::FP_MOD); }
-fe host_inv(Fq, const fe& a) { return host_inv_mod(a, hostfield::FQ_MOD); }
-
 struct PendingNorm { void* p; size_t count; int curve; };
 struct PendingCopy { void* dst; const void* src; size_t bytes; };
 static thread_local std::vector<PendingNorm> t_norms;
@@ -171,19 +65,20 @@ void wait_pending_sync() {
   copies.swap(t_copies);
   if (ev) VDF_CUDA_CHECK(cudaEventSynchronize(ev));
   for (const PendingCopy& cp : copies) std::memcpy(cp.dst, cp.src, cp.bytes);
-  // all points of one call share ONE inversion per curve (Montgomery's trick): a fold step returns two commitments
-  for (int curve = 0; curve < 2; curve++) {
-    uint8_t* pts[16];
-    size_t m = 0;
+  // all points of one call share ONE inversion per curve (Montgomery's trick): a fold step returns two commitments.
+  // They are gathered into one buffer, normalised there and handed back.
+  for (int curve : {VDFGPU_PALLAS, VDFGPU_VESTA}) {
+    std::vector<uint8_t> pts;
     for (const PendingNorm& n : norms)
-      for (size_t k = 0; k < n.count; k++) {
-        if (n.curve != curve) continue;
-        uint8_t* p = reinterpret_cast<uint8_t*>(n.p) + 96 * k;
-        if (m < 16) pts[m++] = p;
-        else hostfield::normalise(p, curve);
+      if (n.curve == curve) pts.insert(pts.end(), (const uint8_t*)n.p, (const uint8_t*)n.p + 96 * n.count);
+    if (pts.empty()) continue;
+    with_curve(curve, "normalise", [&](auto, auto F, auto) { normalise_host<decltype(F)>(pts.data(), pts.size() / 96); });
+    const uint8_t* src = pts.data();
+    for (const PendingNorm& n : norms)
+      if (n.curve == curve) {
+        std::memcpy(n.p, src, 96 * n.count);
+        src += 96 * n.count;
       }
-    if (m == 1) hostfield::normalise(pts[0], curve);
-    else if (m > 1) hostfield::normalise_batch(pts, m, curve);
   }
 }
 
@@ -1138,18 +1033,16 @@ int vdfgpu_point_sum(int curve, const void* points96_host, size_t k, void* out_p
 
 int vdfgpu_point_normalise_host(int curve, void* points96_host, size_t count) {
   try {   // host arithmetic only: no device, no lock
-    hostfield::coord_mod(curve);   // ArgError for an unknown curve
-    if (count && !points96_host) throw ArgError("point_normalise_host: null pointer");
+    with_curve(curve, "point_normalise_host", [&](auto, auto F, auto) {
+      if (count && !points96_host) throw ArgError("point_normalise_host: null pointer");
+      normalise_host<decltype(F)>(points96_host, count);
+    });
   } catch (const ArgError& e) {
     set_error(e.what());
     return VDFGPU_ERR_ARG;
-  }
-  for (size_t k = 0; k < count;) {   // 16 points per inversion
-    uint8_t* pts[16];
-    size_t m = 0;
-    for (; m < 16 && k < count; m++, k++) pts[m] = reinterpret_cast<uint8_t*>(points96_host) + 96 * k;
-    if (m == 1) hostfield::normalise(pts[0], curve);
-    else hostfield::normalise_batch(pts, m, curve);
+  } catch (const std::exception& e) {   // the scratch vectors' allocation, mapped as guarded() maps it
+    set_error(e.what());
+    return VDFGPU_ERR_CUDA;
   }
   return VDFGPU_OK;
 }

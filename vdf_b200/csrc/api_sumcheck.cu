@@ -297,7 +297,7 @@ int ipa_prove(vdfgpu_gens* g, void* a_in, void* b_in, bool on_host, size_t ell, 
       CudaLaunch L = api_launch(cur_stream());
       with_curve(g->curve, "ipa_prove", [&](auto, auto, auto SF) {
         using F = decltype(SF);
-        r_inv = host_inv(SF, r);
+        r_inv = F::inv(r);
         L.run<256>(h > nc ? h : nc, IpaFoldFn<F>{a, b, h, s.coef[cur], s.coef[cur ^ 1], nc, r, r_inv});
       });
     });
@@ -382,37 +382,25 @@ static IpaVerifyPlan ipa_verify_prepare(size_t ell, size_t k, const IpaVerifyArg
     return i < nt ? a.comm + 96 * (q * a.comm_stride + i)
                   : i < nt + ell ? a.L + 96 * (q * a.lr_stride + i - nt) : a.R + 96 * (q * a.lr_stride + i - nt - ell);
   };
-  std::vector<fe> X(k * per), Y(k * per), Z(k * per), zi;
-  std::vector<size_t> zi_at;
+  std::vector<jac_t> P(k * per);   // proof q's points at [q per, (q + 1) per); those not read stay the identity
   for (size_t q = 0; q < k; q++) {
     good[q] = (!a.admit || a.admit[q]) && SF::is_canonical(a.a_hat[q]) && SF::is_canonical(a.c[q]) &&
               SF::is_canonical(a.b_hat[q]) && SF::is_canonical(a.u_scale[q]);
     for (size_t i = 0; good[q] && i < per; i++) {
-      const size_t at = q * per + i;
-      std::memcpy(&X[at], point(q, i), 32);
-      std::memcpy(&Y[at], point(q, i) + 32, 32);
-      std::memcpy(&Z[at], point(q, i) + 64, 32);
-      good[q] = BF::is_canonical(X[at]) && BF::is_canonical(Y[at]) && BF::is_canonical(Z[at]);
-      if (good[q] && !BF::is_zero(Z[at]) && !BF::eq(Z[at], one)) {
-        zi.push_back(Z[at]);
-        zi_at.push_back(at);
-      }
+      jac_t& pt = P[q * per + i];
+      std::memcpy(&pt, point(q, i), sizeof(jac_t));
+      good[q] = BF::is_canonical(pt.X) && BF::is_canonical(pt.Y) && BF::is_canonical(pt.Z);
+      if (!good[q]) pt = jac_t{};   // a non-canonical Z (m itself is one) must not join the shared inversion
     }
   }
-  batch_invert<BF>(zi);
-  for (size_t m = 0; m < zi.size(); m++) {   // x = X / Z^2, y = Y / Z^3
-    const size_t at = zi_at[m];
-    const fe z2 = BF::mul(zi[m], zi[m]);
-    X[at] = BF::mul(X[at], z2);
-    Y[at] = BF::mul(Y[at], BF::mul(z2, zi[m]));
-  }
+  normalise_host<BF>(P.data(), P.size());
   IpaVerifyPlan p;
   p.per = per;
   for (size_t q = 0; q < k; q++) {
     for (size_t i = 0; good[q] && i < per; i++) {
-      const size_t at = q * per + i;
-      if (!BF::is_zero(Z[at]))
-        good[q] = BF::eq(BF::mul(Y[at], Y[at]), BF::add(BF::mul(BF::mul(X[at], X[at]), X[at]), b));
+      const jac_t& pt = P[q * per + i];
+      if (!BF::is_zero(pt.Z))
+        good[q] = BF::eq(BF::mul(pt.Y, pt.Y), BF::add(BF::mul(BF::mul(pt.X, pt.X), pt.X), b));
     }
     if (good[q]) p.active.push_back(q);
   }
@@ -440,13 +428,13 @@ static IpaVerifyPlan ipa_verify_prepare(size_t ell, size_t k, const IpaVerifyArg
       sm[nt + ell + j] = SF::mul(nw, SF::mul(r_inv[x * ell + j], r_inv[x * ell + j]));
     }
     for (size_t i = 0; i < per; i++) {
-      const size_t at = q * per + i;
+      const jac_t& pt = P[q * per + i];
       uint8_t* rec = p.pts72.data() + (x * per + i) * 72;
-      if (BF::is_zero(Z[at])) {
+      if (BF::is_zero(pt.Z)) {
         rec[64] = 1;   // the infinity flag
       } else {
-        std::memcpy(rec, &X[at], 32);
-        std::memcpy(rec + 32, &Y[at], 32);
+        std::memcpy(rec, &pt.X, 32);
+        std::memcpy(rec + 32, &pt.Y, 32);
       }
     }
   }
@@ -774,12 +762,13 @@ int vdfgpu_ipa_gens_hat(vdfgpu_gens* g, const void* r_host, size_t ell, void* ou
   return guarded([&] {
     if (!g || !out_point96_host || (ell && !r_host)) throw ArgError("ipa_gens_hat: null pointer");
     if (ell > 40 || g->n < (size_t)1 << ell) throw ArgError("ipa_gens_hat: the generator set needs at least 2^ell points");
-    std::vector<fe> r(ell ? ell : 1), r_inv(ell ? ell : 1);
+    std::vector<fe> r(ell ? ell : 1);
     if (ell) std::memcpy(r.data(), r_host, ell * sizeof(fe));
+    std::vector<fe> r_inv(r.begin(), r.begin() + ell);
     with_curve(g->curve, "ipa_gens_hat", [&](auto, auto, auto SF) {
       for (size_t j = 0; j < ell; j++)
         if (!usable_challenge<decltype(SF)>(r[j])) throw ArgError("ipa_gens_hat: a challenge is 0 or non-canonical");
-      for (size_t j = 0; j < ell; j++) r_inv[j] = host_inv(SF, r[j]);
+      batch_invert<decltype(SF)>(r_inv);
       require_ready();
       ipa_gens_hat_enqueue<decltype(SF)>(g, r.data(), r_inv.data(), ell, out_point96_host);
     });

@@ -4,6 +4,7 @@
 
 #include <atomic>
 #include <cstdio>
+#include <cstring>
 #include <memory>
 #include <mutex>
 #include <stdexcept>
@@ -243,15 +244,13 @@ void msm_batch_on_device(vdfgpu_gens* g, const fe* const* d_scalars, const size_
 // divide by Z on the host once the copy has landed: one field inversion is a strictly sequential chain of ~335
 // multiplications -- 0.12 ms in a single GPU thread, ~15 us on a CPU core -- and the bytes are identical.  (Same
 // split as the north star's: what cannot be parallelised stays on the host; Rust's to_affine() does this inversion on
-// the host for pasta-msm's results today.)  `count` consecutive 96-byte points at host_ptr, after the pending wait.
+// the host for pasta-msm's results today.)  `count` consecutive 96-byte points at host_ptr, after the pending wait;
+// all the points of one call on one curve go through one normalise_host.
 void normalise_after_sync(void* host_ptr, size_t count, int curve);
 // after the pending wait, before the normalisations: memcpy(dst, src, bytes) -- results land in a pinned bounce buffer
 // with ONE asynchronous copy and are handed to the caller's (usually pageable) pointers on the host
 void copy_after_sync(void* dst, const void* src, size_t bytes);
 bool host_normalise_wanted(const vdfgpu_gens* g);
-// a^-1 in Montgomery form, computed on the host (a != 0): the per-round challenge inverse of the IPA
-fe host_inv(Fp, const fe& a);
-fe host_inv(Fq, const fe& a);
 
 // api_sumcheck.cu's building blocks, for the Spartan prover of the running instance (api_r1cs.cu).  Instances: Fp and
 // Fq, K = 2 and 3.
@@ -288,11 +287,44 @@ void batch_invert(std::vector<fe>& v) {
     pre[i] = acc;
     acc = F::mul(acc, v[i]);
   }
-  fe inv = host_inv(F{}, acc);
+  fe inv = F::inv(acc);
   for (size_t i = v.size(); i-- > 0;) {
     const fe vi = v[i];
     v[i] = F::mul(inv, pre[i]);
     inv = F::mul(inv, vi);
+  }
+}
+
+// `count` 96-byte Jacobian points (X, Y, Z) with coordinates in F, in place and at any alignment: (X / Z^2, Y / Z^3, 1),
+// 96 zero bytes for the identity Z = 0.  Points with Z = 1 are left as they are (every L_j and R_j of
+// vdfgpu_ipa_prove); all the other Zs share one batch_invert.
+template <class F>
+void normalise_host(void* points96, size_t count) {
+  uint8_t* const p = static_cast<uint8_t*>(points96);
+  const fe one = F::one();
+  std::vector<fe> zi;
+  std::vector<uint8_t*> at;
+  for (size_t i = 0; i < count; i++) {
+    fe z;
+    std::memcpy(&z, p + 96 * i + 64, 32);
+    if (F::is_zero(z)) {
+      std::memset(p + 96 * i, 0, 96);
+    } else if (!F::eq(z, one)) {
+      zi.push_back(z);
+      at.push_back(p + 96 * i);
+    }
+  }
+  batch_invert<F>(zi);
+  for (size_t m = 0; m < zi.size(); m++) {
+    fe x, y;
+    std::memcpy(&x, at[m], 32);
+    std::memcpy(&y, at[m] + 32, 32);
+    const fe z2 = F::mul(zi[m], zi[m]);
+    x = F::mul(x, z2);
+    y = F::mul(y, F::mul(z2, zi[m]));
+    std::memcpy(at[m], &x, 32);
+    std::memcpy(at[m] + 32, &y, 32);
+    std::memcpy(at[m] + 64, &one, 32);
   }
 }
 

@@ -7,10 +7,12 @@
 // reduction row needs 3 real 32x32 products (M1, M2, M3) plus a shift for the 2^30 limb.
 //
 // Device path: PTX mad.lo.cc/madc.hi.cc chains laid out in even/odd columns so ptxas fuses every
-// (lo, hi) pair into one IMAD.WIDE.U32(.X) with the carry in a predicate.  Host path (only compiled
-// for the CPU emulation tool under tests/emul, never for the product): plain 64-bit C.
+// (lo, hi) pair into one IMAD.WIDE.U32(.X) with the carry in a predicate.  Host path (the library's host-side
+// checks, normalisations and inversions, and the CPU emulation under tests/emul): plain C, the multiplier over
+// 4 x 64-bit limbs with 128-bit products.
 #pragma once
 #include <cstdint>
+#include <cstring>
 
 #if defined(__CUDACC__)
 #define VDF_HD __host__ __device__ __forceinline__
@@ -447,38 +449,45 @@ struct Field {
     }
     merge_final(r, even, odd);
 #else
-    // generic CIOS, 32-bit limbs (host emulation only)
-    uint32_t t[10] = {0};
-    for (int i = 0; i < 8; i++) {
-      uint64_t c = 0;
-      for (int j = 0; j < 8; j++) {
-        c += (uint64_t)a.v[j] * b.v[i] + t[j];
-        t[j] = (uint32_t)c;
-        c >>= 32;
+    // CIOS over 4 x 64-bit limbs: the 32-bit limbs above read as little-endian u64 pairs, m = [(M1 << 32) | 1,
+    // (M3 << 32) | M2, 0, 2^62] and -m^-1 mod 2^64 = (M1 << 32) - 1
+    typedef unsigned __int128 u128;
+    const uint64_t m[4] = {((uint64_t)M1 << 32) | 1u, ((uint64_t)M3 << 32) | M2, 0, (uint64_t)M7 << 32};
+    const uint64_t minv = ((uint64_t)M1 << 32) - 1u;
+    uint64_t x[4], y[4], t[6] = {0, 0, 0, 0, 0, 0};
+    std::memcpy(x, a.v, 32);
+    std::memcpy(y, b.v, 32);
+    for (int i = 0; i < 4; i++) {
+      u128 c = 0;
+      for (int j = 0; j < 4; j++) {
+        c += (u128)x[j] * y[i] + t[j];
+        t[j] = (uint64_t)c;
+        c >>= 64;
       }
-      c += t[8];
-      t[8] = (uint32_t)c;
-      t[9] = (uint32_t)(c >> 32);
-      uint32_t mi = 0u - t[0];
-      c = ((uint64_t)mi * 1u + t[0]) >> 32;
-      for (int j = 1; j < 8; j++) {
-        c += (uint64_t)mi * mod_limb(j) + t[j];
-        t[j - 1] = (uint32_t)c;
-        c >>= 32;
+      c += t[4];
+      t[4] = (uint64_t)c;
+      t[5] = (uint64_t)(c >> 64);
+      const uint64_t q = t[0] * minv;
+      c = ((u128)q * m[0] + t[0]) >> 64;
+      for (int j = 1; j < 4; j++) {
+        c += (u128)q * m[j] + t[j];
+        t[j - 1] = (uint64_t)c;
+        c >>= 64;
       }
-      c += t[8];
-      t[7] = (uint32_t)c;
-      t[8] = t[9] + (uint32_t)(c >> 32);
+      c += t[4];
+      t[3] = (uint64_t)c;
+      t[4] = t[5] + (uint64_t)(c >> 64);
     }
-    int64_t bw = 0;
-    uint32_t s[8];
-    for (int j = 0; j < 8; j++) {
-      bw += (int64_t)t[j] - mod_limb(j);
-      s[j] = (uint32_t)bw;
-      bw >>= 32;
+    uint64_t s[4];
+    u128 bw = 0;
+    for (int j = 0; j < 4; j++) {
+      const u128 d = (u128)t[j] - m[j] - (uint64_t)bw;
+      s[j] = (uint64_t)d;
+      bw = (d >> 64) & 1;
     }
-    bool ge = (t[8] != 0) || (bw == 0);
-    for (int j = 0; j < 8; j++) r.v[j] = ge ? s[j] : t[j];
+    const bool ge = t[4] != 0 || bw == 0;
+    for (int j = 0; j < 4; j++) t[j] = ge ? s[j] : t[j];
+    std::memcpy(r.v, t, 32);
 #endif
     return r;
   }
